@@ -9,6 +9,9 @@
 //     chunk entirely before the target the threshold is nextafter(s_t, -inf) (s >= s_t  <=>  s > that), for
 //     a chunk entirely after it s_t; only the single chunk that contains the target takes the exact path;
 //   * the top-K list is touched only when the chunk maximum beats the current K-th best.
+// The tensor-core kernel hands over scores in a power-of-two scaled domain, s' = s f (f = 2^k, exact): the thresholds
+// are scaled instead of the scores (s' > thr f  <=>  s > thr), and only a score entering the list is scaled back
+// (s' inv).  The exact kernel passes f = inv = 1.
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -19,7 +22,6 @@ template <int TMAX>
 struct RankState {
   static constexpr int N = TMAX > 0 ? TMAX : 1;
   float st[N];      // target score
-  float st_lo[N];   // nextafter(st, -inf)
   int tg[N];        // target item id
   int rk[N];        // running count
   unsigned in_train = 0;  // bit t: the target is one of the user's train items (reported rank -1)
@@ -65,15 +67,23 @@ static __device__ __noinline__ void topk_finalize(float* __restrict__ topv, int3
   }
 }
 
+// nextafterf(x, -inf) without its branches: one ulp down for finite x and +inf, -0 / +0 -> -denorm_min, -inf and nan stay
+__device__ __forceinline__ float next_down(float x) {
+  const int b = __float_as_int(x);
+  const int n = x == 0.f ? (int)0x80000001 : (b < 0 ? b + 1 : b - 1);
+  return (x == -INFINITY || x != x) ? x : __int_as_float(n);
+}
+
 // (a): per target, count the scores of this chunk that outrank it
 template <int NC, int TMAX>
-__device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t base, int T, RankState<TMAX>& rs) {
+__device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t base, int T, RankState<TMAX>& rs, float f = 1.f) {
 #pragma unroll
   for (int t = 0; t < TMAX; ++t) {
     if (t < T) {
       const int tg = rs.tg[t];
       if (base + NC <= tg || base > tg) {          // warp-uniform: targets are the same for every user
-        const float thr = base > tg ? rs.st[t] : rs.st_lo[t];
+        const float st = rs.st[t] * f;             // nextafter(st, -inf) is derived here, not carried in a register
+        const float thr = base > tg ? st : next_down(st);
         int c0 = 0, c1 = 0, c2 = 0, c3 = 0;          // four independent chains: one warp per scheduler has
 #pragma unroll                                     // nothing else to hide the add latency behind
         for (int e = 0; e < NC; e += 4) {
@@ -84,11 +94,12 @@ __device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t b
         }
         rs.rk[t] += (c0 + c1) + (c2 + c3);
       } else {                                     // the one chunk that holds the target itself
+        const float st = rs.st[t] * f;
 #pragma unroll
         for (int e = 0; e < NC; ++e) {
           const int item = (int)base + e;
           if (item == tg) continue;
-          rs.rk[t] += (item < tg ? s[e] >= rs.st[t] : s[e] > rs.st[t]) ? 1 : 0;
+          rs.rk[t] += (item < tg ? s[e] >= st : s[e] > st) ? 1 : 0;
         }
       }
     }
@@ -98,9 +109,9 @@ __device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t b
 template <int NC, int TMAX>
 __device__ __forceinline__ void rank_topk_chunk(float (&s)[NC], int64_t base, int T, RankState<TMAX>& rs, float& tau,
                                                 float* __restrict__ topv, int32_t* __restrict__ topi, int K, int stride,
-                                                int slot, int& min_pos) {
+                                                int slot, int& min_pos, float f = 1.f, float inv = 1.f) {
   static_assert(NC % 8 == 0, "chunks are scanned in groups of 8");
-  rank_count_chunk<NC, TMAX>(s, base, T, rs);
+  rank_count_chunk<NC, TMAX>(s, base, T, rs, f);
   // group maxima (8 consecutive items each): only a group that beats tau is looked at element by element
   float gm[NC / 8];
 #pragma unroll
@@ -112,13 +123,17 @@ __device__ __forceinline__ void rank_topk_chunk(float (&s)[NC], int64_t base, in
   float cmax = gm[0];
 #pragma unroll
   for (int q = 1; q < NC / 8; ++q) cmax = fmaxf(cmax, gm[q]);
-  if (cmax > tau) {
+  float ts = tau * f;                                // tau in the scores' domain
+  if (cmax > ts) {
 #pragma unroll
     for (int q = 0; q < NC / 8; ++q) {
-      if (gm[q] > tau) {
+      if (gm[q] > ts) {
 #pragma unroll
         for (int e = 8 * q; e < 8 * q + 8; ++e)
-          if (s[e] > tau) tau = topk_replace(s[e], (int32_t)(base + e), topv, topi, K, stride, slot, min_pos);
+          if (s[e] > ts) {
+            tau = topk_replace(s[e] * inv, (int32_t)(base + e), topv, topi, K, stride, slot, min_pos);
+            ts = tau * f;
+          }
       }
     }
   }
@@ -129,7 +144,7 @@ __device__ __forceinline__ void rank_state_init(RankState<TMAX>& rs, int T, cons
                                                 const int32_t* __restrict__ train_col, int64_t lo0, int64_t hi0) {
 #pragma unroll
   for (int t = 0; t < RankState<TMAX>::N; ++t) {
-    rs.st[t] = 0.f; rs.st_lo[t] = 0.f; rs.tg[t] = -1; rs.rk[t] = 0;
+    rs.st[t] = 0.f; rs.tg[t] = -1; rs.rk[t] = 0;
     if (t < T && t < TMAX) {
       rs.tg[t] = targets[t];
       int64_t lo = lo0, hi = hi0;
@@ -142,7 +157,6 @@ __device__ __forceinline__ void rank_state_init(RankState<TMAX>& rs, int T, cons
 template <int TMAX>
 __device__ __forceinline__ void rank_state_set_score(RankState<TMAX>& rs, int t, float score) {
   rs.st[t] = score;
-  rs.st_lo[t] = nextafterf(score, -INFINITY);
 }
 
 }  // namespace recad

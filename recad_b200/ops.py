@@ -426,9 +426,10 @@ def fullrank_eval(user_emb, item_emb, user_ids, train_rowptr, train_col, targets
                   precision=None):
     """Fused score + mask + top-K + target rank (normal.py:57-93 without the score matrix).
     score(u, i) = <user_emb[u], item_emb[i]> (+ item_bias[i]).  Returns (topk_idx, topk_val, target_rank,
-    target_score).  precision "tf32x3": tcgen05 tensor-core kernel (needs D <= 64, K <= 32; fp32-accurate scores,
-    ranks may differ from "exact" between near-tied items only); "exact": CUDA-core kernel whose scores are the
-    bit-exact ascending-d FMA chain."""
+    target_score).  precision "tf32x3" (the name is kept for RECAD_EVAL_PRECISION and existing callers): tcgen05
+    tensor-core kernel, three-pass split, ~2^-21 accuracy (power-of-two scaled fp16 hi / lo operands; needs D <= 64,
+    K <= 32; ranks may differ from "exact" between near-tied items only); "exact": CUDA-core kernel whose scores are
+    the bit-exact ascending-d FMA chain."""
     _need_cuda(user_emb, item_emb, user_ids, train_rowptr, train_col, item_bias)
     dev = user_emb.device
     I, D = item_emb.shape
