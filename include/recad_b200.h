@@ -571,24 +571,14 @@ int recad_recall_ndcg(const int32_t* topk_idx, int64_t n_eval, int32_t K, const 
 int recad_mt19937_pairwise(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items,
                            int64_t train_size, const int64_t* allpos_rowptr,
                            const int32_t* allpos_col, int64_t* out, int64_t* n_out);
-/* Same result and same stream consumption as recad_mt19937_pairwise, built for 10^7..10^8 samples: the sequential
- * stream parse normally reads ONE 64-byte line per sample (filter [host] uint64[n_users * 16]: word 0 = the user's
- * row start | row length << 40, words 1..7 = 448 filter bits, words 8..15 = 512 more bits consulted only when the
- * first probe hits; filled once per dataset by recad_pairwise_filter_build; no false negatives, a "maybe" falls
- * back to the exact search; ext [host] uint32[nnz] = second-level filter of users with more than 96 positives),
- * and the positive items are gathered afterwards on n_threads host threads. */
 int recad_host_advise_huge(void* ptr, int64_t bytes);   /* madvise(MADV_HUGEPAGE) on an untouched host buffer; best effort */
-int recad_pairwise_filter_build(const int64_t* allpos_rowptr, const int32_t* allpos_col, int64_t n_users,
-                                uint64_t* filter, uint32_t* ext, int32_t n_threads);
-/* The same for users [u_lo, n_users) only; the other users' blocks are left untouched (dataset injection: the parent's
- * blocks are copied, only the appended fake users' are built). */
+/* Per-user filter blocks of recad_mt19937_pairwise_soa for users [u_lo, n_users); the other users' blocks are left
+ * untouched (dataset injection: the parent's blocks are copied, only the appended fake users' are built).
+ * filter [host] uint64[n_users * 16]: word 0 = the user's row start | row length << 40, words 1..7 = 448 filter bits,
+ * words 8..15 = 512 more bits consulted only when the first probe hits; no false negatives, a "maybe" falls back to
+ * the exact search.  ext [host] uint32[nnz of allpos] = second-level filter of the users with more than 96 positives. */
 int recad_pairwise_filter_build_range(const int64_t* allpos_rowptr, const int32_t* allpos_col, int64_t u_lo, int64_t n_users,
                                       uint64_t* filter, uint32_t* ext, int32_t n_threads);
-int recad_mt19937_pairwise_fast(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items,
-                                int64_t train_size, const int64_t* allpos_rowptr,
-                                const int32_t* allpos_col, const uint64_t* filter, const uint32_t* ext,
-                                int32_t n_threads, int64_t* out, int64_t* n_out);
-/* ext [host] uint32[nnz of allpos]: second-level filter of the users with more than 96 positives. */
 
 /* Per user k (dict order): its |pos| positives (label 1, stored order) then
  * ratio * |pos| negatives drawn with replacement from the ascending complement.
@@ -603,20 +593,15 @@ int recad_mt19937_permutation(uint32_t* key, int32_t* pos, int64_t n, int64_t* p
  * consumes the stream (j_out [host] uint32[n], j_out[i] = random_interval(i) for i = n-1 .. 1), _apply turns
  * the draws into the permutation without touching the generator -- so the caller can start drawing the next
  * epoch while another thread applies the swaps of this one. */
-/* recad_mt19937_pairwise_fast followed by recad_mt19937_permutation_draw over its *n_out rows, as ONE call: the shuffle
- * draws (j_out [host] uint32[train_size]) are made on the calling thread right behind the parse while the other
- * threads still gather the positive items and write `out` -- same results, same stream consumption. */
-int recad_mt19937_pairwise_epoch(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items, int64_t train_size,
-                                 const int64_t* allpos_rowptr, const int32_t* allpos_col, const uint64_t* filter,
-                                 const uint32_t* ext, int32_t n_threads, int64_t* out, int64_t* n_out,
-                                 uint32_t* j_out);
 int recad_mt19937_permutation_draw(uint32_t* key, int32_t* pos, int64_t n, uint32_t* j_out);
-/* Second-generation epoch sampler for 10^7..10^8 samples: same samples and stream consumption as
- * recad_mt19937_pairwise (+ recad_mt19937_permutation_draw when j_out != NULL), in 32-bit structure-of-arrays form:
+/* Epoch sampler for 10^7..10^8 samples: same samples and stream consumption as recad_mt19937_pairwise
+ * (+ recad_mt19937_permutation_draw when j_out != NULL), in 32-bit structure-of-arrays form (n_users, n_items and
+ * train_size at most 2^31 - 1):
  *   users / rel / negs [host] uint32[train_size]: user id, INDEX of the positive inside the user's row of allPos,
  *   negative item; the positive ITEM is looked up on the device by recad_samples_expand.
  * A producer thread generates the MT19937 stream into a ring, helper threads gather row lengths and verify the
- * optimistically drawn negatives; the calling thread runs the sequential parse (csrc/sampler.cpp). */
+ * optimistically drawn negatives; the calling thread runs the sequential parse (csrc/sampler.cpp).
+ * filter / ext: built by recad_pairwise_filter_build_range. */
 int recad_mt19937_pairwise_soa(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items, int64_t train_size,
                                const int64_t* allpos_rowptr, const int32_t* allpos_col, const uint64_t* filter,
                                const uint32_t* ext, int32_t n_threads, uint32_t* users, uint32_t* rel, uint32_t* negs,

@@ -153,10 +153,7 @@ SIGNATURES = {
     "recad_rank_from_scores": (C.c_int, [vp, i64, i64, vp, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp]),
     "recad_mt19937_pairwise": (C.c_int, [vp, C.POINTER(i32), i64, i64, i64, vp, vp, vp, C.POINTER(i64)]),
     "recad_host_advise_huge": (C.c_int, [vp, i64]),
-    "recad_pairwise_filter_build": (C.c_int, [vp, vp, i64, vp, vp, i32]),
     "recad_pairwise_filter_build_range": (C.c_int, [vp, vp, i64, i64, vp, vp, i32]),
-    "recad_mt19937_pairwise_fast": (C.c_int, [vp, C.POINTER(i32), i64, i64, i64, vp, vp, vp, vp, i32, vp, C.POINTER(i64)]),
-    "recad_mt19937_pairwise_epoch": (C.c_int, [vp, C.POINTER(i32), i64, i64, i64, vp, vp, vp, vp, i32, vp, C.POINTER(i64), vp]),
     "recad_mt19937_pointwise": (C.c_int, [vp, C.POINTER(i32), i64, vp, vp, vp, vp, i64, i32, vp]),
     "recad_mt19937_permutation": (C.c_int, [vp, C.POINTER(i32), i64, vp]),
     "recad_mt19937_permutation_draw": (C.c_int, [vp, C.POINTER(i32), i64, vp]),

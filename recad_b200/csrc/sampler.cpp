@@ -93,45 +93,9 @@ struct MT {
     if (__builtin_expect(pos >= 624, 0)) { mt_refill(key, buf); pos = 0; }
     return buf[pos++];
   }
-  void reset(int p) { mt_temper_only(key, buf); pos = p; }   // after the caller restored `key` from a checkpoint
-  // Both draws of a pairwise sample -- random_interval(r1) (skipped, as numpy does, when r1 == 0) then
-  // random_interval(r2) -- from a four-output window: all loads and compares are issued at once and the only
-  // loop-carried dependency is pos -> selects -> pos.  Returns false, consuming nothing, when the window does not
-  // settle both draws (a double rejection, ~10 %, or the end of the buffer): the caller then uses masked_with().
-  inline bool draw_pair(uint32_t r1, uint32_t m1, uint32_t r2, uint32_t m2, uint32_t& v1, uint32_t& v2) {
-    if (__builtin_expect(pos + 4 > 624, 0)) return false;
-    const uint32_t o0 = buf[pos], o1 = buf[pos + 1], o2 = buf[pos + 2], o3 = buf[pos + 3];
-    const uint32_t a0 = o0 & m1, a1 = o1 & m1;
-    const bool none = r1 == 0, okA0 = a0 <= r1, okA1 = a1 <= r1;
-    const int cA = none ? 0 : (okA0 ? 1 : 2);
-    const uint32_t x0 = cA == 0 ? o0 : (cA == 1 ? o1 : o2), x1 = cA == 0 ? o1 : (cA == 1 ? o2 : o3);
-    const uint32_t b0 = x0 & m2, b1 = x1 & m2;
-    const bool okB0 = b0 <= r2, okB1 = b1 <= r2;
-    if (__builtin_expect(!((none | okA0 | okA1) & (okB0 | okB1)), 0)) return false;
-    v1 = none ? 0u : (okA0 ? a0 : a1);
-    v2 = okB0 ? b0 : b1;
-    pos += cA + (okB0 ? 1 : 2);
-    return true;
-  }
-  // n draws of random_interval(r) with ONE mask, written to dst[0..n): every output is stored at the cursor and the
-  // cursor advances only if it is accepted -- no branch on the (random) acceptance, a 2-cycle dependency per output
-  void fill_masked(uint32_t* dst, int64_t n, uint32_t r, uint32_t mask) {
-    int64_t k = 0;
-    while (k < n) {
-      if (pos >= 624) { mt_refill(key, buf); pos = 0; }
-      int p = pos;
-      // the cursor can advance at most once per output: stay inside dst for the whole buffer pass
-      const int stop = (int)std::min<int64_t>(624, p + (n - k));
-      for (; p < stop; ++p) {
-        const uint32_t v = buf[p] & mask;
-        dst[k] = v;
-        k += v <= r;
-      }
-      pos = p;
-    }
-  }
   // the draws of a Fisher-Yates pass over one power-of-two band: j[i] = random_interval(i) for i = hi, hi-1, .., lo
-  // (all share `mask`); same branchless cursor, moving down
+  // (all share `mask`): every output is stored at the cursor and the cursor moves down only if it is accepted -- no
+  // branch on the (random) acceptance
   void fill_band_desc(uint32_t* j, int64_t hi, int64_t lo, uint32_t mask) {
     int64_t i = hi;
     while (i >= lo) {
@@ -296,13 +260,9 @@ int recad_mt19937_pairwise(uint32_t* key, int32_t* pos, int64_t n_users, int64_t
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Fast exact pairwise sampler.  The stream parse is inherently sequential (every draw's position depends on all
-// earlier rejections), so it is made as light as possible: per sample it touches the row pointer and ONE OR TWO
-// cache lines of a per-user 1024-bit membership filter (no false negatives; a "maybe" falls back to the exact
-// binary search of the user's sorted list, a "no" accepts the negative without ever reading the list).  Both
-// addresses are known in advance (all users are drawn first) and software-prefetched.  The positive ITEM is only
-// recorded as an index during the parse; the gather of the items -- the other random access -- runs afterwards on
-// all host threads.
+// Per-user membership filter of the large-epoch sampler (recad_mt19937_pairwise_soa).  Checking a negative
+// candidate touches ONE OR TWO cache lines of a 1024-bit filter (no false negatives; a "maybe" falls back to the
+// exact binary search of the user's sorted list, a "no" accepts the negative without ever reading the list).
 // ---------------------------------------------------------------------------------------------------------
 // Two 64-byte lines per user, of which a sample normally touches only the FIRST:
 //   line 0: word 0 = first entry of the user's row | row length << 40, words 1..7 = 448 filter bits (region A)
@@ -356,12 +316,7 @@ static inline uint64_t ext_probe(uint32_t item, int j, uint64_t nbits) {
   return ((uint64_t)h * nbits) >> 32;
 }
 
-int recad_pairwise_filter_build(const int64_t* allpos_rowptr, const int32_t* allpos_col, int64_t n_users, uint64_t* filter,
-                                uint32_t* ext, int32_t n_threads) {
-  return recad_pairwise_filter_build_range(allpos_rowptr, allpos_col, 0, n_users, filter, ext, n_threads);
-}
-
-// users [u_lo, u_hi) only: the blocks of the other users are left as they are (an injected dataset copies its parent's
+// users [u_lo, n_users) only: the blocks of the other users are left as they are (an injected dataset copies its parent's
 // blocks -- appended fake users do not move anybody's row -- and builds only the new ones)
 int recad_pairwise_filter_build_range(const int64_t* allpos_rowptr, const int32_t* allpos_col, int64_t u_lo, int64_t n_users,
                                       uint64_t* filter, uint32_t* ext, int32_t n_threads) {
@@ -407,279 +362,10 @@ int recad_pairwise_filter_build_range(const int64_t* allpos_rowptr, const int32_
   return RECAD_OK;
 }
 
-// j_out != NULL: the draws of the epoch shuffle (recad_mt19937_permutation_draw over the *n_out rows) are made right
-// behind the parse, on this thread, WHILE the other threads gather the positive items and write the 64-bit rows
-static int pairwise_fast_impl(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items, int64_t train_size,
-                              const int64_t* allpos_rowptr, const int32_t* allpos_col, const uint64_t* filter,
-                              const uint32_t* ext, int32_t n_threads, int64_t* out, int64_t* n_out, uint32_t* j_out) {
-  if (!key || !pos || !allpos_rowptr || !filter || !ext || !out || !n_out || n_users <= 0 || n_items <= 0 || train_size < 0 ||
-      n_users > 0xffffffffLL || n_items > 0xffffffffLL) {
-    recad::set_error("mt19937_pairwise_fast: bad argument");
-    return RECAD_ERR_ARG;
-  }
-  MT mt(key, *pos);
-  const bool trace = getenv("RECAD_SAMPLER_TRACE") != nullptr;
-  auto t0 = std::chrono::steady_clock::now();
-  auto lap = [&](const char* what) {
-    if (!trace) return;
-    auto t1 = std::chrono::steady_clock::now();
-    fprintf(stderr, "[sampler] %s %.3f s\n", what, std::chrono::duration<double>(t1 - t0).count());
-    t0 = t1;
-  };
-  // scratch of the sequential part, kept between calls (callers are serialised: the epochs of one stream cannot be
-  // drawn concurrently anyway): 32-bit users and compact (user, index of the positive, negative) triples -- the
-  // 64-bit rows of `out` are written by the parallel pass below, so the sequential thread moves 16 instead of 32
-  // bytes per sample
-  static std::mutex scratch_mutex;
-  static Scratch<uint32_t> users_buf;
-  static Scratch<uint32_t> neg_buf;
-  std::lock_guard<std::mutex> scratch_lock(scratch_mutex);
-  uint32_t* users = users_buf.get(train_size);
-  uint32_t* negs = neg_buf.get(train_size);
-  if (!users || !negs) {
-    recad::set_error("mt19937_pairwise_fast: out of host memory");
-    return RECAD_ERR_ARG;
-  }
-  {
-    const uint32_t r = (uint32_t)(n_users - 1), mask = MT::mask_of(r);
-    if (r == 0) {
-      memset(users, 0, (size_t)train_size * sizeof(uint32_t));
-    } else {
-      mt.fill_masked(users, train_size, r, mask);
-    }
-  }
-  lap("draw users");
-  // The stream is parsed block by block (kBlock samples) in two decoupled steps:
-  //  DRAW (this thread, cache resident): every sample of the block is drawn OPTIMISTICALLY -- position of the positive,
-  //    then the first negative candidate the mask accepts, assuming the candidate is not one of the user's positives
-  //    (true for all but ~deg/I of the samples).  It touches only the row pointer (8 MB).
-  //  CHECK (a pool of spinning helper threads): the assumption is verified against the per-user filter lines -- the
-  //    DRAM-bound part, which one core can only do at ~75 M random lines/s (line-fill buffers), spread over several,
-  //    and it runs WHILE this thread already draws the next block.
-  //  When a candidate IS a positive (about one block in eight) the generator is rewound to the checkpoint, the draws
-  //  up to that sample are replayed (same outputs), the sample is finished with the exact inline loop, the checkpoint
-  //  moves behind it and everything drawn behind it (rest of the block, the speculative next block) is drawn again.  Result and stream consumption are exactly
-  //  those of the plain loop (tests/test_cpu_boundary.py).
-  constexpr int64_t kBlock = 512, kAhead = 16, kAheadLen = 32;
-  constexpr uint32_t kDropped = 0xffffffffu;
-  constexpr int64_t kNoFail = INT64_MAX;
-  const uint32_t neg_r = (uint32_t)(n_items - 1), neg_mask = MT::mask_of(neg_r);
-  static Scratch<uint32_t> rel_buf;
-  uint32_t* rel = rel_buf.get(train_size);           // index of the positive inside the user's row, or kDropped
-  if (!rel) {
-    recad::set_error("mt19937_pairwise_fast: out of host memory");
-    return RECAD_ERR_ARG;
-  }
-  auto is_positive = [&](const uint64_t* f, int64_t lo, int64_t len, uint32_t neg) -> bool {
-    const uint32_t a = probe_a(neg);
-    if (!((f[a >> 6] >> (a & 63)) & 1ull)) return false;                                       // definitely not a positive
-    uint32_t b, c;
-    probes_bc(neg, len <= kLight, b, c);
-    if (!((f[b >> 6] >> (b & 63)) & (f[c >> 6] >> (c & 63)) & 1ull)) return false;
-    if (len > kHeavy) {                                                                        // heavy user: second level
-      const uint64_t nbits = (uint64_t)len * 32;
-      const uint64_t p0 = ext_probe(neg, 0, nbits), p1 = ext_probe(neg, 1, nbits), p2 = ext_probe(neg, 2, nbits);
-      if (!((ext[lo + (p0 >> 5)] >> (p0 & 31)) & (ext[lo + (p1 >> 5)] >> (p1 & 31)) & (ext[lo + (p2 >> 5)] >> (p2 & 31)) & 1u))
-        return false;
-    }
-    return std::binary_search(allpos_col + lo, allpos_col + lo + len, (int32_t)neg);           // filter false positive?
-  };
-  // first sample of [a0, a1) whose candidate is one of its user's positives
-  auto check = [&](int64_t a0, int64_t a1) -> int64_t {
-    for (int64_t k = a0; k < std::min(a1, a0 + kAhead); ++k) __builtin_prefetch(filter + (int64_t)users[k] * kFilterWords);
-    for (int64_t k = a0; k < a1; ++k) {
-      if (k + kAhead < a1) __builtin_prefetch(filter + (int64_t)users[k + kAhead] * kFilterWords);
-      if (rel[k] == kDropped) continue;
-      const uint64_t* f = filter + (int64_t)users[k] * kFilterWords;
-      if (__builtin_expect(is_positive(f, (int64_t)(f[0] & (((uint64_t)1 << 40) - 1)), (int64_t)(f[0] >> 40), negs[k]), 0)) return k;
-    }
-    return kNoFail;
-  };
-  // helper pool: spins on `go`, checks its slice of [job_lo, job_hi), reports the first failure, bumps `done`
-  struct alignas(64) Slot { std::atomic<int64_t> fail; };
-  const int n_help = getenv("RECAD_SAMPLER_HELPERS") ? atoi(getenv("RECAD_SAMPLER_HELPERS")) : (int)std::max(0, std::min(n_threads / 2 - 1, 7));   // half the cores at most: the swaps of the previous epoch and the caller run too
-  std::vector<Slot> slots((size_t)n_help + 1);
-  std::atomic<int64_t> go{0}, done{0};
-  std::atomic<bool> quit{false};
-  int64_t job_lo = 0, job_hi = 0;
-  auto slice = [&](int t, int64_t& a0, int64_t& a1) {      // helper t = 1 .. n_help
-    const int64_t n = job_hi - job_lo, per = (n + n_help - 1) / n_help;
-    a0 = std::min(job_hi, job_lo + (t - 1) * per);
-    a1 = std::min(job_hi, a0 + per);
-  };
-  std::vector<std::thread> helpers;
-  for (int t = 1; t <= n_help; ++t)
-    helpers.emplace_back([&, t]() {
-      int64_t seen = 0;
-      for (;;) {
-        int spins = 0;
-        while (go.load(std::memory_order_acquire) == seen) {
-          if (quit.load(std::memory_order_relaxed)) return;
-          if (++spins > 2000) { std::this_thread::yield(); spins = 0; } else { cpu_relax(); }
-        }
-        ++seen;
-        int64_t a0, a1;
-        slice(t, a0, a1);
-        slots[(size_t)t].fail.store(check(a0, a1), std::memory_order_relaxed);
-        done.fetch_add(1, std::memory_order_release);
-      }
-    });
-  // the check of [lo_, hi_) runs on the helpers while this thread goes on drawing; finish_check() collects the result
-  int64_t inline_result = kNoFail;
-  bool pool_busy = false;
-  auto start_check = [&](int64_t lo_, int64_t hi_) {
-    if (n_help == 0 || hi_ - lo_ < 64) { inline_result = check(lo_, hi_); pool_busy = false; return; }
-    job_lo = lo_; job_hi = hi_;
-    done.store(0, std::memory_order_relaxed);
-    go.fetch_add(1, std::memory_order_release);
-    pool_busy = true;
-  };
-  auto finish_check = [&]() -> int64_t {
-    if (!pool_busy) return inline_result;
-    while (done.load(std::memory_order_acquire) < n_help) cpu_relax();
-    int64_t first = kNoFail;
-    for (int t = 1; t <= n_help; ++t) first = std::min(first, slots[(size_t)t].fail.load(std::memory_order_relaxed));
-    pool_busy = false;
-    return first;
-  };
-  // DRAW for samples [k0, k1)
-  auto draw = [&](int64_t k0, int64_t k1) -> int {
-    for (int64_t k = k0; k < k1; ++k) {
-      if (k + kAheadLen < train_size) __builtin_prefetch(allpos_rowptr + users[k + kAheadLen]);
-      const int64_t u = users[k];
-      const int64_t len = allpos_rowptr[u + 1] - allpos_rowptr[u];
-      if (len == 0) { rel[k] = kDropped; continue; }                     // implicit.py:63-64
-      if (len >= n_items) {
-        recad::set_error("mt19937_pairwise_fast: user %lld interacted with every item; negative sampling cannot terminate",
-                         (long long)u);
-        return RECAD_ERR_ARG;
-      }
-      const uint32_t r1 = (uint32_t)(len - 1), m1 = r1 ? 0xffffffffu >> __builtin_clz(r1) : 0u;
-      if (__builtin_expect(neg_r != 0 && mt.draw_pair(r1, m1, neg_r, neg_mask, rel[k], negs[k]), 1)) continue;
-      rel[k] = r1 ? mt.masked_with(r1, m1) : 0u;
-      negs[k] = neg_r == 0 ? 0u : mt.masked_with(neg_r, neg_mask);
-    }
-    return RECAD_OK;
-  };
-  int rc = RECAD_OK;
-  int64_t n_rewind = 0;
-  uint32_t ck_key[624], nx_key[624];
-  int ck_pos = mt.pos, nx_pos = 0;
-  memcpy(ck_key, key, sizeof(ck_key));                     // checkpoint: generator state in front of sample ck_from
-  int64_t ck_from = 0;
-  rc = draw(0, std::min(train_size, kBlock));
-  for (int64_t b0 = 0; b0 < train_size && rc == RECAD_OK; b0 += kBlock) {
-    // invariant: block [b0, b1) is drawn (optimistically) from the checkpoint at ck_from = b0
-    const int64_t b1 = std::min(train_size, b0 + kBlock), n1 = std::min(train_size, b1 + kBlock);
-    start_check(b0, b1);
-    memcpy(nx_key, key, sizeof(nx_key));                   // state behind block b = checkpoint of block b + 1
-    nx_pos = mt.pos;
-    if (b1 < train_size && (rc = draw(b1, n1))) { finish_check(); break; }   // speculative: runs under the check of block b
-    int64_t k = finish_check();
-    if (k == kNoFail) {
-      memcpy(ck_key, nx_key, sizeof(ck_key));
-      ck_pos = nx_pos;
-      ck_from = b1;
-      continue;
-    }
-    // a candidate of block b is a positive: what was drawn behind it (rest of b, all of b + 1) is void
-    while (k != kNoFail) {
-      // rewind, replay the draws up to and including sample k (same outputs), finish it with the exact loop, move the
-      // checkpoint behind it, redraw and recheck the rest of the block
-      memcpy(key, ck_key, sizeof(ck_key));
-      mt.reset(ck_pos);
-      if ((rc = draw(ck_from, k + 1))) break;
-      const int64_t u = users[k];
-      const int64_t lo = allpos_rowptr[u], len = allpos_rowptr[u + 1] - lo;
-      const uint64_t* f = filter + u * kFilterWords;
-      uint32_t neg;
-      do { neg = neg_r == 0 ? 0u : mt.masked_with(neg_r, neg_mask); } while (is_positive(f, lo, len, neg));
-      negs[k] = neg;
-      memcpy(ck_key, key, sizeof(ck_key));
-      ck_pos = mt.pos;
-      ck_from = k + 1;
-      if ((rc = draw(k + 1, b1))) break;
-      ++n_rewind;
-      start_check(ck_from, b1);
-      k = finish_check();
-    }
-    if (rc) break;
-    memcpy(ck_key, key, sizeof(ck_key));                   // block b is final; block b + 1 is drawn again from here
-    ck_pos = mt.pos;
-    ck_from = b1;
-    if (b1 < train_size) rc = draw(b1, n1);
-  }
-  quit.store(true, std::memory_order_relaxed);
-  for (auto& h : helpers) h.join();
-  if (rc) return rc;
-  if (trace) fprintf(stderr, "[sampler] %lld rewinds, %d helper threads\n", (long long)n_rewind, n_help);
-  lap("parse stream");
-  // ---- compaction (users without positives are dropped) + gather of the positive items + 64-bit rows, all threads
-  int64_t w = 0;
-  {
-    const int nt = (int)std::max<int64_t>(1, std::min<int64_t>(n_threads, (train_size + 65535) / 65536));
-    const int64_t per = (train_size + nt - 1) / nt;
-    std::vector<int64_t> cnt((size_t)nt + 1, 0);
-    parallel_for(nt, nt, [&](int64_t t0, int64_t t1) {
-      for (int64_t t = t0; t < t1; ++t) {
-        int64_t c = 0;
-        for (int64_t k = t * per; k < std::min(train_size, (t + 1) * per); ++k) c += rel[k] != kDropped;
-        cnt[(size_t)t + 1] = c;
-      }
-    });
-    for (int t = 0; t < nt; ++t) cnt[(size_t)t + 1] += cnt[(size_t)t];
-    w = cnt[(size_t)nt];
-    std::vector<std::thread> th;
-    for (int t = 0; t < nt; ++t) {
-      th.emplace_back([&, t]() {
-        int64_t o = cnt[(size_t)t];
-        const int64_t a1 = std::min(train_size, (t + 1) * per);
-        constexpr int64_t kAheadG = 16;
-        for (int64_t k = t * per; k < a1; ++k) {
-          if (k + kAheadG < a1 && rel[k + kAheadG] != kDropped)
-            __builtin_prefetch(allpos_col + allpos_rowptr[users[k + kAheadG]] + rel[k + kAheadG]);
-          if (rel[k] == kDropped) continue;
-          const int64_t u = users[k];
-          out[3 * o] = u;
-          out[3 * o + 1] = allpos_col[allpos_rowptr[u] + rel[k]];
-          out[3 * o + 2] = negs[k];
-          ++o;
-        }
-      });
-    }
-    if (j_out) {                       // the stream goes on while the rows are being written
-      shuffle_draws(mt, w, j_out);
-      lap("shuffle draws (under the gather)");
-    }
-    for (auto& x : th) x.join();
-  }
-  lap("gather positives");
-  *n_out = w;
-  *pos = mt.pos;
-  return RECAD_OK;
-}
-
-int recad_mt19937_pairwise_fast(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items, int64_t train_size,
-                                const int64_t* allpos_rowptr, const int32_t* allpos_col, const uint64_t* filter,
-                                const uint32_t* ext, int32_t n_threads, int64_t* out, int64_t* n_out) {
-  return pairwise_fast_impl(key, pos, n_users, n_items, train_size, allpos_rowptr, allpos_col, filter, ext, n_threads, out,
-                            n_out, nullptr);
-}
-
-int recad_mt19937_pairwise_epoch(uint32_t* key, int32_t* pos, int64_t n_users, int64_t n_items, int64_t train_size,
-                                 const int64_t* allpos_rowptr, const int32_t* allpos_col, const uint64_t* filter,
-                                 const uint32_t* ext, int32_t n_threads, int64_t* out, int64_t* n_out, uint32_t* j_out) {
-  if (!j_out) {
-    recad::set_error("mt19937_pairwise_epoch: bad argument");
-    return RECAD_ERR_ARG;
-  }
-  return pairwise_fast_impl(key, pos, n_users, n_items, train_size, allpos_rowptr, allpos_col, filter, ext, n_threads, out,
-                            n_out, j_out);
-}
-
 // ---------------------------------------------------------------------------------------------------------
-// Second-generation epoch sampler (recad_mt19937_pairwise_soa).  Same samples, same stream consumption as
-// recad_mt19937_pairwise (implicit.py:50-74) + the shuffle draws (implicit.py:24-25); what changed is who does what:
+// Large-epoch sampler (recad_mt19937_pairwise_soa).  Same samples, same stream consumption as
+// recad_mt19937_pairwise (implicit.py:50-74) + the shuffle draws (implicit.py:24-25).  The stream parse is inherently
+// sequential (every draw's position depends on all earlier rejections), so everything else is moved off it:
 //   * a PRODUCER thread generates the MT19937 output stream into a ring -- the stream does not depend on the parse,
 //     so rewinding the parser is just resetting an index (no generator checkpoints), and the parser never runs a twist;
 //   * the users are drawn first (implicit.py:57); while they are drawn, helper threads already gather every sample's
@@ -851,9 +537,8 @@ int recad_mt19937_pairwise_soa(uint32_t* key, int32_t* pos, int64_t n_users, int
   std::atomic<int64_t> next_chunk{0}, chunks_done{0};
   std::vector<std::atomic<uint8_t>> chunk_done((size_t)std::max<int64_t>(n_chunks, 1));
   for (auto& c : chunk_done) c.store(0, std::memory_order_relaxed);
-  const int64_t kBlock = getenv("RECAD_SAMPLER_BLOCK") ? atoll(getenv("RECAD_SAMPLER_BLOCK")) : 512;   // power of two
+  constexpr int64_t kBlock = 512;               // power of two: the offsets ring below is indexed with a mask
   constexpr int64_t kAhead = 16;
-  const uint64_t kStreamAhead = getenv("RECAD_SAMPLER_PF") ? (uint64_t)atoll(getenv("RECAD_SAMPLER_PF")) : 512;
   constexpr uint32_t kDropped = 0xffffffffu;
   constexpr int64_t kNoFail = INT64_MAX;
   const uint32_t neg_r = (uint32_t)(n_items - 1), neg_mask = MT::mask_of(neg_r);
@@ -957,7 +642,7 @@ int recad_mt19937_pairwise_soa(uint32_t* key, int32_t* pos, int64_t n_users, int
   // ---- parse
   std::vector<uint32_t> tst_v((size_t)4 * kBlock);            // stream offset in front of each sample (ring of 4 blocks)
   uint32_t* tst = tst_v.data();
-  const int64_t kTstMask = 4 * kBlock - 1;
+  constexpr int64_t kTstMask = 4 * kBlock - 1;
   int rc = RECAD_OK;
   // optimistic draw of samples [k0, k1): position of the positive, first candidate the mask accepts.  The stream
   // cursor and every pointer live in locals: the loop-carried chain is cursor -> 4 loads -> compares -> selects -> cursor
@@ -1027,9 +712,7 @@ int recad_mt19937_pairwise_soa(uint32_t* key, int32_t* pos, int64_t n_users, int
   };
   int64_t inline_result = kNoFail;
   bool pool_busy = false;
-  const bool dbg_nocheck = getenv("RECAD_SAMPLER_DEBUG_NOCHECK") != nullptr;   // timing experiments only: WRONG samples
   auto start_check = [&](int64_t lo_, int64_t hi_) {
-    if (dbg_nocheck) { inline_result = kNoFail; pool_busy = false; return; }
     if (hi_ - lo_ < 64) { inline_result = check(lo_, hi_); pool_busy = false; return; }
     job_lo = lo_; job_hi = hi_;
     done.store(0, std::memory_order_relaxed);

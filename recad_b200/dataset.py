@@ -155,8 +155,7 @@ class _EpochPipe:
         """Large pairwise epochs take the 32-bit structure-of-arrays path: the host sampler emits (user, index of the
         positive, negative) as uint32, the positive ITEM is gathered on the device, rows and permutation stay int32."""
         d = self.data
-        return (cuda and d.config["sample"] == "pairwise" and d.traindataSize >= ops.FAST_SAMPLER_MIN
-                and d.traindataSize < (1 << 31) and d.n_users < (1 << 31) and d.n_items < (1 << 31))
+        return cuda and d.config["sample"] == "pairwise" and ops.fits_soa_sampler(d.n_users, d.n_items, d.traindataSize)
 
     _POOL = []          # pinned 32-bit buffer sets of pipes that were garbage collected (page-locking 0.8 GB costs ~0.3 s)
 
@@ -201,11 +200,8 @@ class _EpochPipe:
             ops.permutation_apply32(jb[:m], p.numpy())
             return ("soa", u[:m], r[:m], g[:m], p[:m])
         _, s, p, jb = buf
-        if d.config["sample"] == "pairwise":          # sampler + shuffle draws in one call (draws under the row gather)
-            S, j = ops.mt_pairwise_epoch_raw(key, pos, d.n_users, d.n_items, d.traindataSize, *d._allpos, out=s.numpy(), j_out=jb)
-        else:
-            S = d._draw_samples(key, pos, s.numpy())
-            j = ops.mt_permutation_draw_raw(key, pos, len(S), jb)
+        S = d._draw_samples(key, pos, s.numpy())
+        j = ops.mt_permutation_draw_raw(key, pos, len(S), jb)
         if after_rng is not None:
             after_rng()
         perm = ops.permutation_apply(j, p.numpy())
@@ -501,12 +497,6 @@ class ImplicitData:
             return ops.mt_pointwise_raw(key, pos, *self._tr, self.n_items, self.config["negative_ratio"], out=out)
         raise NotImplementedError("Not implemented yet")
 
-    def _draw_epoch(self, key, pos, buf=None):
-        """Sampler + shuffle from an EXPLICIT MT19937 state (key, pos are advanced in place)."""
-        S = self._draw_samples(key, pos, None if buf is None else buf[0])
-        perm = ops.mt_permutation_raw(key, pos, len(S), out=None if buf is None else buf[1])
-        return S, perm
-
     def generate_batch(self, **config):
         c = self.config
         if self.mode() == "train":
@@ -637,7 +627,6 @@ class ArrayImplicitData:
     switch_mode = ImplicitData.switch_mode
     epoch_samples = ImplicitData.epoch_samples
     _draw_samples = ImplicitData._draw_samples
-    _draw_epoch = ImplicitData._draw_epoch
     generate_batch = ImplicitData.generate_batch
 
     def allpos_device(self, device):

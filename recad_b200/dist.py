@@ -428,7 +428,6 @@ class _Rank0Epochs:
         self.n_users, self.n_items, self.traindataSize = int(n_users), int(n_items), int(len(allpos_col))
         self._allpos = (allpos_rowptr, allpos_col)
         self._draw_samples = ImplicitData._draw_samples.__get__(self)
-        self._draw_epoch = ImplicitData._draw_epoch.__get__(self)
 
 
 # ---------------------------------------------------------------------------------------------- bench.py --gpus N

@@ -529,40 +529,24 @@ def _np(a, dtype=np.int64):
 # *_raw: explicit MT19937 state -- key: uint32[624] (advanced in place), pos: one-element list.
 # The ctypes calls release the GIL, so a raw sampler can run on a background thread.
 def mt_pairwise_raw(key, pos, n_users, n_items, train_size, allpos_rowptr, allpos_col, out=None):
+    """pairwise_sample (implicit.py:50-74) as int64 rows (user, positive, negative).  A large epoch is drawn by
+    mt_pairwise_soa_raw and its positive items are gathered here; any other by the plain sampler."""
     rp, col = _np(allpos_rowptr), _np(allpos_col, np.int32)
     if out is None:
         out = np.empty((max(train_size, 1), 3), dtype=np.int64)
     assert out.dtype == np.int64 and out.flags.c_contiguous and out.shape[0] >= train_size
+    if fits_soa_sampler(n_users, n_items, train_size):
+        users, rel, negs = (host_empty(train_size, np.uint32) for _ in range(3))
+        m = mt_pairwise_soa_raw(key, pos, n_users, n_items, train_size, rp, col, users, rel, negs)
+        out[:m, 0] = users[:m]
+        out[:m, 1] = col[rp[users[:m]] + rel[:m]]
+        out[:m, 2] = negs[:m]
+        return out[:m]
     n_out, cpos = C.c_int64(), C.c_int32(pos[0])
-    if train_size >= FAST_SAMPLER_MIN:
-        filt, ext = pairwise_filter(rp, col, n_users)
-        check(_lib.lib().recad_mt19937_pairwise_fast(key.ctypes.data, C.byref(cpos), n_users, n_items, train_size, rp.ctypes.data,
-                                                     col.ctypes.data, filt.ctypes.data, ext.ctypes.data, min(os.cpu_count() or 1, 32),
-                                                     out.ctypes.data, C.byref(n_out)), "recad_mt19937_pairwise_fast")
-    else:
-        check(_lib.lib().recad_mt19937_pairwise(key.ctypes.data, C.byref(cpos), n_users, n_items, train_size, rp.ctypes.data,
-                                                col.ctypes.data, out.ctypes.data, C.byref(n_out)), "recad_mt19937_pairwise")
+    check(_lib.lib().recad_mt19937_pairwise(key.ctypes.data, C.byref(cpos), n_users, n_items, train_size, rp.ctypes.data,
+                                            col.ctypes.data, out.ctypes.data, C.byref(n_out)), "recad_mt19937_pairwise")
     pos[0] = cpos.value
     return out[:n_out.value]
-
-
-def mt_pairwise_epoch_raw(key, pos, n_users, n_items, train_size, allpos_rowptr, allpos_col, out, j_out):
-    """Sampler + the draws of the epoch shuffle as one call (large epochs only): -> (samples [n, 3], j [n]); the draws run
-    on the calling thread while the other threads still write the rows.  Same stream consumption as
-    mt_pairwise_raw followed by mt_permutation_draw_raw."""
-    if train_size < FAST_SAMPLER_MIN:
-        S = mt_pairwise_raw(key, pos, n_users, n_items, train_size, allpos_rowptr, allpos_col, out=out)
-        return S, mt_permutation_draw_raw(key, pos, len(S), j_out)
-    rp, col = _np(allpos_rowptr), _np(allpos_col, np.int32)
-    assert out.dtype == np.int64 and out.flags.c_contiguous and out.shape[0] >= train_size
-    assert j_out.dtype == np.uint32 and j_out.flags.c_contiguous and j_out.shape[0] >= train_size
-    filt, ext = pairwise_filter(rp, col, n_users)
-    n_out, cpos = C.c_int64(), C.c_int32(pos[0])
-    check(_lib.lib().recad_mt19937_pairwise_epoch(key.ctypes.data, C.byref(cpos), n_users, n_items, train_size, rp.ctypes.data,
-                                                  col.ctypes.data, filt.ctypes.data, ext.ctypes.data, min(os.cpu_count() or 1, 32),
-                                                  out.ctypes.data, C.byref(n_out), j_out.ctypes.data), "recad_mt19937_pairwise_epoch")
-    pos[0] = cpos.value
-    return out[:n_out.value], j_out[:n_out.value]
 
 
 def mt_pairwise_soa_raw(key, pos, n_users, n_items, train_size, allpos_rowptr, allpos_col, users, rel, negs, j_out=None):
@@ -618,6 +602,12 @@ def to_host(t, dtype=None):
 FAST_SAMPLER_MIN = 1 << 20      # samples per epoch from which the filter-based parser pays off
 
 
+def fits_soa_sampler(n_users, n_items, train_size):
+    """Whether a pairwise epoch is drawn by mt_pairwise_soa_raw: large enough for its filter to pay off, and every id
+    and count within the sampler's 32-bit arrays."""
+    return FAST_SAMPLER_MIN <= train_size < (1 << 31) and n_users < (1 << 31) and n_items < (1 << 31)
+
+
 class _DerivedCache:
     """Per-dataset host structures derived from the positives (filter blocks, sorted lists), keyed by the identity of
     the source arrays.  The entry keeps those arrays alive, so an address can never be reused by another dataset while
@@ -661,7 +651,7 @@ def _filter_key(rowptr, col, n_users):
 
 
 def pairwise_filter(allpos_rowptr, allpos_col, n_users):
-    """Per-user 128-byte blocks (row bounds + two-level membership filter, first line decisive) for mt_pairwise_raw(fast);
+    """Per-user 128-byte blocks (row bounds + two-level membership filter, first line decisive) for mt_pairwise_soa_raw;
     built once per positives array -- or, for a dataset derived by injection from one whose blocks are still cached,
     copied from the parent and completed for the appended users only."""
     def build():

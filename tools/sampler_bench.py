@@ -3,6 +3,7 @@
     RECAD_SAMPLER_TRACE=1 python tools/sampler_bench.py [--epochs 3] [--cache /tmp/sb/allpos.npz]
 """
 import argparse
+import ctypes as C
 import os
 import sys
 import time
@@ -12,7 +13,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench  # noqa: E402
-from recad_b200 import ops  # noqa: E402
+from recad_b200 import _lib, ops  # noqa: E402
 
 
 def allpos(w, cache):
@@ -34,7 +35,8 @@ def main():
     ap.add_argument("--epochs", type=int, default=3)
     ap.add_argument("--workload", default="synthetic")
     ap.add_argument("--cache", default="")
-    ap.add_argument("--compare", action="store_true", help="also run the round-1 sampler and compare every output")
+    ap.add_argument("--compare", action="store_true",
+                    help="also run the plain sampler + shuffle draws (recad_mt19937_pairwise) and compare every output")
     a = ap.parse_args()
     w = bench.WORKLOADS[a.workload]
     t0 = time.time()
@@ -60,14 +62,19 @@ def main():
         print(f"epoch {e} [soa]: sampler+draws {t1 - t0:.3f} s, swaps {t2 - t1:.3f} s", flush=True)
         if a.compare:
             t0 = time.time()
-            S, jj = ops.mt_pairwise_epoch_raw(key, pos, w["n_users"], w["n_items"], n, hp, hc, out, j)
+            n_out, cpos = C.c_int64(), C.c_int32(pos[0])
+            _lib.check(_lib.lib().recad_mt19937_pairwise(key.ctypes.data, C.byref(cpos), w["n_users"], w["n_items"], n, hp.ctypes.data,
+                                                         hc.ctypes.data, out.ctypes.data, C.byref(n_out)), "recad_mt19937_pairwise")
+            pos[0] = cpos.value
+            S = out[:n_out.value]
+            jj = ops.mt_permutation_draw_raw(key, pos, len(S), j)
             t1 = time.time()
             ops.permutation_apply(jj, perm)
             t2 = time.time()
             same = (m == len(S) and np.array_equal(users[:m], S[:, 0]) and np.array_equal(hc[hp[users[:m]] + rel[:m]], S[:, 1])
                     and np.array_equal(negs[:m], S[:, 2]) and np.array_equal(j2[:m], jj) and np.array_equal(perm32[:m], perm[:m])
                     and np.array_equal(key, key2) and pos[0] == pos2[0])
-            print(f"epoch {e} [round 1]: sampler+draws {t1 - t0:.3f} s, swaps {t2 - t1:.3f} s; identical to soa: {same}", flush=True)
+            print(f"epoch {e} [plain]: sampler+draws {t1 - t0:.3f} s, swaps {t2 - t1:.3f} s; identical: {same}", flush=True)
 
 
 if __name__ == "__main__":
