@@ -405,6 +405,30 @@ int recad_dot_scores(const float* O, int64_t n_users, const int64_t* users, cons
                      int64_t B, int32_t D, float* scores, void* stream);
 
 /* ------------------------------------------------------------------------ *
+ * Autograd backward passes of the victims' scores (what `loss.backward()` through
+ * lightgcn.py:82-113 / 174-183, mf.py:40-47 and ncf.py:112-131 computes)
+ * ------------------------------------------------------------------------ */
+
+/* Backward of pair scores s_b = <Xa[ia[b]], Xb[ib[b]]> (+ ba[ia[b]] + bb[ib[b]]) for the upstream gradient g [dev] float[B]:
+ *   dXa [dev] float[n_a, D] = sum over the b with ia[b] = r of g[b] Xb[ib[b]], dXb [dev] float[n_b, D] likewise (dense:
+ *   rows no sample names are zero), dba [dev] float[n_a] / dbb [dev] float[n_b] = sum of g[b] per row (NULL: not wanted).
+ * Atomic-free and bit-stable from run to run at any B: the samples of a row are grouped by a stable radix sort and added in
+ * ascending sample order by the row's only writer.  Xa / Xb and the outputs are 16-byte aligned, D % 4 == 0; dXa and dXb
+ * may be two halves of one buffer.  scratch [dev]: recad_pair_scores_backward_scratch_bytes(B) bytes.  Synchronises the
+ * stream: an id outside its table gives RECAD_ERR_ARG (no memory outside the tables is addressed; the outputs are then
+ * unspecified). */
+int64_t recad_pair_scores_backward_scratch_bytes(int64_t B);
+int recad_pair_scores_backward(const float* Xa, int64_t n_a, const float* Xb, int64_t n_b, int32_t D, const int64_t* ia,
+                               const int64_t* ib, int64_t B, const float* g, float* dXa, float* dXb, float* dba, float* dbb,
+                               void* scratch, int64_t scratch_bytes, void* stream);
+
+/* Backward of recad_lightgcn_propagate: gE [dev] float[N, D] = (1 / (L + 1)) sum_l (A^T)^l gO for gO [dev] float[N, D]
+ * (A^T = st->graph_t when set, else st->graph), by the Horner loop of the epoch driver.  Reads st->graph / graph_t,
+ * n_users, n_items, D, n_layers; uses X0 (L >= 2) and X1 (L >= 3) as work; E, O, g, cnt, m, v and loss_acc are not
+ * touched, so a caller may pass a copy of its state with work buffers of its own. */
+int recad_lightgcn_backward(const recad_lightgcn* st, const float* gO, float* gE, void* stream);
+
+/* ------------------------------------------------------------------------ *
  * MF pointwise BCE step  (recad/model/victim/mf.py:40-69)
  * ------------------------------------------------------------------------ */
 typedef struct recad_mf {
@@ -495,6 +519,13 @@ int64_t recad_ncf_graph_launches(void);
 /* The gradient half of ONE step (ncf.py:139-148): as recad_mf_grad, into st->grads (layout of recad_ncf_layout). */
 int recad_ncf_grad(const recad_ncf* st, const int64_t* samples, const int64_t* perm, int64_t B, int64_t B_norm,
                    void* stream);
+/* Backward of recad_ncf_forward for an upstream gradient dpred [dev] float[B] (autograd): grads [dev] float[n_params]
+ * (layout of recad_ncf_layout, written whole) = sum_b dpred[b] d pred[b] / d params over the pairs (users[b], items[b]),
+ * B <= max_batch.  The forward is recomputed in the model's tower precision; st->grads, st->m, st->v and st->loss_acc
+ * are not touched.  The embedding rows are added in ascending sample order (bit-stable) for B <= 8192.  Synchronises the
+ * stream: an id out of range gives RECAD_ERR_ARG (no memory outside the tables is addressed). */
+int recad_ncf_backward(const recad_ncf* st, const int64_t* users, const int64_t* items, int64_t B, const float* dpred,
+                       float* grads, void* stream);
 
 /* The tensor-core GEMM of the NCF tower, exposed for testing: C[M, N] = A[M, K] . B[N, K]^T (+ bias[N]) (ReLU) on
  * tcgen05 (kind::tf32, fp32 accumulators in TMEM, TMA operands) with the 3xTF32 operand split, i.e. fp32-accurate.

@@ -129,6 +129,9 @@ SIGNATURES = {
     "recad_aush_generate": (C.c_int, [C.POINTER(Aush), vp, vp, i64, vp, vp]),
     "recad_mt19937_aush_batch": (C.c_int, [vp, C.POINTER(i32), i64, vp, vp, vp, vp, i32, i32, vp, C.c_double, vp, vp, vp]),
     "recad_dot_scores": (C.c_int, [vp, i64, vp, vp, i64, i32, vp, vp]),
+    "recad_pair_scores_backward_scratch_bytes": (i64, [i64]),
+    "recad_pair_scores_backward": (C.c_int, [vp, i64, vp, i64, i32, vp, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp]),
+    "recad_lightgcn_backward": (C.c_int, [C.POINTER(LightGCN), vp, vp, vp]),
     "recad_mf_forward": (C.c_int, [C.POINTER(MF), vp, vp, i64, vp, vp]),
     "recad_mf_train_epoch": (C.c_int, [C.POINTER(MF), vp, vp, i64, i64, i64, vp]),
     "recad_mf_grad": (C.c_int, [C.POINTER(MF), vp, vp, i64, i64, vp]),
@@ -142,6 +145,7 @@ SIGNATURES = {
     "recad_ncf_train_epoch": (C.c_int, [C.POINTER(NCF), vp, vp, i64, i64, i64, vp]),
     "recad_ncf_graph_launches": (i64, []),
     "recad_ncf_grad": (C.c_int, [C.POINTER(NCF), vp, vp, i64, i64, vp]),
+    "recad_ncf_backward": (C.c_int, [C.POINTER(NCF), vp, vp, i64, vp, vp, vp]),
     "recad_gemm_tn_tf32x3": (C.c_int, [vp, vp, i32, i32, i32, vp, i32, vp, vp, vp]),
     "recad_transpose_items": (C.c_int, [vp, i64, i32, vp, i64, vp]),
     "recad_fullrank_eval": (C.c_int, [vp, vp, i64, i64, i32, vp, i64, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp]),

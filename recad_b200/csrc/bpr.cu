@@ -351,6 +351,82 @@ __global__ void dot_scores_kernel(const float* __restrict__ O, int64_t n_users, 
   if (lane == 0) out[b] = acc;
 }
 
+// ------------------------------------------------------------------------------------------
+// Backward of pair scores s_b = <Xa[ia_b], Xb[ib_b]> (+ ba[ia_b] + bb[ib_b]) for an upstream gradient g, atomic-free.
+// One side at a time: key_b = ia_b << bbits | b, stably radix-sorted, groups the samples of a row in ascending sample
+// order; the warp of a group's first key is the row's only writer and adds g_b Xb[ib_b] over the group with plain stores.
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+pair_keys_kernel(const int64_t* __restrict__ ids, int64_t n_rows, int64_t B, int bbits, uint64_t* __restrict__ keys,
+                 int* __restrict__ bad) {
+  for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (int64_t)gridDim.x * blockDim.x) {
+    int64_t id = ids[b];
+    if (id < 0 || id >= n_rows) { atomicOr(bad, 1); id = 0; }
+    keys[b] = ((uint64_t)id << bbits) | (uint64_t)b;
+  }
+}
+
+// one warp per sorted key; the warp of a row's first key writes dX[row] (and db[row]), every other warp returns
+__global__ void __launch_bounds__(256)
+pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, const float* __restrict__ g,
+                      const int64_t* __restrict__ other, int64_t n_other, const float* __restrict__ X, int nvec,
+                      float* __restrict__ dX, float* __restrict__ db) {
+  const int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (k >= B) return;
+  const uint64_t row = keys[k] >> bbits;
+  if (k > 0 && (keys[k - 1] >> bbits) == row) return;
+  const uint64_t bmask = (1ull << bbits) - 1;
+  const float4* __restrict__ X4 = reinterpret_cast<const float4*>(X);
+  float4* __restrict__ dX4 = reinterpret_cast<float4*>(dX);
+  for (int c0 = 0; c0 < nvec; c0 += 32) {
+    const int c = c0 + lane;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    float gsum = 0.f;
+    for (int64_t j = k; j < B; ++j) {
+      const uint64_t key = keys[j];
+      if ((key >> bbits) != row) break;
+      const int64_t b = (int64_t)(key & bmask);
+      int64_t o = other[b];
+      if (o < 0 || o >= n_other) o = 0;            // reported by the other side's key pass
+      const float gv = g[b];
+      gsum += gv;
+      if (c < nvec) {
+        const float4 x = __ldg(X4 + o * nvec + c);
+        acc.x += gv * x.x; acc.y += gv * x.y; acc.z += gv * x.z; acc.w += gv * x.w;
+      }
+    }
+    if (c < nvec) dX4[(int64_t)row * nvec + c] = acc;
+    if (c0 == 0 && lane == 0 && db) db[row] = gsum;
+  }
+}
+
+static int64_t align256(int64_t x) { return (x + 255) / 256 * 256; }
+
+static int bit_width(int64_t n) {     // bits needed for the values 0 .. n - 1 (at least 1)
+  int b = 1;
+  while (b < 63 && ((int64_t)1 << b) < n) ++b;
+  return b;
+}
+
+// Horner: t <- g + A t, L times, so that t = (I + A + ... + A^L) g, over graph_t when set.  The last step is scaled by
+// alpha and lands in `out`; out == nullptr: it lands in the X0 / X1 ping-pong buffer of its parity.  *res = the result.
+static int lightgcn_horner(const recad_lightgcn* st, const float* g, float alpha, float* out, const float** res,
+                           void* stream) {
+  const recad_csr* A = st->graph_t ? st->graph_t : st->graph;
+  const int L = st->n_layers;
+  const float* t = g;
+  for (int k = 0; k < L; ++k) {
+    const bool last = k == L - 1;
+    float* z = (last && out) ? out : ((k & 1) ? st->X1 : st->X0);
+    const int rc = recad_spmm(A, t, nullptr, g, z, last ? alpha : 1.0f, st->D, stream);
+    if (rc) return rc;
+    t = z;
+  }
+  *res = t;
+  return RECAD_OK;
+}
+
 static int check_lightgcn(const recad_lightgcn* st) {
   RECAD_REQUIRE(st && st->graph, RECAD_ERR_ARG, "lightgcn: null state");
   RECAD_REQUIRE(st->n_users > 0 && st->n_items > 0 && st->graph->n_rows == st->n_users + st->n_items, RECAD_ERR_ARG,
@@ -433,14 +509,10 @@ static int lightgcn_train_epoch_t(const recad_lightgcn* st, const IdxT* samples,
     rc = launch_bpr(st->O, st->E, st->n_users, st->n_items, perm ? samples : samples + 3 * b0, perm ? perm + b0 : (const IdxT*)nullptr, B, B,
                     1.0f / (float)(L + 1), st->g, st->cnt, st->loss_acc, D, reinterpret_cast<int*>(st->loss_acc + 3), s);
     if (rc) return rc;
-    // Horner: t <- g + A t, L times, so that t = (I + A + ... + A^L) g
-    const float* t = st->g;
-    for (int k = 0; k < L; ++k) {
-      float* z = (k & 1) ? st->X1 : st->X0;
-      rc = recad_spmm(st->graph_t ? st->graph_t : st->graph, t, nullptr, st->g, z, 1.0f, D, stream);
-      if (rc) return rc;
-      t = z;
-    }
+    // g already carries the 1 / (L + 1) of the layer mean (BPR's grad_scale)
+    const float* t = nullptr;
+    rc = lightgcn_horner(st, st->g, 1.0f, nullptr, &t, stream);
+    if (rc) return rc;
     LossFold fold{st->loss_acc, 1.0 / (double)B, 0.5 * (double)st->lambda};
     rc = launch_adam(st->E, t, st->cnt, st->lambda / (float)B, st->m, st->v, N * D, D,
                      adam_scalars(st->lr, st->beta1, st->beta2, st->eps, step), fold, s);
@@ -514,6 +586,71 @@ int recad_dot_scores(const float* O, int64_t n_users, const int64_t* users, cons
   dot_scores_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, as_stream(stream)>>>(O, n_users, users, items, B, D / 4, scores);
   RECAD_LAUNCH_CHECK();
   return RECAD_OK;
+}
+
+int64_t recad_pair_scores_backward_scratch_bytes(int64_t B) {
+  if (B < 0) return -1;
+  return 2 * align256(B * 8) + align256(sort_scratch_bytes(B)) + 256;
+}
+
+int recad_pair_scores_backward(const float* Xa, int64_t n_a, const float* Xb, int64_t n_b, int32_t D, const int64_t* ia,
+                               const int64_t* ib, int64_t B, const float* g, float* dXa, float* dXb, float* dba, float* dbb,
+                               void* scratch, int64_t scratch_bytes, void* stream) {
+  RECAD_REQUIRE(Xa && Xb && dXa && dXb && n_a > 0 && n_b > 0 && B >= 0 && (B == 0 || (ia && ib && g && scratch)),
+                RECAD_ERR_ARG, "pair_scores_backward: bad argument");
+  RECAD_REQUIRE(D >= 4 && D % 4 == 0 && D <= 1024, RECAD_ERR_UNSUPPORTED, "pair_scores_backward: D must be a multiple of 4 in [4, 1024]");
+  RECAD_REQUIRE(n_a < ((int64_t)1 << 31) && n_b < ((int64_t)1 << 31) && B < ((int64_t)1 << 32) - 1, RECAD_ERR_OVERFLOW,
+                "pair_scores_backward: tables below 2^31 rows and B below 2^32 - 1");
+  RECAD_REQUIRE(B == 0 || scratch_bytes >= recad_pair_scores_backward_scratch_bytes(B), RECAD_ERR_SCRATCH,
+                "pair_scores_backward: scratch too small");
+  cudaStream_t s = as_stream(stream);
+  RECAD_CUDA_CHECK(cudaMemsetAsync(dXa, 0, n_a * D * sizeof(float), s));
+  RECAD_CUDA_CHECK(cudaMemsetAsync(dXb, 0, n_b * D * sizeof(float), s));
+  if (dba) RECAD_CUDA_CHECK(cudaMemsetAsync(dba, 0, n_a * sizeof(float), s));
+  if (dbb) RECAD_CUDA_CHECK(cudaMemsetAsync(dbb, 0, n_b * sizeof(float), s));
+  if (B == 0) return RECAD_OK;
+  char* p = static_cast<char*>(scratch);
+  uint64_t* keys = reinterpret_cast<uint64_t*>(p);    p += align256(B * 8);
+  uint64_t* tmp = reinterpret_cast<uint64_t*>(p);     p += align256(B * 8);
+  void* sort_scr = p;                                 p += align256(sort_scratch_bytes(B));
+  int* bad = reinterpret_cast<int*>(p);
+  RECAD_CUDA_CHECK(cudaMemsetAsync(bad, 0, sizeof(int), s));
+  const int bbits = bit_width(B);
+  const unsigned kgrid = (unsigned)std::min<int64_t>((B + 255) / 256, (int64_t)sm_count() * 16);
+  const unsigned wgrid = (unsigned)((B * 32 + 255) / 256);
+  for (int side = 0; side < 2; ++side) {
+    const int64_t n_rows = side == 0 ? n_a : n_b, n_other = side == 0 ? n_b : n_a;
+    const int64_t* ids = side == 0 ? ia : ib;
+    pair_keys_kernel<<<kgrid, 256, 0, s>>>(ids, n_rows, B, bbits, keys, bad);
+    RECAD_LAUNCH_CHECK();
+    int rc = radix_sort_u64(keys, tmp, B, bbits + bit_width(n_rows), sort_scr, s);
+    if (rc) return rc;
+    pair_grad_rows_kernel<<<wgrid, 256, 0, s>>>(keys, B, bbits, g, side == 0 ? ib : ia, n_other, side == 0 ? Xb : Xa, D / 4,
+                                                side == 0 ? dXa : dXb, side == 0 ? dba : dbb);
+    RECAD_LAUNCH_CHECK();
+  }
+  int h_bad = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "pair_scores_backward: an id is out of range");
+  return RECAD_OK;
+}
+
+int recad_lightgcn_backward(const recad_lightgcn* st, const float* gO, float* gE, void* stream) {
+  RECAD_REQUIRE(st && st->graph && gO && gE && gO != gE, RECAD_ERR_ARG, "lightgcn_backward: bad argument");
+  RECAD_REQUIRE(st->n_users > 0 && st->n_items > 0 && st->graph->n_rows == st->n_users + st->n_items &&
+                    (!st->graph_t || st->graph_t->n_rows == st->graph->n_rows),
+                RECAD_ERR_ARG, "lightgcn_backward: graph shape");
+  RECAD_REQUIRE(st->D >= 4 && st->D % 4 == 0 && st->n_layers >= 0, RECAD_ERR_UNSUPPORTED, "lightgcn_backward: bad D / layers");
+  RECAD_REQUIRE((st->n_layers < 2 || st->X0) && (st->n_layers < 3 || st->X1), RECAD_ERR_ARG,
+                "lightgcn_backward: null work buffer");
+  const int64_t N = st->n_users + st->n_items;
+  if (st->n_layers == 0) {
+    RECAD_CUDA_CHECK(cudaMemcpyAsync(gE, gO, N * st->D * sizeof(float), cudaMemcpyDeviceToDevice, as_stream(stream)));
+    return RECAD_OK;
+  }
+  const float* t = nullptr;
+  return lightgcn_horner(st, gO, 1.0f / (float)(st->n_layers + 1), gE, &t, stream);
 }
 
 }  // extern "C"

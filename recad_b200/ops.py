@@ -9,6 +9,7 @@ import os
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import RecadError, check
@@ -397,6 +398,172 @@ def dot_scores(O, n_users, users, items):
         check(_lib.lib().recad_dot_scores(_ptr(O), n_users, _ptr(users), _ptr(items), users.numel(), O.shape[1], _ptr(out),
                                           _stream(O.device)), "recad_dot_scores")
     return out
+
+
+def mf_forward(st, users, items):
+    """recad_mf_forward over the tables of an MF state: <Ue[u], Ie[i]> + Ub[u] + Ib[i] + mean."""
+    dev = users.device
+    out = torch.empty(users.numel(), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        check(_lib.lib().recad_mf_forward(C.byref(st), _ptr(users), _ptr(items), users.numel(), _ptr(out), _stream(dev)),
+              "recad_mf_forward")
+    return out
+
+
+def ncf_forward(st, users, items):
+    """recad_ncf_forward in slices of st.max_batch pairs."""
+    dev = users.device
+    n = users.numel()
+    out = torch.empty(n, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        for s in range(0, n, st.max_batch):
+            e = min(s + st.max_batch, n)
+            check(_lib.lib().recad_ncf_forward(C.byref(st), _ptr(users[s:e]), _ptr(items[s:e]), e - s, _ptr(out[s:e]), _stream(dev)),
+                  "recad_ncf_forward")
+    return out
+
+
+# --------------------------------------------------------------------------- #
+# autograd: backward passes of the victims' scores
+# --------------------------------------------------------------------------- #
+def pair_scores_backward(Xa, Xb, ia, ib, g, bias=False):
+    """Gradient of s_b = <Xa[ia_b], Xb[ib_b]> (+ ba[ia_b] + bb[ib_b]) for the upstream gradient g (recad_pair_scores_backward):
+    (dX [n_a + n_b, D] with the rows of Xa first, dba [n_a], dbb [n_b]); the bias gradients are None unless `bias`.
+    Atomic-free: the same bits on every run at any batch size.  An id out of range raises RecadError."""
+    _need_cuda(Xa, Xb, ia, ib, g)
+    dev = Xa.device
+    (n_a, D), n_b, B = Xa.shape, Xb.shape[0], ia.numel()
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        dX = torch.empty((n_a + n_b, D), dtype=torch.float32, device=dev)
+        dba = torch.empty(n_a, dtype=torch.float32, device=dev) if bias else None
+        dbb = torch.empty(n_b, dtype=torch.float32, device=dev) if bias else None
+        nbytes = int(L.recad_pair_scores_backward_scratch_bytes(B))
+        scratch = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+        check(L.recad_pair_scores_backward(_ptr(Xa), n_a, _ptr(Xb), n_b, D, _ptr(ia), _ptr(ib), B, _ptr(g), _ptr(dX[:n_a]),
+                                           _ptr(dX[n_a:]), _ptr(dba), _ptr(dbb), _ptr(scratch), nbytes, _stream(dev)),
+              "recad_pair_scores_backward")
+    return dX, dba, dbb
+
+
+def lightgcn_backward(st, gO):
+    """gE = (1 / (L + 1)) sum_l (A^T)^l gO (recad_lightgcn_backward) for a LightGCN state; the Horner loop runs through work
+    buffers of its own, so the state's X0 / X1 are left alone."""
+    _need_cuda(gO)
+    dev = gO.device
+    with torch.cuda.device(dev):
+        gE = torch.empty_like(gO)
+        work = [torch.empty_like(gO) for _ in range(min(max(st.n_layers - 1, 0), 2))]
+        sb = _lib.LightGCN()
+        C.memmove(C.byref(sb), C.byref(st), C.sizeof(sb))
+        sb.X0 = work[0].data_ptr() if len(work) > 0 else None
+        sb.X1 = work[1].data_ptr() if len(work) > 1 else None
+        check(_lib.lib().recad_lightgcn_backward(C.byref(sb), _ptr(gO), _ptr(gE), _stream(dev)), "recad_lightgcn_backward")
+    return gE
+
+
+def ncf_backward(st, users, items, dpred):
+    """Flat gradient (recad_ncf_layout order) of sum_b dpred[b] pred[b] for an NCF state (recad_ncf_backward), in slices of
+    st.max_batch pairs."""
+    _need_cuda(users, items, dpred)
+    dev = dpred.device
+    n = users.numel()
+    with torch.cuda.device(dev):
+        grads = torch.empty(st.n_params, dtype=torch.float32, device=dev)
+        part = torch.empty_like(grads) if n > st.max_batch else None
+        for s in range(0, n, st.max_batch):
+            e = min(s + st.max_batch, n)
+            dst = grads if s == 0 else part
+            check(_lib.lib().recad_ncf_backward(C.byref(st), _ptr(users[s:e]), _ptr(items[s:e]), e - s, _ptr(dpred[s:e]), _ptr(dst),
+                                                _stream(dev)), "recad_ncf_backward")
+            if s:
+                grads += part
+    return grads
+
+
+class LightGCNPropagate(torch.autograd.Function):
+    """O = mean_l A^l E (lightgcn.py:82-113) into a fresh [N, D] buffer; backward by recad_lightgcn_backward.  graph_t /
+    vals_t: the transposed matrix of a dropped graph and the values this propagation drew for it -- restored before the
+    backward, so that it uses this forward's mask even if a later forward drew another."""
+
+    @staticmethod
+    def forward(ctx, st, graph_t, vals_t, user_w, item_w):
+        N = st.n_users + st.n_items
+        dev = user_w.device
+        with torch.cuda.device(dev):
+            O = torch.empty((N, st.D), dtype=torch.float32, device=dev)
+            sf = _lib.LightGCN()
+            C.memmove(C.byref(sf), C.byref(st), C.sizeof(sf))
+            sf.O = O.data_ptr()
+            check(_lib.lib().recad_lightgcn_propagate(C.byref(sf), _stream(dev)), "recad_lightgcn_propagate")
+        ctx.st, ctx.graph_t, ctx.vals_t = sf, graph_t, vals_t
+        return O
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gO):
+        if ctx.graph_t is not None:
+            ctx.graph_t.set_values(ctx.vals_t)
+        gE = lightgcn_backward(ctx.st, gO.contiguous())
+        U = ctx.st.n_users
+        return None, None, None, gE[:U], gE[U:]
+
+
+class DotScores(torch.autograd.Function):
+    """scores[b] = <O[users[b]], O[n_users + items[b]]> (lightgcn.py:174-183); backward by recad_pair_scores_backward."""
+
+    @staticmethod
+    def forward(ctx, O, n_users, users, items):
+        ctx.save_for_backward(O, users, items)
+        ctx.n_users = n_users
+        return dot_scores(O, n_users, users, items)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        O, users, items = ctx.saved_tensors
+        U = ctx.n_users
+        dO, _, _ = pair_scores_backward(O[:U], O[U:], users, items, g.contiguous().float())
+        return dO, None, None, None
+
+
+class MFScores(torch.autograd.Function):
+    """pred = <Ue[u], Ie[i]> + Ub[u] + Ib[i] + mean (mf.py:40-47) over the tables of an MF state (the four tables and mean are
+    passed so that autograd routes their gradients); backward by recad_pair_scores_backward."""
+
+    @staticmethod
+    def forward(ctx, st, users, items, Ue, Ub, Ie, Ib, mean):
+        ctx.save_for_backward(users, items, Ue, Ie)
+        return mf_forward(st, users, items)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        users, items, Ue, Ie = ctx.saved_tensors
+        U, I = Ue.shape[0], Ie.shape[0]
+        g = g.contiguous().float()
+        dX, dUb, dIb = pair_scores_backward(Ue, Ie, users, items, g, bias=True)
+        dmean = g.sum().view(1) if ctx.needs_input_grad[7] else None
+        return None, None, None, dX[:U], dUb.view(U, 1), dX[U:], dIb.view(I, 1), dmean
+
+
+class NCFScores(torch.autograd.Function):
+    """pred = NCF(users, items) (ncf.py:112-131) over the flat parameter buffer of an NCF state; `params` are the parameter
+    views in recad_ncf_layout order at float offsets `offs`, so that autograd routes the flat gradient back onto them."""
+
+    @staticmethod
+    def forward(ctx, st, offs, users, items, *params):
+        ctx.st, ctx.offs = st, offs
+        ctx.save_for_backward(users, items, *params)     # the backward recomputes the forward: in-place edits must fail it
+        return ncf_forward(st, users, items)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        users, items = ctx.saved_tensors[:2]
+        flat = ncf_backward(ctx.st, users, items, g.contiguous().float())
+        grads = tuple(flat[o:o + n].view(s) for o, n, s in ctx.offs)
+        return (None, None, None, None) + grads
 
 
 # --------------------------------------------------------------------------- #

@@ -89,6 +89,19 @@ class BaseVictim(LazyMixin, torch.nn.Module):
             raise ops.RecadError(f"{type(self).__name__}.train_step: a sample id is out of range")
         return (float(acc[2]) / n_batches,)
 
+    def _graph_mode(self):
+        """Autograd applies to this call (the usual torch rule): grad mode is on and a parameter requires a gradient.
+        Otherwise the victim runs its plain kernels and returns tensors without a grad_fn."""
+        return torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
+
+    @staticmethod
+    def _check_ids(users, n_users, items, n_items):
+        """RecadError unless every id lies inside its table (one device->host copy)."""
+        if users.numel() != items.numel():
+            raise ops.RecadError(f"{users.numel()} users but {items.numel()} items")
+        if users.numel() and bool(((users < 0) | (users >= n_users)).any() | ((items < 0) | (items >= n_items)).any()):
+            raise ops.RecadError("a user or item id is out of range")
+
     @staticmethod
     def _vp(t):
         return C.c_void_p(t.data_ptr()) if t is not None else None

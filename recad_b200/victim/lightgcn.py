@@ -95,6 +95,7 @@ class LightGCN(BaseVictim):
         self._st = st
         self._drop_graph = self._drop_graph_t = self._st_drop = None
         self._O_valid = False      # O was just (re)allocated: never score from it before a propagate
+        self._O_version = -1
 
     def load_state_dict(self, *args, **kwargs):
         out = super().load_state_dict(*args, **kwargs)
@@ -116,12 +117,13 @@ class LightGCN(BaseVictim):
             self._alloc(dev, self.E[:self.num_users], self.E[self.num_users:], self.m, self.v)
 
     # ------------------------------------------------------------------ graph dropout
-    def _dropped_state(self):
+    def _dropped_state(self, with_vals_t=False):
         """lightgcn.py:62-80 `__dropout_x`: keep an entry when int(rand + keep_prob) is 1, rescale the kept values by
         1 / keep_prob.  The mask is drawn exactly as the reference draws it -- torch.rand(nnz) on the CPU generator, in the
         coalesced (row-major) entry order, which is the CSR order -- so a seeded run drops the same entries.  Dropped
         entries keep their place in the structure with value 0 (the plan and both SpMM directions are unchanged): the
-        state returned is this model's with the graph swapped for that matrix."""
+        state returned is this model's with the graph swapped for that matrix (and, with_vals_t, the transposed values,
+        which an autograd backward restores)."""
         g = self.Graph
         keep = (torch.rand(g.nnz) + self.keep_prob).int().bool()
         with torch.cuda.device(self._dev):
@@ -140,18 +142,39 @@ class LightGCN(BaseVictim):
             else:
                 self._drop_graph.set_values(vals)
                 self._drop_graph_t.set_values(vals_t)
-        return self._st_drop
+        return (self._st_drop, vals_t) if with_vals_t else self._st_drop
 
     # ------------------------------------------------------------------ compute
+    def _propagate_graph(self):
+        """The propagation as an autograd node: a fresh [N, D] output differentiable with respect to both tables."""
+        if self.dropout and self.training:
+            st, vals_t = self._dropped_state(with_vals_t=True)
+            graph_t = self._drop_graph_t
+        else:
+            st, graph_t, vals_t = self._st, None, None
+        return ops.LightGCNPropagate.apply(st, graph_t, vals_t, self.embedding_user.weight, self.embedding_item.weight)
+
+    def _cached_O(self):
+        """self.O, propagated again unless it is current: the tables have not changed since (train_step, load_state_dict,
+        in-place updates such as a torch optimizer's step, which bump the tables' version) and no dropout mask applies."""
+        if not self._O_valid or self._O_version != self.E._version or (self.dropout and self.training):
+            self.computer()
+        return self.O
+
     def computer(self):
         """lightgcn.py:82-113: (users, items) propagated embeddings = mean of the layer outputs (over a freshly dropped
-        graph when dropout is on and the module is in training mode)."""
+        graph when dropout is on and the module is in training mode).  Differentiable with respect to the two tables when
+        grad mode is on and one of them requires a gradient."""
         self._require_instance("computer")
+        if self._graph_mode():
+            O = self._propagate_graph()
+            return O[:self.num_users], O[self.num_users:]
         dropped = self.dropout and self.training
         st = self._dropped_state() if dropped else self._st
         with torch.cuda.device(self._dev):
             self._check(_lib.lib().recad_lightgcn_propagate(C.byref(st), ops._stream(self._dev)), "recad_lightgcn_propagate")
         self._O_valid = not dropped      # a dropped propagation is never reused: the next call draws a new mask
+        self._O_version = self.E._version
         return self.O[:self.num_users], self.O[self.num_users:]
 
     def getUsersRating(self, users):
@@ -206,21 +229,24 @@ class LightGCN(BaseVictim):
 
     def forward(self, users, items):
         """lightgcn.py:174-183: <O_u, O_i>.  The propagation is redone only when the tables changed
-        (the reference redoes it on every call, i.e. once per evaluated user)."""
+        (the reference redoes it on every call, i.e. once per evaluated user).  In autograd (grad mode on and a table
+        that requires a gradient) every call propagates again, as the reference does, and the scores are differentiable
+        with respect to both tables."""
         self._require_instance("forward")
-        if not self._O_valid or (self.dropout and self.training):
-            self.computer()
         users = users.to(self._dev).long().contiguous()
         items = items.to(self._dev).long().contiguous()
-        return ops.dot_scores(self.O, self.num_users, users, items)
+        if self._graph_mode():
+            self._check_ids(users, self.num_users, items, self.num_items)
+            return ops.DotScores.apply(self._propagate_graph(), self.num_users, users, items)
+        return ops.dot_scores(self._cached_O(), self.num_users, users, items)
 
     def full_rank(self, user_ids, targets, K, train_rowptr, train_col):
         """Batched evaluation entry used by recad_b200.evaluate (fused score/mask/top-K kernel)."""
         self._require_instance("full_rank")
-        if not self._O_valid or (self.dropout and self.training):
-            self.computer()
+        with torch.no_grad():
+            O = self._cached_O()
         U = self.num_users
-        return ops.fullrank_eval(self.O[:U], self.O[U:], user_ids, train_rowptr, train_col, targets, K) + (0.0,)
+        return ops.fullrank_eval(O[:U], O[U:], user_ids, train_rowptr, train_col, targets, K) + (0.0,)
 
     def input_describe(self):
         return {

@@ -59,6 +59,7 @@ class MF(BaseVictim):
         self.item_emb = nn.Embedding(I, D, _weight=Ie.view(I, D))
         self.item_bias = nn.Embedding(I, 1, _weight=Ib.view(I, 1))
         self.mean = nn.Parameter(torch.tensor([self.mean_value], device=dev), False)
+        self._mean_version = self.mean._version
         for p in self.parameters():
             p.requires_grad_(False)
         self.optimizer = None
@@ -78,16 +79,26 @@ class MF(BaseVictim):
             self._alloc(dev, [self.user_emb.weight.data, self.user_bias.weight.data, self.item_emb.weight.data,
                               self.item_bias.weight.data], self.m, self.v)
 
+    def _sync_mean(self):
+        """The kernels read `mean` from the state: take over an in-place update of the parameter (a torch optimizer's step
+        once the user made it trainable)."""
+        if self.mean._version != self._mean_version:
+            self.mean_value = float(self.mean.detach().view(-1)[0])
+            self._st.mean = self.mean_value
+            self._mean_version = self.mean._version
+
     def forward(self, users, items):
-        """mf.py:40-47."""
+        """mf.py:40-47.  Differentiable with respect to the four tables (and `mean` once it requires a gradient) when grad
+        mode is on and a parameter requires a gradient."""
         self._require_instance("forward")
         users = users.to(self._dev).long().contiguous()
         items = items.to(self._dev).long().contiguous()
-        out = torch.empty(users.numel(), dtype=torch.float32, device=self._dev)
-        with torch.cuda.device(self._dev):
-            self._check(_lib.lib().recad_mf_forward(C.byref(self._st), self._vp(users), self._vp(items), users.numel(),
-                                                    self._vp(out), ops._stream(self._dev)), "recad_mf_forward")
-        return out
+        self._sync_mean()
+        if self._graph_mode():
+            self._check_ids(users, self.num_users, items, self.num_items)
+            return ops.MFScores.apply(self._st, users, items, self.user_emb.weight, self.user_bias.weight, self.item_emb.weight,
+                                      self.item_bias.weight, self.mean)
+        return ops.mf_forward(self._st, users, items)
 
     def train_step(self, **config):
         """One epoch (mf.py:49-69): returns (mean batch loss,)."""
@@ -113,10 +124,12 @@ class MF(BaseVictim):
         """score = <U_u, V_i> + b_i (+ b_u + mean, constant per user): the item bias is added inside the
         fused full-rank kernel, the per-user constants afterwards."""
         self._require_instance("full_rank")
-        topi, topv, rank, score = ops.fullrank_eval(self.user_emb.weight, self.item_emb.weight, user_ids, train_rowptr,
-                                                    train_col, targets, K, item_bias=self.item_bias.weight.view(-1))
-        # b_u and the mean shift every score of a user equally: they never change a rank, only the reported score
-        score = score + self.user_bias.weight.view(-1)[user_ids].unsqueeze(1)
+        self._sync_mean()
+        with torch.no_grad():
+            topi, topv, rank, score = ops.fullrank_eval(self.user_emb.weight, self.item_emb.weight, user_ids, train_rowptr,
+                                                        train_col, targets, K, item_bias=self.item_bias.weight.view(-1))
+            # b_u and the mean shift every score of a user equally: they never change a rank, only the reported score
+            score = score + self.user_bias.weight.view(-1)[user_ids].unsqueeze(1)
         return topi, topv, rank, score, self.mean_value
 
     def input_describe(self):

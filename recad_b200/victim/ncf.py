@@ -114,6 +114,7 @@ class NCF(BaseVictim):
             vw = self.flat[off:off + src.numel()].view(src.shape)
             vw.copy_(src)
             views.append(vw)
+        self._grad_slots = tuple((off, src.numel(), src.shape) for off, src in zip(offs[:-1], pieces))
         U, I, f, w = self.num_users, self.num_items, self.f, self.f * (2 ** (self.L - 1))
         self.embed_user_GMF = nn.Embedding(U, f, _weight=views[0])
         self.embed_item_GMF = nn.Embedding(I, f, _weight=views[1])
@@ -137,13 +138,16 @@ class NCF(BaseVictim):
         st.work, st.work_floats, st.max_batch, st.loss_acc = self.work.data_ptr(), work_floats, self.max_batch, self.loss_acc.data_ptr()
         self._st = st
 
-    def _pieces(self):
-        out = [self.embed_user_GMF.weight.data, self.embed_item_GMF.weight.data, self.embed_user_MLP.weight.data,
-               self.embed_item_MLP.weight.data]
+    def _param_views(self):
+        """The parameters in recad_ncf_layout order."""
+        out = [self.embed_user_GMF.weight, self.embed_item_GMF.weight, self.embed_user_MLP.weight, self.embed_item_MLP.weight]
         for mod in self.MLP_layers:
             if isinstance(mod, nn.Linear):
-                out += [mod.weight.data, mod.bias.data]
-        return out + [self.predict_layer.weight.data, self.predict_layer.bias.data]
+                out += [mod.weight, mod.bias]
+        return out + [self.predict_layer.weight, self.predict_layer.bias]
+
+    def _pieces(self):
+        return [p.data for p in self._param_views()]
 
     def _move(self, dev):
         if dev.index is None:
@@ -152,18 +156,15 @@ class NCF(BaseVictim):
             self._alloc(dev, [p.clone() for p in self._pieces()], self.m, self.v)
 
     def forward(self, user, item):
-        """ncf.py:112-131 (NeuMF-end)."""
+        """ncf.py:112-131 (NeuMF-end).  Differentiable with respect to every parameter when grad mode is on and a parameter
+        requires a gradient."""
         self._require_instance("forward")
         user = user.to(self._dev).long().contiguous()
         item = item.to(self._dev).long().contiguous()
-        n = user.numel()
-        out = torch.empty(n, dtype=torch.float32, device=self._dev)
-        with torch.cuda.device(self._dev):
-            for s in range(0, n, self.max_batch):
-                e = min(s + self.max_batch, n)
-                self._check(_lib.lib().recad_ncf_forward(C.byref(self._st), self._vp(user[s:e]), self._vp(item[s:e]), e - s,
-                                                         self._vp(out[s:e]), ops._stream(self._dev)), "recad_ncf_forward")
-        return out
+        if self._graph_mode():
+            self._check_ids(user, self.num_users, item, self.num_items)
+            return ops.NCFScores.apply(self._st, self._grad_slots, user, item, *self._param_views())
+        return ops.ncf_forward(self._st, user, item)
 
     def train_step(self, **config):
         """One epoch (ncf.py:133-153): returns (mean batch loss,)."""
@@ -233,7 +234,8 @@ class NCF(BaseVictim):
                 ub = user_ids[s:s + per]
                 uu = ub.repeat_interleave(I)
                 ii = all_items.repeat(ub.numel())
-                scores = self.forward(uu, ii).view(ub.numel(), I)
+                with torch.no_grad():
+                    scores = self.forward(uu, ii).view(ub.numel(), I)
                 outs.append(ops.rank_from_scores(scores, ub, train_rowptr, train_col, targets, K))
         return tuple(torch.cat([o[k] for o in outs]) for k in range(4)) + (0.0,)
 
