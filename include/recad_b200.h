@@ -89,6 +89,21 @@ int recad_csr_append_users(const int64_t* rowptr, const int32_t* colidx, const f
                            int32_t* new_degree, void* scratch, int64_t scratch_bytes, void* stream);
 int64_t recad_csr_append_scratch_bytes(int64_t n_users, int64_t n_items, int64_t n_fake, int64_t n_fake_edges);
 
+/* The weights -> values chain of the normalisation above for caller-supplied per-entry weights w [dev] float[nnz]
+ * (in place of mult):  vals_k = d_r w_k d_c,  d_r = (s_r + 1e-14)^(-1/2).
+ * recad_csr_row_sums: sums [dev] float[n_rows] = s_r, the weights of row r added in a fixed order in double and rounded
+ *   to float once (the host then evaluates d_inv from them, as from the degrees).
+ * recad_csr_normalize_backward: for a square, structurally symmetric matrix, the gradient gw [dev] float[nnz] of
+ *   sum_k gv_k vals_k:  gw_k = gv_k d_r d_c - 0.5 d_r^3 P_r,  P_r = sum over row r's entries k' of
+ *   (gv_k' w_k' + gv_{T k'} w_{T k'}) d_{c(k')}, where tperm [dev] int64[nnz] maps entry (r, c) to the position of (c, r).
+ *   Two passes: a per-row reduction into coef [dev] float[n_rows] (work) in a fixed order, then a per-entry epilogue;
+ *   deterministic.  d_inv [dev] float[n_rows] is the forward's.
+ * Both read rowptr[n_rows] back (synchronising the stream) and return RECAD_ERR_ARG unless it equals nnz. */
+int recad_csr_row_sums(const int64_t* rowptr, const float* w, int64_t n_rows, int64_t nnz, float* sums, void* stream);
+int recad_csr_normalize_backward(const int64_t* rowptr, const int32_t* colidx, const int64_t* tperm, const float* w,
+                                 const float* d_inv, const float* gv, int64_t n_rows, int64_t nnz, float* coef, float* gw,
+                                 void* stream);
+
 /* ------------------------------------------------------------------------ *
  * Propagation  (recad/model/victim/lightgcn.py:82-113 `computer`; its autograd
  * backward is the same product because A_hat is symmetric)
@@ -130,6 +145,13 @@ int recad_spmm_pack_cv(const int32_t* colidx, const float* vals, int64_t nnz, vo
  * Z = accumulated mean) and every Horner step of the backward (Z = g + A t). */
 int recad_spmm(const recad_csr* A, const float* X, float* Y, const float* C, float* Z,
                float alpha, int32_t D, void* stream);
+
+/* SDDMM, the gradient of an SpMM with respect to the matrix's values: out[k] = alpha * <G[r_k], X[c_k]> for every stored
+ * entry k = (r_k, c_k) of A (accumulate != 0: out[k] += ...).  G [dev] float[n_rows, D], X [dev] float[n_cols, D], 16-byte
+ * aligned; out [dev] float[nnz] in A's CSR entry order.  Driven by A's plan (reads seg_meta and colidx, not cv or vals);
+ * every entry has one writer: atomic-free and bit-stable.  Same bytes as one SpMM (no-reuse model). */
+int recad_csr_sddmm(const recad_csr* A, const float* G, const float* X, int32_t D, float alpha, int32_t accumulate,
+                    float* out, void* stream);
 
 /* Sharded path (SURVEY.md 8e): Y = A X where row i is not stored locally but written, as soon as it is
  * finished, to dst[i / slice_rows] + (i % slice_rows) * D.  dst[r] [host array of n_dst <= 16 device pointers]
@@ -427,6 +449,15 @@ int recad_pair_scores_backward(const float* Xa, int64_t n_a, const float* Xb, in
  * n_users, n_items, D, n_layers; uses X0 (L >= 2) and X1 (L >= 3) as work; E, O, g, cnt, m, v and loss_acc are not
  * touched, so a caller may pass a copy of its state with work buffers of its own. */
 int recad_lightgcn_backward(const recad_lightgcn* st, const float* gO, float* gE, void* stream);
+
+/* The same backward with respect to the values of st->graph as well:
+ *   gvals [dev] float[nnz] (st->graph's entry order) = (1 / (L + 1)) sum_{j < L} <t_j[r_k], X_{L-1-j}[c_k]>,
+ *   t_0 = gO, t_{j+1} = gO + A^T t_j (the Horner iterates; A^T = graph_t when set, which it must be unless the values are
+ *   symmetric), X [host] array of L device pointers to the forward's layers X_0 = E, X_1 = A E, .., X_{L-1}.
+ * One Horner loop: the SDDMM of step j (recad_csr_sddmm over st->graph) runs next to its SpMM.  gE as in
+ * recad_lightgcn_backward, or NULL (then the last SpMM is skipped).  L = 0: gvals = 0.  Work buffers as above. */
+int recad_lightgcn_backward_values(const recad_lightgcn* st, const float* gO, const float* const* X, float* gE, float* gvals,
+                                   void* stream);
 
 /* ------------------------------------------------------------------------ *
  * MF pointwise BCE step  (recad/model/victim/mf.py:40-69)

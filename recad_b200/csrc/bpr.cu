@@ -409,15 +409,33 @@ static int bit_width(int64_t n) {     // bits needed for the values 0 .. n - 1 (
   return b;
 }
 
+// Edge-value gradient riding on the Horner loop: at step k, before t_k's ping-pong buffer is written again,
+// gvals[e] (+)= scale * <t_k[r_e], X[L - 1 - k][c_e]> over the entries of st->graph (A's own entry order; k = 0 writes).
+struct HornerValues {
+  const float* const* X;   // host array of the L forward layers X_0 = E .. X_{L-1}
+  float* gvals;
+  float scale;
+};
+
 // Horner: t <- g + A t, L times, so that t = (I + A + ... + A^L) g, over graph_t when set.  The last step is scaled by
 // alpha and lands in `out`; out == nullptr: it lands in the X0 / X1 ping-pong buffer of its parity.  *res = the result.
+// hv: the SDDMM of each step on its t_k; with out == nullptr as well, the last SpMM (which gvals does not need) is skipped
+// and *res is nullptr.
 static int lightgcn_horner(const recad_lightgcn* st, const float* g, float alpha, float* out, const float** res,
-                           void* stream) {
+                           void* stream, const HornerValues* hv = nullptr) {
   const recad_csr* A = st->graph_t ? st->graph_t : st->graph;
   const int L = st->n_layers;
   const float* t = g;
   for (int k = 0; k < L; ++k) {
     const bool last = k == L - 1;
+    if (hv) {
+      const int rc = recad_csr_sddmm(st->graph, t, hv->X[L - 1 - k], st->D, hv->scale, k > 0, hv->gvals, stream);
+      if (rc) return rc;
+      if (last && !out) {
+        *res = nullptr;
+        return RECAD_OK;
+      }
+    }
     float* z = (last && out) ? out : ((k & 1) ? st->X1 : st->X0);
     const int rc = recad_spmm(A, t, nullptr, g, z, last ? alpha : 1.0f, st->D, stream);
     if (rc) return rc;
@@ -651,6 +669,31 @@ int recad_lightgcn_backward(const recad_lightgcn* st, const float* gO, float* gE
   }
   const float* t = nullptr;
   return lightgcn_horner(st, gO, 1.0f / (float)(st->n_layers + 1), gE, &t, stream);
+}
+
+int recad_lightgcn_backward_values(const recad_lightgcn* st, const float* gO, const float* const* X, float* gE, float* gvals,
+                                   void* stream) {
+  RECAD_REQUIRE(st && st->graph && gO && gvals && gO != gE, RECAD_ERR_ARG, "lightgcn_backward_values: bad argument");
+  RECAD_REQUIRE(st->n_users > 0 && st->n_items > 0 && st->graph->n_rows == st->n_users + st->n_items &&
+                    st->graph->n_cols == st->graph->n_rows &&
+                    (!st->graph_t || (st->graph_t->n_rows == st->graph->n_rows && st->graph_t->nnz == st->graph->nnz)),
+                RECAD_ERR_ARG, "lightgcn_backward_values: graph shape");
+  RECAD_REQUIRE(st->D >= 4 && st->D % 4 == 0 && st->n_layers >= 0, RECAD_ERR_UNSUPPORTED,
+                "lightgcn_backward_values: bad D / layers");
+  const int L = st->n_layers;
+  RECAD_REQUIRE((L < 2 || st->X0) && (L < 3 || st->X1), RECAD_ERR_ARG, "lightgcn_backward_values: null work buffer");
+  RECAD_REQUIRE(L == 0 || X, RECAD_ERR_ARG, "lightgcn_backward_values: null layer array");
+  for (int l = 0; l < L; ++l) RECAD_REQUIRE(X[l], RECAD_ERR_ARG, "lightgcn_backward_values: layer %d is null", l);
+  cudaStream_t s = as_stream(stream);
+  const int64_t N = st->n_users + st->n_items;
+  if (L == 0) {
+    if (st->graph->nnz) RECAD_CUDA_CHECK(cudaMemsetAsync(gvals, 0, st->graph->nnz * sizeof(float), s));
+    if (gE) RECAD_CUDA_CHECK(cudaMemcpyAsync(gE, gO, N * st->D * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return RECAD_OK;
+  }
+  const HornerValues hv{X, gvals, 1.0f / (float)(L + 1)};
+  const float* t = nullptr;
+  return lightgcn_horner(st, gO, 1.0f / (float)(L + 1), gE, &t, stream, &hv);
 }
 
 }  // extern "C"

@@ -113,6 +113,68 @@ __global__ void normalize_kernel(const int64_t* __restrict__ rowptr, const int32
 }
 
 // ------------------------------------------------------------------------------------------
+// weights -> values chain: vals_k = d_r w_k d_c, d_r = (s_r + 1e-14)^(-1/2), s_r = sum of row r's weights
+// ------------------------------------------------------------------------------------------
+// s_r: one warp per row, fixed order, double accumulator rounded to fp32 once
+__global__ void __launch_bounds__(256)
+row_sums_kernel(const int64_t* __restrict__ rowptr, const float* __restrict__ w, int64_t n_rows, float* __restrict__ sums) {
+  const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= n_rows) return;
+  const int64_t lo = rowptr[row], hi = rowptr[row + 1];
+  double acc = 0.0;
+  for (int64_t e = lo + lane; e < hi; e += 32) acc += (double)w[e];
+  acc = warp_sum(acc);
+  if (lane == 0) sums[row] = (float)acc;
+}
+
+// pass 1 of the backward, one warp per row: coef_r = -0.5 d_r^3 P_r with
+// P_r = sum over row r's entries k of (gv_k w_k + gv_{T k} w_{T k}) d_{c(k)} -- row r's own entries carry d_r as their row
+// factor, their transposes (the entries of column r) as their column factor
+__global__ void __launch_bounds__(256)
+norm_bwd_rows_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ colidx, const int64_t* __restrict__ tperm,
+                     const float* __restrict__ w, const float* __restrict__ d_inv, const float* __restrict__ gv, int64_t n_rows,
+                     float* __restrict__ coef) {
+  const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= n_rows) return;
+  const int64_t lo = rowptr[row], hi = rowptr[row + 1];
+  double acc = 0.0;
+  for (int64_t e = lo + lane; e < hi; e += 32) {
+    const int64_t t = tperm[e];
+    acc += ((double)gv[e] * (double)w[e] + (double)gv[t] * (double)w[t]) * (double)d_inv[colidx[e]];
+  }
+  acc = warp_sum(acc);
+  if (lane == 0) {
+    const double d = d_inv[row];
+    coef[row] = (float)(-0.5 * d * d * d * acc);
+  }
+}
+
+// pass 2, per entry: gw_k = gv_k d_r d_c + coef_r
+__global__ void __launch_bounds__(256)
+norm_bwd_entries_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ colidx, const float* __restrict__ d_inv,
+                        const float* __restrict__ gv, const float* __restrict__ coef, int64_t n_rows, int64_t nnz,
+                        float* __restrict__ gw) {
+  const int64_t e0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * kNormPerThread;
+  if (e0 >= nnz) return;
+  int64_t row = find_row(rowptr, n_rows, e0);
+  int64_t row_end = rowptr[row + 1];
+  float dr = d_inv[row], cr = coef[row];
+  for (int k = 0; k < kNormPerThread; ++k) {
+    const int64_t e = e0 + k;
+    if (e >= nnz) break;
+    while (e >= row_end) {
+      ++row;
+      row_end = rowptr[row + 1];
+      dr = d_inv[row];
+      cr = coef[row];
+    }
+    gw[e] = fmaf(gv[e] * dr, d_inv[colidx[e]], cr);
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // in-place fake-user injection
 // ------------------------------------------------------------------------------------------
 __global__ void count_fake_items_kernel(const int32_t* __restrict__ fake_items, int64_t n, int64_t I,
@@ -272,6 +334,45 @@ int recad_csr_normalize(const int64_t* rowptr, const int32_t* colidx, const floa
   const int T = 256;
   const int64_t threads = (nnz + kNormPerThread - 1) / kNormPerThread;
   normalize_kernel<<<(unsigned)((threads + T - 1) / T), T, 0, s>>>(rowptr, colidx, mult, d_inv, n_rows, nnz, vals);
+  RECAD_LAUNCH_CHECK();
+  return RECAD_OK;
+}
+
+// rowptr[n_rows] must be nnz (one 8-byte device->host copy, synchronises the stream)
+static int check_nnz(const int64_t* rowptr, int64_t n_rows, int64_t nnz, cudaStream_t s, const char* who) {
+  int64_t have = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&have, rowptr + n_rows, 8, cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(have == nnz, RECAD_ERR_ARG, "%s: the row pointer ends at %lld, not at nnz = %lld", who, (long long)have,
+                (long long)nnz);
+  return RECAD_OK;
+}
+
+int recad_csr_row_sums(const int64_t* rowptr, const float* w, int64_t n_rows, int64_t nnz, float* sums, void* stream) {
+  cudaStream_t s = as_stream(stream);
+  RECAD_REQUIRE(rowptr && sums && n_rows > 0 && nnz >= 0 && (nnz == 0 || w), RECAD_ERR_ARG, "csr_row_sums: bad argument");
+  int rc = check_nnz(rowptr, n_rows, nnz, s, "csr_row_sums");
+  if (rc) return rc;
+  const int T = 256;
+  row_sums_kernel<<<(unsigned)((n_rows * 32 + T - 1) / T), T, 0, s>>>(rowptr, w, n_rows, sums);
+  RECAD_LAUNCH_CHECK();
+  return RECAD_OK;
+}
+
+int recad_csr_normalize_backward(const int64_t* rowptr, const int32_t* colidx, const int64_t* tperm, const float* w,
+                                 const float* d_inv, const float* gv, int64_t n_rows, int64_t nnz, float* coef, float* gw,
+                                 void* stream) {
+  cudaStream_t s = as_stream(stream);
+  RECAD_REQUIRE(rowptr && d_inv && coef && n_rows > 0 && nnz >= 0, RECAD_ERR_ARG, "csr_normalize_backward: bad argument");
+  RECAD_REQUIRE(nnz == 0 || (colidx && tperm && w && gv && gw), RECAD_ERR_ARG, "csr_normalize_backward: null pointer");
+  int rc = check_nnz(rowptr, n_rows, nnz, s, "csr_normalize_backward");
+  if (rc) return rc;
+  if (nnz == 0) return RECAD_OK;
+  const int T = 256;
+  norm_bwd_rows_kernel<<<(unsigned)((n_rows * 32 + T - 1) / T), T, 0, s>>>(rowptr, colidx, tperm, w, d_inv, gv, n_rows, coef);
+  RECAD_LAUNCH_CHECK();
+  const int64_t threads = (nnz + kNormPerThread - 1) / kNormPerThread;
+  norm_bwd_entries_kernel<<<(unsigned)((threads + T - 1) / T), T, 0, s>>>(rowptr, colidx, d_inv, gv, coef, n_rows, nnz, gw);
   RECAD_LAUNCH_CHECK();
   return RECAD_OK;
 }

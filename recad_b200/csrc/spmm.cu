@@ -223,6 +223,117 @@ spmm_generic_kernel(const __grid_constant__ SpmmArgs a, int D) {
   }
 }
 
+// ---------------------------------------------------------------------------------------------- SDDMM
+// out[k] (+)= alpha * <G[r_k], X[c_k]> for every stored entry k = (r_k, c_k): the gradient of an SpMM with respect to
+// the matrix's values.  The same packed plan drives it (one warp per segment, its entry loaded one segment ahead); G[row]
+// sits in registers for the whole segment, the X rows are gathered with D/4 lanes of 128-bit loads, UNR in flight, and
+// each dot product is reduced over its LPR lanes with shuffles in a fixed order.  Every entry has exactly one writer, so
+// the kernel needs no atomics, partial slots or arrival counters even for multi-segment or column-blocked rows, and
+// gives the same bits on every run.  It reads colidx (4 bytes) instead of the (col, val) pairs: the value is not needed.
+struct SddmmArgs {
+  const int4* seg_meta;
+  int64_t n_seg;
+  const int32_t* colidx;
+  const float* G;
+  const float* X;
+  float* out;
+  float alpha;
+  int accumulate;
+};
+
+template <int D, int UNR>
+__global__ void __launch_bounds__(kSpmmWarps * 32, 4)
+sddmm_kernel(const __grid_constant__ SddmmArgs a) {
+  constexpr int LPR = D / 4;               // lanes per row (float4 each)
+  constexpr int NPL = 32 / LPR;            // entries per warp-wide gather
+  constexpr int R = NPL * UNR;             // entries per round
+  const int lane = threadIdx.x & 31;
+  const int sub = lane / LPR, l = lane % LPR;
+  const int64_t n_warps = (int64_t)gridDim.x * kSpmmWarps;
+  int64_t seg = (int64_t)blockIdx.x * kSpmmWarps + (threadIdx.x >> 5);
+  if (seg >= a.n_seg) return;
+  const float4* __restrict__ X4 = reinterpret_cast<const float4*>(a.X);
+  const float4* __restrict__ G4 = reinterpret_cast<const float4*>(a.G);
+  int4 meta = __ldg(a.seg_meta + seg);
+  while (true) {
+    const int64_t next = seg + n_warps;
+    int4 meta_n = make_int4(0, 0, 0, 0);
+    if (next < a.n_seg) meta_n = __ldg(a.seg_meta + next);      // one segment ahead
+    const int64_t lo = (int64_t)(uint32_t)meta.x | ((int64_t)meta.y << 32);
+    const int cnt = meta.w & 2047;
+    const float4 g = cnt ? __ldg(G4 + (int64_t)meta.z * LPR + l) : make_float4(0.f, 0.f, 0.f, 0.f);
+    const int32_t* __restrict__ p = a.colidx + lo + sub;
+    int nc[UNR];
+#pragma unroll
+    for (int u = 0; u < UNR; ++u) nc[u] = (u * NPL + sub < cnt) ? __ldg(p + u * NPL) : 0;
+    for (int j = 0; j < cnt; j += R) {
+      float4 x[UNR];
+#pragma unroll
+      for (int u = 0; u < UNR; ++u)
+        x[u] = (j + u * NPL + sub < cnt) ? __ldg(X4 + ((uint32_t)nc[u] * (uint32_t)LPR + (uint32_t)l))   // < 2^32 checked on the host
+                                         : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+      for (int u = 0; u < UNR; ++u)                               // columns of the next round, under the gathers
+        nc[u] = (j + R + u * NPL + sub < cnt) ? __ldg(p + j + R + u * NPL) : 0;
+#pragma unroll
+      for (int u = 0; u < UNR; ++u) {
+        float d = g.x * x[u].x + g.y * x[u].y + g.z * x[u].z + g.w * x[u].w;
+#pragma unroll
+        for (int o = LPR / 2; o > 0; o >>= 1) d += __shfl_xor_sync(kFull, d, o);
+        const int64_t e = lo + j + u * NPL + sub;
+        if (l == 0 && j + u * NPL + sub < cnt) a.out[e] = a.accumulate ? fmaf(a.alpha, d, a.out[e]) : a.alpha * d;
+      }
+    }
+    if (next >= a.n_seg) break;
+    seg = next;
+    meta = meta_n;
+  }
+}
+
+// any D that is a multiple of 4 (<= 1024): a lane owns float4 columns lane, lane + 32, ...; one entry at a time
+__global__ void __launch_bounds__(kSpmmWarps * 32)
+sddmm_generic_kernel(const __grid_constant__ SddmmArgs a, int D) {
+  const int lane = threadIdx.x & 31;
+  const int nvec = D / 4;
+  const int64_t n_warps = (int64_t)gridDim.x * kSpmmWarps;
+  const float4* __restrict__ X4 = reinterpret_cast<const float4*>(a.X);
+  const float4* __restrict__ G4 = reinterpret_cast<const float4*>(a.G);
+  for (int64_t seg = (int64_t)blockIdx.x * kSpmmWarps + (threadIdx.x >> 5); seg < a.n_seg; seg += n_warps) {
+    const int4 meta = __ldg(a.seg_meta + seg);
+    const int64_t lo = (int64_t)(uint32_t)meta.x | ((int64_t)meta.y << 32);
+    const int row = meta.z, cnt = meta.w & 2047;
+    if (!cnt) continue;
+    float4 g[kGenericMaxVec];
+#pragma unroll
+    for (int q = 0; q < kGenericMaxVec; ++q)
+      g[q] = (lane + q * 32 < nvec) ? __ldg(G4 + (int64_t)row * nvec + lane + q * 32) : make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int k = 0; k < cnt; ++k) {
+      const int64_t c = __ldg(a.colidx + lo + k);
+      float d = 0.f;
+#pragma unroll
+      for (int q = 0; q < kGenericMaxVec; ++q) {
+        if (lane + q * 32 < nvec) {
+          const float4 x = __ldg(X4 + c * nvec + lane + q * 32);
+          d += g[q].x * x.x + g[q].y * x.y + g[q].z * x.z + g[q].w * x.w;
+        }
+      }
+      d = warp_sum(d);
+      if (lane == 0) a.out[lo + k] = a.accumulate ? fmaf(a.alpha, d, a.out[lo + k]) : a.alpha * d;
+    }
+  }
+}
+
+template <int D>
+static int launch_sddmm(const SddmmArgs& a, cudaStream_t s) {
+  auto kern = sddmm_kernel<D, 4>;
+  static int per_sm = 0;
+  if (!per_sm) RECAD_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kSpmmWarps * 32, 0));
+  const int64_t grid = std::min<int64_t>((a.n_seg + kSpmmWarps - 1) / kSpmmWarps, (int64_t)sm_count() * std::max(per_sm, 1));
+  kern<<<(unsigned)grid, kSpmmWarps * 32, 0, s>>>(a);
+  RECAD_LAUNCH_CHECK();
+  return RECAD_OK;
+}
+
 __global__ void pack_cv_kernel(const int32_t* __restrict__ col, const float* __restrict__ val, int64_t nnz, int2* __restrict__ cv) {
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += (int64_t)gridDim.x * blockDim.x)
     cv[e] = make_int2(col[e], __float_as_int(val[e]));
@@ -299,6 +410,38 @@ extern "C" int recad_spmm(const recad_csr* A, const float* X, float* Y, const fl
   }
   const int64_t grid = std::min<int64_t>((A->n_seg + kSpmmWarps - 1) / kSpmmWarps, (int64_t)sm_count() * 8);
   spmm_generic_kernel<<<(unsigned)grid, kSpmmWarps * 32, 0, s>>>(a, D);
+  RECAD_LAUNCH_CHECK();
+  return RECAD_OK;
+}
+
+extern "C" int recad_csr_sddmm(const recad_csr* A, const float* G, const float* X, int32_t D, float alpha, int32_t accumulate,
+                               float* out, void* stream) {
+  cudaStream_t s = as_stream(stream);
+  RECAD_REQUIRE(A, RECAD_ERR_ARG, "csr_sddmm: null matrix");
+  RECAD_REQUIRE(A->n_rows > 0 && A->n_seg >= A->n_rows && A->seg_meta, RECAD_ERR_ARG, "csr_sddmm: matrix has no plan (ops.PackedPlan)");
+  RECAD_REQUIRE(G && X && (A->nnz == 0 || (A->colidx && out)), RECAD_ERR_ARG, "csr_sddmm: null pointer");
+  RECAD_REQUIRE(D >= 4 && D % 4 == 0 && D <= 4 * 32 * kGenericMaxVec, RECAD_ERR_UNSUPPORTED,
+                "csr_sddmm: D = %d must be a multiple of 4 in [4, %d]", D, 4 * 32 * kGenericMaxVec);
+  RECAD_REQUIRE(A->n_cols > 0 && A->n_cols * (int64_t)(D / 4) < ((int64_t)1 << 32), RECAD_ERR_OVERFLOW,
+                "csr_sddmm: %lld columns x D = %d exceed the 32-bit gather offset", (long long)A->n_cols, D);
+  RECAD_REQUIRE((((uintptr_t)G | (uintptr_t)X) & 15) == 0, RECAD_ERR_ARG, "csr_sddmm: G and X must be 16-byte aligned");
+  if (A->nnz == 0) return RECAD_OK;
+  SddmmArgs a;
+  a.seg_meta = reinterpret_cast<const int4*>(A->seg_meta);
+  a.n_seg = A->n_seg;
+  a.colidx = A->colidx;
+  a.G = G; a.X = X; a.out = out; a.alpha = alpha; a.accumulate = accumulate != 0;
+  switch (D) {
+    case 4: return launch_sddmm<4>(a, s);
+    case 8: return launch_sddmm<8>(a, s);
+    case 16: return launch_sddmm<16>(a, s);
+    case 32: return launch_sddmm<32>(a, s);
+    case 64: return launch_sddmm<64>(a, s);
+    case 128: return launch_sddmm<128>(a, s);
+    default: break;
+  }
+  const int64_t grid = std::min<int64_t>((A->n_seg + kSpmmWarps - 1) / kSpmmWarps, (int64_t)sm_count() * 8);
+  sddmm_generic_kernel<<<(unsigned)grid, kSpmmWarps * 32, 0, s>>>(a, D);
   RECAD_LAUNCH_CHECK();
   return RECAD_OK;
 }

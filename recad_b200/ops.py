@@ -320,6 +320,25 @@ class Graph:
             self._tperm = T
         return self._tperm
 
+    def entry_index(self, rows, cols):
+        """int64 positions (CSR entry order) of the stored entries (rows[j], cols[j]); RecadError if a pair is not stored.
+        With transpose_permutation, entry_index(r, c) and T[entry_index(r, c)] are the two entries of one interaction."""
+        with torch.cuda.device(self.device):
+            rows = torch.as_tensor(rows, device=self.device).long()
+            cols = torch.as_tensor(cols, device=self.device).long()
+            if rows.shape != cols.shape:
+                raise RecadError(f"entry_index: {tuple(rows.shape)} rows but {tuple(cols.shape)} columns")
+            if rows.numel() and bool(((rows < 0) | (rows >= self.n_rows) | (cols < 0) | (cols >= self.n_cols)).any()):
+                raise RecadError("entry_index: a row or column is out of range")
+            if getattr(self, "_ekeys", None) is None:
+                r = torch.repeat_interleave(torch.arange(self.n_rows, device=self.device), self.rowptr[1:] - self.rowptr[:-1])
+                self._ekeys = r * self.n_cols + self.colidx.long()              # ascending: CSR order with sorted columns
+            q = rows * self.n_cols + cols
+            k = torch.searchsorted(self._ekeys, q.reshape(-1)).clamp_(max=max(self.nnz - 1, 0)).reshape(q.shape)
+            if q.numel() and (self.nnz == 0 or not bool((self._ekeys[k] == q).all())):
+                raise RecadError("entry_index: a (row, column) pair is not a stored entry")
+        return k
+
     def set_values(self, vals):
         with torch.cuda.device(self.device):
             self.vals.copy_(vals)
@@ -348,6 +367,27 @@ def spmm(graph, X, Y=None, C_=None, Z=None, alpha=1.0):
         check(_lib.lib().recad_spmm(C.byref(graph.struct(D)), _ptr(X), _ptr(Y), _ptr(C_), _ptr(Z), float(alpha), D,
                                     _stream(X.device)), "recad_spmm")
     return Y, Z
+
+
+def sddmm(graph, G, X, alpha=1.0, out=None, accumulate=False):
+    """out[k] = alpha * <G[r_k], X[c_k]> for every stored entry k = (r_k, c_k), in CSR entry order (recad_csr_sddmm); with
+    `accumulate`, out[k] += ... into the given `out`.  The gradient of sum(gY * (A X)) with respect to A's values for
+    G = gY.  Returns out (float32 [nnz])."""
+    _need_cuda(G, X, out)
+    D = int(X.shape[1]) if X.dim() == 2 else -1
+    if G.dtype != torch.float32 or X.dtype != torch.float32 or tuple(G.shape) != (graph.n_rows, D) or \
+            tuple(X.shape) != (graph.n_cols, D):
+        raise RecadError(f"sddmm: G must be float32 [{graph.n_rows}, D] and X float32 [{graph.n_cols}, D]")
+    if accumulate and out is None:
+        raise RecadError("sddmm: accumulate needs out")
+    if out is not None and (out.dtype != torch.float32 or out.numel() != graph.nnz or not out.is_contiguous()):
+        raise RecadError(f"sddmm: out must be a contiguous float32 tensor of {graph.nnz} entries")
+    with torch.cuda.device(X.device):
+        if out is None:
+            out = torch.empty(graph.nnz, dtype=torch.float32, device=X.device)
+        check(_lib.lib().recad_csr_sddmm(C.byref(graph.struct(D)), _ptr(G.contiguous()), _ptr(X.contiguous()), D, float(alpha),
+                                         int(bool(accumulate)), _ptr(out), _stream(X.device)), "recad_csr_sddmm")
+    return out
 
 
 def axpby(z, a, x, b, y):
@@ -507,6 +547,162 @@ class LightGCNPropagate(torch.autograd.Function):
         gE = lightgcn_backward(ctx.st, gO.contiguous())
         U = ctx.st.n_users
         return None, None, None, gE[:U], gE[U:]
+
+
+def check_values(graph, values, what):
+    """RecadError unless `values` is a float32 CUDA tensor [graph.nnz] on the graph's device."""
+    if not isinstance(values, torch.Tensor) or not values.is_cuda:
+        raise RecadError(f"{what}: a float32 CUDA tensor [{graph.nnz}] is needed (got {type(values).__name__}"
+                         f"{' on the CPU' if isinstance(values, torch.Tensor) else ''})")
+    if values.dtype != torch.float32 or tuple(values.shape) != (graph.nnz,) or values.device != graph.device:
+        raise RecadError(f"{what}: float32 [{graph.nnz}] on {graph.device} needed, got {values.dtype} "
+                         f"{list(values.shape)} on {values.device}")
+
+
+class ValueGraphs:
+    """A LightGCN state whose propagation runs over caller-supplied values instead of its graph's: a value copy of the graph
+    and of its transpose (the same structure and plan, values[T]), made by Graph.with_values on the first `load` and
+    refilled in place by set_values after that.  A victim keeps one, as it keeps its dropped graph."""
+
+    def __init__(self, graph, st):
+        self.graph, self.base, self.g, self.g_t, self.st = graph, st, None, None, None
+
+    def load(self, values):
+        """Fill both matrices with `values` / values[T] and return the state that propagates over them."""
+        with torch.cuda.device(self.graph.device):
+            values = values.detach()
+            vals_t = values[self.graph.transpose_permutation()]
+            if self.g is None:
+                self.g, self.g_t = self.graph.with_values(values), self.graph.with_values(vals_t)
+                st = _lib.LightGCN()
+                C.memmove(C.byref(st), C.byref(self.base), C.sizeof(st))
+                st.graph = C.pointer(self.g.struct(st.D))
+                st.graph_t = C.pointer(self.g_t.struct(st.D))
+                self.st = st
+            else:
+                self.g.set_values(values)
+                self.g_t.set_values(vals_t)
+        return self.st
+
+
+def lightgcn_propagate_layers(st, E, keep):
+    """O = mean_l A^l E over st.graph into a fresh [N, D] buffer, layer by layer with recad_spmm (the calls
+    recad_lightgcn_propagate makes, so the bits are the same), and the layers [E, X_1, .., X_{L-1}] when `keep`."""
+    N, D, L = st.n_users + st.n_items, st.D, st.n_layers
+    dev = E.device
+    lib = _lib.lib()
+    with torch.cuda.device(dev):
+        O = torch.empty((N, D), dtype=torch.float32, device=dev)
+        if L == 0:
+            O.copy_(E)
+            return O, [E]
+        layers, x = [E], E
+        work = [torch.empty_like(O) for _ in range(min(L - 1, 2))] if not keep else []
+        for k in range(L):
+            last = k == L - 1
+            y = None if last else (torch.empty_like(O) if keep else work[k & 1])
+            check(lib.recad_spmm(st.graph, _ptr(x), _ptr(y), _ptr(E if k == 0 else O), _ptr(O),
+                                 1.0 / (L + 1) if last else 1.0, D, _stream(dev)), "recad_spmm")
+            if keep and y is not None:
+                layers.append(y)
+            x = y
+    return O, (layers if keep else None)
+
+
+class LightGCNPropagateValues(torch.autograd.Function):
+    """O = mean_l A^l E with A's values given as a tensor [nnz] (CSR entry order), differentiable with respect to those
+    values and both tables.  `vg` is the victim's ValueGraphs; E is the victim's table, of which user_w / item_w are the
+    views.  The layers X_1 .. X_{L-1} are kept for the backward, which first restores its own forward's values into the
+    value graphs (a later forward may have loaded others) and then runs recad_lightgcn_backward_values (edge values
+    wanted) or recad_lightgcn_backward."""
+
+    @staticmethod
+    def forward(ctx, vg, E, values, user_w, item_w):
+        st = vg.load(values)
+        O, layers = lightgcn_propagate_layers(st, E, keep=True)
+        ctx.vg, ctx.E, ctx.layers = vg, E, layers
+        ctx.save_for_backward(values, user_w, item_w)
+        return O
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gO):
+        values, _, _ = ctx.saved_tensors
+        need_v, need_u, need_i = ctx.needs_input_grad[2:5]
+        st = ctx.vg.load(values)
+        gO = gO.contiguous()
+        dev, U, L = gO.device, st.n_users, st.n_layers
+        lib = _lib.lib()
+        with torch.cuda.device(dev):
+            gE = torch.empty_like(gO) if (need_u or need_i) else None
+            work = [torch.empty_like(gO) for _ in range(min(max(L - 1, 0), 2))]
+            sb = _lib.LightGCN()
+            C.memmove(C.byref(sb), C.byref(st), C.sizeof(sb))
+            sb.X0 = work[0].data_ptr() if len(work) > 0 else None
+            sb.X1 = work[1].data_ptr() if len(work) > 1 else None
+            gvals = None
+            if need_v:
+                gvals = torch.empty(values.numel(), dtype=torch.float32, device=dev)
+                X = (_lib.vp * max(L, 1))(*[x.data_ptr() for x in ctx.layers[:L]])
+                check(lib.recad_lightgcn_backward_values(C.byref(sb), _ptr(gO), X, _ptr(gE), _ptr(gvals), _stream(dev)),
+                      "recad_lightgcn_backward_values")
+            else:
+                check(lib.recad_lightgcn_backward(C.byref(sb), _ptr(gO), _ptr(gE), _stream(dev)), "recad_lightgcn_backward")
+        return (None, None, gvals, gE[:U] if need_u else None, gE[U:] if need_i else None)
+
+
+def lightgcn_propagate_values(st_vals, E):
+    """recad_lightgcn_propagate over a value-graph state into fresh buffers (no autograd)."""
+    O, _ = lightgcn_propagate_layers(st_vals, E, keep=False)
+    return O
+
+
+class NormalizedValues(torch.autograd.Function):
+    """vals_k = d_r w_k d_c from per-entry weights (recad_csr_row_sums, the host d_inv, recad_csr_normalize); backward by
+    recad_csr_normalize_backward."""
+
+    @staticmethod
+    def forward(ctx, graph, weights):
+        dev = graph.device
+        lib = _lib.lib()
+        with torch.cuda.device(dev):
+            sums = torch.empty(graph.n_rows, dtype=torch.float32, device=dev)
+            check(lib.recad_csr_row_sums(_ptr(graph.rowptr), _ptr(weights), graph.n_rows, graph.nnz, _ptr(sums), _stream(dev)),
+                  "recad_csr_row_sums")
+            d_inv = torch.from_numpy(d_inv_from_degree(sums.cpu().numpy())).to(dev)
+            vals = torch.empty(graph.nnz, dtype=torch.float32, device=dev)
+            check(lib.recad_csr_normalize(_ptr(graph.rowptr), _ptr(graph.colidx), _ptr(weights), _ptr(d_inv), graph.n_rows,
+                                          _ptr(vals), _stream(dev)), "recad_csr_normalize")
+        ctx.graph, ctx.d_inv = graph, d_inv
+        ctx.save_for_backward(weights)
+        return vals
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gv):
+        weights, = ctx.saved_tensors
+        g = ctx.graph
+        dev = g.device
+        with torch.cuda.device(dev):
+            gv = gv.contiguous().float()
+            coef = torch.empty(g.n_rows, dtype=torch.float32, device=dev)
+            gw = torch.empty(g.nnz, dtype=torch.float32, device=dev)
+            check(_lib.lib().recad_csr_normalize_backward(_ptr(g.rowptr), _ptr(g.colidx), _ptr(g.transpose_permutation()),
+                                                          _ptr(weights), _ptr(ctx.d_inv), _ptr(gv), g.n_rows, g.nnz, _ptr(coef),
+                                                          _ptr(gw), _stream(dev)), "recad_csr_normalize_backward")
+        return None, gw
+
+
+def normalized_values(graph, weights):
+    """The symmetric normalisation (implicit.py:269-276) as a differentiable map from per-entry weights [nnz] (CSR entry
+    order) to values: vals_k = d_r w_k d_c, d_r = (sum of row r's weights + 1e-14)^(-1/2), d_inv evaluated on the host
+    exactly as for the dataset's graph, so normalized_values(g, g.mult) equals g.vals.  For a square, structurally
+    symmetric graph; the weights need not be symmetric."""
+    if graph.n_rows != graph.n_cols:
+        raise RecadError("normalized_values: the matrix is not square")
+    check_values(graph, weights, "normalized_values")
+    graph.transpose_permutation()                 # RecadError unless the structure is symmetric
+    return NormalizedValues.apply(graph, weights.contiguous())
 
 
 class DotScores(torch.autograd.Function):

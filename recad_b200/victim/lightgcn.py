@@ -94,6 +94,7 @@ class LightGCN(BaseVictim):
             setattr(st, k, getattr(self, k).data_ptr())
         self._st = st
         self._drop_graph = self._drop_graph_t = self._st_drop = None
+        self._value_graphs = None  # ops.ValueGraphs for caller-supplied edge values, made on first use
         self._O_valid = False      # O was just (re)allocated: never score from it before a propagate
         self._O_version = -1
 
@@ -154,6 +155,21 @@ class LightGCN(BaseVictim):
             st, graph_t, vals_t = self._st, None, None
         return ops.LightGCNPropagate.apply(st, graph_t, vals_t, self.embedding_user.weight, self.embedding_item.weight)
 
+    def _propagate_values(self, edge_values):
+        """The propagation over caller-supplied edge values (float32 CUDA [Graph.nnz], CSR entry order) into a fresh buffer:
+        differentiable with respect to them and to the tables when grad mode is on and one of them requires a gradient.
+        The cached propagation (self.O) is neither read nor written."""
+        ops.check_values(self.Graph, edge_values, "LightGCN edge_values")
+        if self.dropout and self.training:
+            raise ops.RecadError("LightGCN: edge_values cannot be combined with graph dropout in training mode")
+        if self._value_graphs is None:
+            self._value_graphs = ops.ValueGraphs(self.Graph, self._st)
+        w_u, w_i = self.embedding_user.weight, self.embedding_item.weight
+        if torch.is_grad_enabled() and (edge_values.requires_grad or w_u.requires_grad or w_i.requires_grad):
+            return ops.LightGCNPropagateValues.apply(self._value_graphs, self.E, edge_values.contiguous(), w_u, w_i)
+        st = self._value_graphs.load(edge_values)
+        return ops.lightgcn_propagate_values(st, self.E)
+
     def _cached_O(self):
         """self.O, propagated again unless it is current: the tables have not changed since (train_step, load_state_dict,
         in-place updates such as a torch optimizer's step, which bump the tables' version) and no dropout mask applies."""
@@ -161,11 +177,16 @@ class LightGCN(BaseVictim):
             self.computer()
         return self.O
 
-    def computer(self):
+    def computer(self, edge_values=None):
         """lightgcn.py:82-113: (users, items) propagated embeddings = mean of the layer outputs (over a freshly dropped
         graph when dropout is on and the module is in training mode).  Differentiable with respect to the two tables when
-        grad mode is on and one of them requires a gradient."""
+        grad mode is on and one of them requires a gradient.
+        edge_values: float32 CUDA tensor [Graph.nnz] in the graph's CSR entry order, propagated over instead of the graph's
+        values (and differentiable with respect to when it requires a gradient); not with graph dropout in training mode."""
         self._require_instance("computer")
+        if edge_values is not None:
+            O = self._propagate_values(edge_values)
+            return O[:self.num_users], O[self.num_users:]
         if self._graph_mode():
             O = self._propagate_graph()
             return O[:self.num_users], O[self.num_users:]
@@ -227,14 +248,22 @@ class LightGCN(BaseVictim):
                            int(samples.shape[0]) if n is None else int(n), B, self._steps if step0 is None else int(step0),
                            ops._stream(self._dev)), name)
 
-    def forward(self, users, items):
+    def forward(self, users, items, edge_values=None):
         """lightgcn.py:174-183: <O_u, O_i>.  The propagation is redone only when the tables changed
         (the reference redoes it on every call, i.e. once per evaluated user).  In autograd (grad mode on and a table
         that requires a gradient) every call propagates again, as the reference does, and the scores are differentiable
-        with respect to both tables."""
+        with respect to both tables.
+        edge_values: see `computer`; such a call always propagates again, and its scores are differentiable with respect
+        to edge_values when it requires a gradient."""
         self._require_instance("forward")
         users = users.to(self._dev).long().contiguous()
         items = items.to(self._dev).long().contiguous()
+        if edge_values is not None:
+            O = self._propagate_values(edge_values)
+            if O.requires_grad:
+                self._check_ids(users, self.num_users, items, self.num_items)
+                return ops.DotScores.apply(O, self.num_users, users, items)
+            return ops.dot_scores(O, self.num_users, users, items)
         if self._graph_mode():
             self._check_ids(users, self.num_users, items, self.num_items)
             return ops.DotScores.apply(self._propagate_graph(), self.num_users, users, items)
