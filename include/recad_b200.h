@@ -460,6 +460,31 @@ int recad_lightgcn_backward_values(const recad_lightgcn* st, const float* gO, co
                                    void* stream);
 
 /* ------------------------------------------------------------------------ *
+ * Hessian-vector products of the training losses (LightGCN's BPR, MF's BCE)
+ * ------------------------------------------------------------------------ */
+
+/* The pair backward with a second gather source: outA [dev] float[n_a, D] = sum over the b with ia[b] = r of
+ * (alpha[b] Xb[ib[b]] + beta[b] Vb[ib[b]]), outB [dev] float[n_b, D] likewise with Xa / Va, dba / dbb = sum of alpha[b] per
+ * row (NULL: not wanted).  beta NULL: Va / Vb are not read and the result is recad_pair_scores_backward's, bit for bit.
+ * Same sort, scratch (recad_pair_scores_backward_scratch_bytes(B)), determinism and id check as that entry. */
+int recad_pair_scores_hvp(const float* Xa, const float* Va, int64_t n_a, const float* Xb, const float* Vb, int64_t n_b,
+                          int32_t D, const int64_t* ia, const int64_t* ib, int64_t B, const float* alpha, const float* beta,
+                          float* outA, float* outB, float* dba, float* dbb, void* scratch, int64_t scratch_bytes, void* stream);
+
+/* Per-sample seeds of H_O dO for the BPR loss (1/B_norm) sum_b softplus(x_b), x_b = <O_u, O_n> - <O_u, O_p>, over the n rows
+ * samples [dev] int64[n, 3] = (user, pos, neg); O, dO [dev] float[n_users + n_items, D] (users first).  With
+ * dx_b = <dO_u, O_n - O_p> + <O_u, dO_n - dO_p>, l' = sigmoid(x), l'' = l'(1 - l') (x > 20: 1 and 0, torch's softplus):
+ *   alpha [dev] float[2n]: alpha[b] = l''(x_b) dx_b / B_norm, alpha[n + b] = -alpha[b];
+ *   beta  [dev] float[2n]: beta[b] = l'(x_b) / B_norm, beta[n + b] = -beta[b],
+ * i.e. the seeds of recad_pair_scores_hvp over the pairs (u, neg) then (u, pos).  dloss [dev] float[n] (NULL: not wanted) =
+ * l'(x_b) dx_b + lambda (<V_u, E_u> + <V_p, E_p> + <V_n, E_n>), the unnormalised derivative of sample b's loss along V when
+ * dO = P V; E and V are then needed.  bad [dev] int32 work flag.  Deterministic.  Synchronises the stream: an id outside
+ * its table gives RECAD_ERR_ARG. */
+int recad_bpr_hvp_seeds(const float* O, const float* dO, int64_t n_users, int64_t n_items, const int64_t* samples, int64_t n,
+                        int64_t B_norm, int32_t D, const float* E, const float* V, float lambda, float* alpha, float* beta,
+                        float* dloss, int32_t* bad, void* stream);
+
+/* ------------------------------------------------------------------------ *
  * MF pointwise BCE step  (recad/model/victim/mf.py:40-69)
  * ------------------------------------------------------------------------ */
 typedef struct recad_mf {
@@ -488,6 +513,16 @@ int recad_mf_train_epoch(const recad_mf* st, const int64_t* samples, const int64
  * allowed (zero gradient). */
 int recad_mf_grad(const recad_mf* st, const int64_t* samples, const int64_t* perm, int64_t B, int64_t B_norm,
                   void* stream);
+/* Per-row seeds of the Hessian-vector product of (1/B_norm) sum_b BCEWithLogits(y_b, label_b) over the n rows samples [dev]
+ * int64[n, 3] = (user, item, label), y = <Ue_u, Ie_i> + Ub_u + Ib_i + st->mean (mean held constant), along the direction
+ * (dUe [U, D], dUb [U], dIe [I, D], dIb [I]) [dev]: with dy_b = <dUe_u, Ie_i> + <Ue_u, dIe_i> + dUb_u + dIb_i,
+ * l' = sigmoid(y) - label, l'' = sigmoid(y)(1 - sigmoid(y)):  alpha [dev] float[n] = l'' dy / B_norm,
+ * beta [dev] float[n] = l' / B_norm (the seeds of recad_pair_scores_hvp over the pairs (user, item); its bias outputs are
+ * the bias rows of the product), dloss [dev] float[n] (NULL: not wanted) = l' dy.  Reads the parameter tables only.
+ * bad [dev] int32 work flag.  Deterministic.  Synchronises the stream: an id outside its table gives RECAD_ERR_ARG. */
+int recad_mf_hvp_seeds(const recad_mf* st, const float* dUe, const float* dUb, const float* dIe, const float* dIb,
+                       const int64_t* samples, int64_t n, int64_t B_norm, float* alpha, float* beta, float* dloss, int32_t* bad,
+                       void* stream);
 
 /* ------------------------------------------------------------------------ *
  * NCF / NeuMF-end pointwise BCE step  (recad/model/victim/ncf.py:32-53, 112-153)

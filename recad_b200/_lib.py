@@ -133,12 +133,15 @@ SIGNATURES = {
     "recad_pair_scores_backward": (C.c_int, [vp, i64, vp, i64, i32, vp, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp]),
     "recad_lightgcn_backward": (C.c_int, [C.POINTER(LightGCN), vp, vp, vp]),
     "recad_lightgcn_backward_values": (C.c_int, [C.POINTER(LightGCN), vp, C.POINTER(vp), vp, vp, vp]),
+    "recad_pair_scores_hvp": (C.c_int, [vp, vp, i64, vp, vp, i64, i32, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, i64, vp]),
+    "recad_bpr_hvp_seeds": (C.c_int, [vp, vp, i64, i64, vp, i64, i64, i32, vp, vp, f32, vp, vp, vp, vp, vp]),
     "recad_csr_sddmm": (C.c_int, [C.POINTER(CSR), vp, vp, i32, f32, i32, vp, vp]),
     "recad_csr_row_sums": (C.c_int, [vp, vp, i64, i64, vp, vp]),
     "recad_csr_normalize_backward": (C.c_int, [vp, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp]),
     "recad_mf_forward": (C.c_int, [C.POINTER(MF), vp, vp, i64, vp, vp]),
     "recad_mf_train_epoch": (C.c_int, [C.POINTER(MF), vp, vp, i64, i64, i64, vp]),
     "recad_mf_grad": (C.c_int, [C.POINTER(MF), vp, vp, i64, i64, vp]),
+    "recad_mf_hvp_seeds": (C.c_int, [C.POINTER(MF), vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp]),
     "recad_ncf_layout": (C.c_int, [i32, i32, i64, i64, C.POINTER(i64)]),
     "recad_ncf_work_floats": (i64, [i32, i32, i64]),
     "recad_ncf_forward": (C.c_int, [C.POINTER(NCF), vp, vp, i64, vp, vp]),

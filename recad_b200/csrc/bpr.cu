@@ -366,11 +366,15 @@ pair_keys_kernel(const int64_t* __restrict__ ids, int64_t n_rows, int64_t B, int
   }
 }
 
-// one warp per sorted key; the warp of a row's first key writes dX[row] (and db[row]), every other warp returns
+// one warp per sorted key; the warp of a row's first key writes dX[row] = sum g_b X[other_b] (+ beta_b V[other_b] when kTwo)
+// and db[row] = sum g_b; every other warp returns.  kTwo sums in double: a Hessian product's popular rows collect 10^5 and
+// more pairs, and a float running sum of that length loses ~sqrt(count) ulps (1e-5 of the row at 10^5 pairs).
+template <bool kTwo>
 __global__ void __launch_bounds__(256)
 pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, const float* __restrict__ g,
-                      const int64_t* __restrict__ other, int64_t n_other, const float* __restrict__ X, int nvec,
-                      float* __restrict__ dX, float* __restrict__ db) {
+                      const float* __restrict__ beta, const int64_t* __restrict__ other, int64_t n_other,
+                      const float* __restrict__ X, const float* __restrict__ V, int nvec, float* __restrict__ dX,
+                      float* __restrict__ db) {
   const int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (k >= B) return;
@@ -378,11 +382,13 @@ pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, c
   if (k > 0 && (keys[k - 1] >> bbits) == row) return;
   const uint64_t bmask = (1ull << bbits) - 1;
   const float4* __restrict__ X4 = reinterpret_cast<const float4*>(X);
+  const float4* __restrict__ V4 = reinterpret_cast<const float4*>(V);
   float4* __restrict__ dX4 = reinterpret_cast<float4*>(dX);
   for (int c0 = 0; c0 < nvec; c0 += 32) {
     const int c = c0 + lane;
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     float gsum = 0.f;
+    double dx = 0.0, dy = 0.0, dz = 0.0, dw = 0.0, dg = 0.0;       // kTwo accumulators
     for (int64_t j = k; j < B; ++j) {
       const uint64_t key = keys[j];
       if ((key >> bbits) != row) break;
@@ -390,14 +396,99 @@ pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, c
       int64_t o = other[b];
       if (o < 0 || o >= n_other) o = 0;            // reported by the other side's key pass
       const float gv = g[b];
-      gsum += gv;
-      if (c < nvec) {
-        const float4 x = __ldg(X4 + o * nvec + c);
-        acc.x += gv * x.x; acc.y += gv * x.y; acc.z += gv * x.z; acc.w += gv * x.w;
+      if constexpr (kTwo) {
+        dg += (double)gv;
+        if (c < nvec) {
+          const double bv = (double)beta[b];
+          const float4 x = __ldg(X4 + o * nvec + c), y = __ldg(V4 + o * nvec + c);
+          dx = fma((double)gv, (double)x.x, fma(bv, (double)y.x, dx));
+          dy = fma((double)gv, (double)x.y, fma(bv, (double)y.y, dy));
+          dz = fma((double)gv, (double)x.z, fma(bv, (double)y.z, dz));
+          dw = fma((double)gv, (double)x.w, fma(bv, (double)y.w, dw));
+        }
+      } else {
+        gsum += gv;
+        if (c < nvec) {
+          const float4 x = __ldg(X4 + o * nvec + c);
+          acc.x += gv * x.x; acc.y += gv * x.y; acc.z += gv * x.z; acc.w += gv * x.w;
+        }
       }
+    }
+    if constexpr (kTwo) {
+      acc = make_float4((float)dx, (float)dy, (float)dz, (float)dw);
+      gsum = (float)dg;
     }
     if (c < nvec) dX4[(int64_t)row * nvec + c] = acc;
     if (c0 == 0 && lane == 0 && db) db[row] = gsum;
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// Seeds of the BPR loss's Hessian-vector product.  Per sample b, x = <O_u, O_n> - <O_u, O_p>, dx its derivative along
+// dO = P v, l' / l'' softplus's first two derivatives (torch's threshold 20, as bpr_kernel); the (u, n) pair gets
+// (a, c) = (l'' dx / B, l' / B) and the (u, p) pair (-a, -c).  dloss[b] = l' dx + lambda (<V_u, E_u> + <V_p, E_p> + <V_n, E_n>).
+// kSeedLanes lanes per sample, 128-bit loads, a fixed shuffle order: no atomics on the results.
+// ------------------------------------------------------------------------------------------
+constexpr int kSeedLanes = 16;
+
+__device__ __forceinline__ float dot4(const float4 a, const float4 b) { return a.x * b.x + a.y * b.y + a.z * b.z + a.w * b.w; }
+
+__global__ void __launch_bounds__(256)
+bpr_hvp_seeds_kernel(const float* __restrict__ O, const float* __restrict__ dO, int64_t n_users, int64_t n_items,
+                     const int64_t* __restrict__ samples, int64_t n, float inv_B, int nvec, const float* __restrict__ E,
+                     const float* __restrict__ V, float lambda, float* __restrict__ alpha, float* __restrict__ beta,
+                     float* __restrict__ dloss, int* __restrict__ bad) {
+  const int l = threadIdx.x % kSeedLanes;
+  const int64_t group = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / kSeedLanes;
+  const int64_t n_groups = (int64_t)gridDim.x * blockDim.x / kSeedLanes;
+  const int64_t iters = (n + n_groups - 1) / n_groups;       // the same count on every lane: the shuffles are warp-wide
+  const float4* __restrict__ O4 = reinterpret_cast<const float4*>(O);
+  const float4* __restrict__ dO4 = reinterpret_cast<const float4*>(dO);
+  const float4* __restrict__ E4 = reinterpret_cast<const float4*>(E);
+  const float4* __restrict__ V4 = reinterpret_cast<const float4*>(V);
+  for (int64_t it = 0; it < iters; ++it) {
+    const int64_t b = it * n_groups + group;
+    const bool valid = b < n;
+    int64_t u = 0, p = 0, q = 0;
+    if (valid) {
+      u = samples[3 * b]; p = samples[3 * b + 1]; q = samples[3 * b + 2];
+      if (u < 0 || u >= n_users || p < 0 || p >= n_items || q < 0 || q >= n_items) {
+        if (l == 0) atomicOr(bad, 1);
+        u = 0; p = 0; q = 0;
+      }
+    }
+    const int64_t ru = u * nvec, rp = (n_users + p) * nvec, rn = (n_users + q) * nvec;
+    float dn = 0.f, dp = 0.f, dx = 0.f, reg = 0.f;
+    if (valid) {
+      for (int c = l; c < nvec; c += kSeedLanes) {
+        const float4 ou = __ldg(O4 + ru + c), op = __ldg(O4 + rp + c), on = __ldg(O4 + rn + c);
+        const float4 du = __ldg(dO4 + ru + c), dp4 = __ldg(dO4 + rp + c), dn4 = __ldg(dO4 + rn + c);
+        dn += dot4(ou, on);
+        dp += dot4(ou, op);
+        dx += dot4(du, make_float4(on.x - op.x, on.y - op.y, on.z - op.z, on.w - op.w)) +
+              dot4(ou, make_float4(dn4.x - dp4.x, dn4.y - dp4.y, dn4.z - dp4.z, dn4.w - dp4.w));
+        if (dloss)
+          reg += dot4(__ldg(V4 + ru + c), __ldg(E4 + ru + c)) + dot4(__ldg(V4 + rp + c), __ldg(E4 + rp + c)) +
+                 dot4(__ldg(V4 + rn + c), __ldg(E4 + rn + c));
+      }
+    }
+#pragma unroll
+    for (int o = kSeedLanes / 2; o > 0; o >>= 1) {
+      dn += __shfl_xor_sync(kFull, dn, o);
+      dp += __shfl_xor_sync(kFull, dp, o);
+      dx += __shfl_xor_sync(kFull, dx, o);
+      reg += __shfl_xor_sync(kFull, reg, o);
+    }
+    if (valid && l == 0) {
+      const float x = dn - dp;
+      float d1, d2;                                 // l'(x), l''(x)
+      if (x > 20.f) { d1 = 1.f; d2 = 0.f; }
+      else { const float z = expf(x); d1 = z / (z + 1.f); d2 = d1 * (1.f - d1); }
+      const float a = d2 * dx * inv_B, c = d1 * inv_B;
+      alpha[b] = a; alpha[n + b] = -a;
+      beta[b] = c;  beta[n + b] = -c;
+      if (dloss) dloss[b] = d1 * dx + lambda * reg;
+    }
   }
 }
 
@@ -614,16 +705,24 @@ int64_t recad_pair_scores_backward_scratch_bytes(int64_t B) {
 int recad_pair_scores_backward(const float* Xa, int64_t n_a, const float* Xb, int64_t n_b, int32_t D, const int64_t* ia,
                                const int64_t* ib, int64_t B, const float* g, float* dXa, float* dXb, float* dba, float* dbb,
                                void* scratch, int64_t scratch_bytes, void* stream) {
-  RECAD_REQUIRE(Xa && Xb && dXa && dXb && n_a > 0 && n_b > 0 && B >= 0 && (B == 0 || (ia && ib && g && scratch)),
-                RECAD_ERR_ARG, "pair_scores_backward: bad argument");
-  RECAD_REQUIRE(D >= 4 && D % 4 == 0 && D <= 1024, RECAD_ERR_UNSUPPORTED, "pair_scores_backward: D must be a multiple of 4 in [4, 1024]");
+  return recad_pair_scores_hvp(Xa, nullptr, n_a, Xb, nullptr, n_b, D, ia, ib, B, g, nullptr, dXa, dXb, dba, dbb, scratch,
+                               scratch_bytes, stream);
+}
+
+int recad_pair_scores_hvp(const float* Xa, const float* Va, int64_t n_a, const float* Xb, const float* Vb, int64_t n_b,
+                          int32_t D, const int64_t* ia, const int64_t* ib, int64_t B, const float* alpha, const float* beta,
+                          float* outA, float* outB, float* dba, float* dbb, void* scratch, int64_t scratch_bytes, void* stream) {
+  RECAD_REQUIRE(Xa && Xb && outA && outB && n_a > 0 && n_b > 0 && B >= 0 && (B == 0 || (ia && ib && alpha && scratch)),
+                RECAD_ERR_ARG, "pair_scores: bad argument");
+  RECAD_REQUIRE(!beta || (Va && Vb), RECAD_ERR_ARG, "pair_scores_hvp: beta needs Va and Vb");
+  RECAD_REQUIRE(D >= 4 && D % 4 == 0 && D <= 1024, RECAD_ERR_UNSUPPORTED, "pair_scores: D must be a multiple of 4 in [4, 1024]");
   RECAD_REQUIRE(n_a < ((int64_t)1 << 31) && n_b < ((int64_t)1 << 31) && B < ((int64_t)1 << 32) - 1, RECAD_ERR_OVERFLOW,
-                "pair_scores_backward: tables below 2^31 rows and B below 2^32 - 1");
+                "pair_scores: tables below 2^31 rows and B below 2^32 - 1");
   RECAD_REQUIRE(B == 0 || scratch_bytes >= recad_pair_scores_backward_scratch_bytes(B), RECAD_ERR_SCRATCH,
-                "pair_scores_backward: scratch too small");
+                "pair_scores: scratch too small");
   cudaStream_t s = as_stream(stream);
-  RECAD_CUDA_CHECK(cudaMemsetAsync(dXa, 0, n_a * D * sizeof(float), s));
-  RECAD_CUDA_CHECK(cudaMemsetAsync(dXb, 0, n_b * D * sizeof(float), s));
+  RECAD_CUDA_CHECK(cudaMemsetAsync(outA, 0, n_a * D * sizeof(float), s));
+  RECAD_CUDA_CHECK(cudaMemsetAsync(outB, 0, n_b * D * sizeof(float), s));
   if (dba) RECAD_CUDA_CHECK(cudaMemsetAsync(dba, 0, n_a * sizeof(float), s));
   if (dbb) RECAD_CUDA_CHECK(cudaMemsetAsync(dbb, 0, n_b * sizeof(float), s));
   if (B == 0) return RECAD_OK;
@@ -643,14 +742,43 @@ int recad_pair_scores_backward(const float* Xa, int64_t n_a, const float* Xb, in
     RECAD_LAUNCH_CHECK();
     int rc = radix_sort_u64(keys, tmp, B, bbits + bit_width(n_rows), sort_scr, s);
     if (rc) return rc;
-    pair_grad_rows_kernel<<<wgrid, 256, 0, s>>>(keys, B, bbits, g, side == 0 ? ib : ia, n_other, side == 0 ? Xb : Xa, D / 4,
-                                                side == 0 ? dXa : dXb, side == 0 ? dba : dbb);
+    const int64_t* other = side == 0 ? ib : ia;
+    const float* X = side == 0 ? Xb : Xa;
+    float* out = side == 0 ? outA : outB;
+    float* db = side == 0 ? dba : dbb;
+    if (beta)
+      pair_grad_rows_kernel<true><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, beta, other, n_other, X, side == 0 ? Vb : Va,
+                                                         D / 4, out, db);
+    else
+      pair_grad_rows_kernel<false><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, nullptr, other, n_other, X, nullptr, D / 4,
+                                                          out, db);
     RECAD_LAUNCH_CHECK();
   }
   int h_bad = 0;
   RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, s));
   RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
-  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "pair_scores_backward: an id is out of range");
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "pair_scores: an id is out of range");
+  return RECAD_OK;
+}
+
+int recad_bpr_hvp_seeds(const float* O, const float* dO, int64_t n_users, int64_t n_items, const int64_t* samples, int64_t n,
+                        int64_t B_norm, int32_t D, const float* E, const float* V, float lambda, float* alpha, float* beta,
+                        float* dloss, int32_t* bad, void* stream) {
+  RECAD_REQUIRE(O && dO && samples && alpha && beta && bad && n_users > 0 && n_items > 0 && n > 0 && B_norm > 0,
+                RECAD_ERR_ARG, "bpr_hvp_seeds: bad argument");
+  RECAD_REQUIRE(!dloss || (E && V), RECAD_ERR_ARG, "bpr_hvp_seeds: dloss needs E and V");
+  RECAD_REQUIRE(D >= 4 && D % 4 == 0 && D <= 1024, RECAD_ERR_UNSUPPORTED, "bpr_hvp_seeds: D must be a multiple of 4 in [4, 1024]");
+  cudaStream_t s = as_stream(stream);
+  RECAD_CUDA_CHECK(cudaMemsetAsync(bad, 0, sizeof(int32_t), s));
+  const int64_t want = (n * kSeedLanes + 255) / 256;
+  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sm_count() * 32));
+  bpr_hvp_seeds_kernel<<<grid, 256, 0, s>>>(O, dO, n_users, n_items, samples, n, 1.0f / (float)B_norm, D / 4, E, V, lambda,
+                                            alpha, beta, dloss, bad);
+  RECAD_LAUNCH_CHECK();
+  int32_t h_bad = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "bpr_hvp_seeds: an id is out of range");
   return RECAD_OK;
 }
 

@@ -127,6 +127,61 @@ static int check_mf(const recad_mf* st, bool train) {
   return RECAD_OK;
 }
 
+// Seeds of the BCE loss's Hessian-vector product (recad_mf_hvp_seeds), 16 lanes per row.  Along the direction (dUe, dUb,
+// dIe, dIb): dy = <dUe_u, Ie_i> + <Ue_u, dIe_i> + dUb_u + dIb_i, l' = sigmoid(y) - label, l'' = sigmoid (1 - sigmoid);
+// alpha[b] = l'' dy / B, beta[b] = l' / B, dloss[b] = l' dy.
+__global__ void __launch_bounds__(256)
+mf_hvp_seeds_kernel(const float* __restrict__ Ue, const float* __restrict__ Ub, const float* __restrict__ Ie,
+                    const float* __restrict__ Ib, float mean, int64_t n_users, int64_t n_items,
+                    const int64_t* __restrict__ samples, int64_t n, float inv_B, int nvec, const float* __restrict__ dUe,
+                    const float* __restrict__ dUb, const float* __restrict__ dIe, const float* __restrict__ dIb,
+                    float* __restrict__ alpha, float* __restrict__ beta, float* __restrict__ dloss, int* __restrict__ bad) {
+  constexpr int LPR = 16;
+  const int l = threadIdx.x % LPR;
+  const int64_t group = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / LPR;
+  const int64_t n_groups = (int64_t)gridDim.x * blockDim.x / LPR;
+  const int64_t iters = (n + n_groups - 1) / n_groups;       // the same count on every lane: the shuffles are warp-wide
+  const float4* __restrict__ U4 = reinterpret_cast<const float4*>(Ue);
+  const float4* __restrict__ I4 = reinterpret_cast<const float4*>(Ie);
+  const float4* __restrict__ dU4 = reinterpret_cast<const float4*>(dUe);
+  const float4* __restrict__ dI4 = reinterpret_cast<const float4*>(dIe);
+  for (int64_t it = 0; it < iters; ++it) {
+    const int64_t b = it * n_groups + group;
+    const bool valid = b < n;
+    int64_t u = 0, i = 0, label = 0;
+    if (valid) {
+      u = samples[3 * b]; i = samples[3 * b + 1]; label = samples[3 * b + 2];
+      if (u < 0 || u >= n_users || i < 0 || i >= n_items) {
+        if (l == 0) atomicOr(bad, 1);
+        u = 0; i = 0;
+      }
+    }
+    float dot = 0.f, dy = 0.f;
+    if (valid) {
+      for (int c = l; c < nvec; c += LPR) {
+        const float4 a = __ldg(U4 + u * nvec + c), q = __ldg(I4 + i * nvec + c);
+        const float4 da = __ldg(dU4 + u * nvec + c), dq = __ldg(dI4 + i * nvec + c);
+        dot += a.x * q.x + a.y * q.y + a.z * q.z + a.w * q.w;
+        dy += da.x * q.x + da.y * q.y + da.z * q.z + da.w * q.w + a.x * dq.x + a.y * dq.y + a.z * dq.z + a.w * dq.w;
+      }
+    }
+#pragma unroll
+    for (int o = LPR / 2; o > 0; o >>= 1) {
+      dot += __shfl_xor_sync(kFull, dot, o);
+      dy += __shfl_xor_sync(kFull, dy, o);
+    }
+    if (valid && l == 0) {
+      const float x = dot + __ldg(Ub + u) + __ldg(Ib + i) + mean;
+      const float sig = 1.f / (1.f + expf(-x));
+      const float d1 = sig - (float)label, d2 = sig * (1.f - sig);
+      const float t = dy + __ldg(dUb + u) + __ldg(dIb + i);
+      alpha[b] = d2 * t * inv_B;
+      beta[b] = d1 * inv_B;
+      if (dloss) dloss[b] = d1 * t;
+    }
+  }
+}
+
 }  // namespace recad
 
 using namespace recad;
@@ -201,6 +256,27 @@ int recad_mf_grad(const recad_mf* st, const int64_t* samples, const int64_t* per
   for (int k = 0; k < 4; ++k) RECAD_CUDA_CHECK(cudaMemsetAsync(G[k], 0, sz[k] * sizeof(float), s));
   if (B == 0) return RECAD_OK;     // a rank may own no row of a short last batch: its gradient is zero
   return launch_mf<true>(st, nullptr, nullptr, samples, perm, B, B_norm, nullptr, s);
+}
+
+int recad_mf_hvp_seeds(const recad_mf* st, const float* dUe, const float* dUb, const float* dIe, const float* dIb,
+                       const int64_t* samples, int64_t n, int64_t B_norm, float* alpha, float* beta, float* dloss, int32_t* bad,
+                       void* stream) {
+  int rc = check_mf(st, false);
+  if (rc) return rc;
+  RECAD_REQUIRE(dUe && dUb && dIe && dIb && samples && alpha && beta && bad && n > 0 && B_norm > 0, RECAD_ERR_ARG,
+                "mf_hvp_seeds: bad argument");
+  cudaStream_t s = as_stream(stream);
+  RECAD_CUDA_CHECK(cudaMemsetAsync(bad, 0, sizeof(int32_t), s));
+  const int64_t want = (n * 16 + 255) / 256;
+  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sm_count() * 32));
+  mf_hvp_seeds_kernel<<<grid, 256, 0, s>>>(st->Ue, st->Ub, st->Ie, st->Ib, st->mean, st->n_users, st->n_items, samples, n,
+                                           1.0f / (float)B_norm, st->D / 4, dUe, dUb, dIe, dIb, alpha, beta, dloss, bad);
+  RECAD_LAUNCH_CHECK();
+  int32_t h_bad = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "mf_hvp_seeds: an id is out of range");
+  return RECAD_OK;
 }
 
 }  // extern "C"

@@ -470,20 +470,68 @@ def pair_scores_backward(Xa, Xb, ia, ib, g, bias=False):
     """Gradient of s_b = <Xa[ia_b], Xb[ib_b]> (+ ba[ia_b] + bb[ib_b]) for the upstream gradient g (recad_pair_scores_backward):
     (dX [n_a + n_b, D] with the rows of Xa first, dba [n_a], dbb [n_b]); the bias gradients are None unless `bias`.
     Atomic-free: the same bits on every run at any batch size.  An id out of range raises RecadError."""
-    _need_cuda(Xa, Xb, ia, ib, g)
+    return pair_scores_hvp(Xa, None, Xb, None, ia, ib, g, None, bias)
+
+
+def pair_scores_hvp(Xa, Va, Xb, Vb, ia, ib, alpha, beta, bias=False):
+    """out[r] = sum over the b with ia_b = r of (alpha_b Xb[ib_b] + beta_b Vb[ib_b]) for the rows of A, and the same with
+    Xa / Va for the rows of B (recad_pair_scores_hvp): (out [n_a + n_b, D] with the rows of A first, dba [n_a], dbb [n_b] =
+    the sums of alpha per row, None unless `bias`).  beta None: the pair backward, and Va / Vb are not read.  Atomic-free and
+    bit-stable; an id out of range raises RecadError."""
+    _need_cuda(Xa, Va, Xb, Vb, ia, ib, alpha, beta)
     dev = Xa.device
     (n_a, D), n_b, B = Xa.shape, Xb.shape[0], ia.numel()
     L = _lib.lib()
     with torch.cuda.device(dev):
-        dX = torch.empty((n_a + n_b, D), dtype=torch.float32, device=dev)
+        out = torch.empty((n_a + n_b, D), dtype=torch.float32, device=dev)
         dba = torch.empty(n_a, dtype=torch.float32, device=dev) if bias else None
         dbb = torch.empty(n_b, dtype=torch.float32, device=dev) if bias else None
         nbytes = int(L.recad_pair_scores_backward_scratch_bytes(B))
         scratch = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
-        check(L.recad_pair_scores_backward(_ptr(Xa), n_a, _ptr(Xb), n_b, D, _ptr(ia), _ptr(ib), B, _ptr(g), _ptr(dX[:n_a]),
-                                           _ptr(dX[n_a:]), _ptr(dba), _ptr(dbb), _ptr(scratch), nbytes, _stream(dev)),
-              "recad_pair_scores_backward")
-    return dX, dba, dbb
+        if beta is None:
+            check(L.recad_pair_scores_backward(_ptr(Xa), n_a, _ptr(Xb), n_b, D, _ptr(ia), _ptr(ib), B, _ptr(alpha),
+                                               _ptr(out[:n_a]), _ptr(out[n_a:]), _ptr(dba), _ptr(dbb), _ptr(scratch), nbytes,
+                                               _stream(dev)), "recad_pair_scores_backward")
+        else:
+            check(L.recad_pair_scores_hvp(_ptr(Xa), _ptr(Va), n_a, _ptr(Xb), _ptr(Vb), n_b, D, _ptr(ia), _ptr(ib), B, _ptr(alpha),
+                                          _ptr(beta), _ptr(out[:n_a]), _ptr(out[n_a:]), _ptr(dba), _ptr(dbb), _ptr(scratch), nbytes,
+                                          _stream(dev)), "recad_pair_scores_hvp")
+    return out, dba, dbb
+
+
+def bpr_hvp_seeds(O, dO, n_users, samples, lam=0.0, E=None, V=None, dloss=False):
+    """Seeds of the BPR loss's Hessian-vector product over the rows samples int64 [n, 3] (recad_bpr_hvp_seeds, B = n):
+    (alpha [2n], beta [2n], dloss [n] or None) for the pairs (u, neg) then (u, pos).  With `dloss`, each sample's derivative
+    along V, l'(x_b) dx_b + lam (<V_u, E_u> + <V_p, E_p> + <V_n, E_n>), where dO = P V."""
+    _need_cuda(O, dO, samples, E, V)
+    dev = O.device
+    N, D = O.shape
+    n = samples.shape[0]
+    with torch.cuda.device(dev):
+        alpha = torch.empty(2 * n, dtype=torch.float32, device=dev)
+        beta = torch.empty(2 * n, dtype=torch.float32, device=dev)
+        dl = torch.empty(n, dtype=torch.float32, device=dev) if dloss else None
+        bad = torch.empty(1, dtype=torch.int32, device=dev)
+        check(_lib.lib().recad_bpr_hvp_seeds(_ptr(O), _ptr(dO), n_users, N - n_users, _ptr(samples), n, n, D,
+                                             _ptr(E if dloss else None), _ptr(V if dloss else None), float(lam), _ptr(alpha),
+                                             _ptr(beta), _ptr(dl), _ptr(bad), _stream(dev)), "recad_bpr_hvp_seeds")
+    return alpha, beta, dl
+
+
+def mf_hvp_seeds(st, dUe, dUb, dIe, dIb, samples, dloss=False):
+    """Seeds of the BCE loss's Hessian-vector product over the (user, item, label) rows samples int64 [n, 3] of an MF state
+    along (dUe, dUb, dIe, dIb) (recad_mf_hvp_seeds, B = n): (alpha [n], beta [n], dloss [n] or None)."""
+    _need_cuda(dUe, dUb, dIe, dIb, samples)
+    dev = samples.device
+    n = samples.shape[0]
+    with torch.cuda.device(dev):
+        alpha = torch.empty(n, dtype=torch.float32, device=dev)
+        beta = torch.empty(n, dtype=torch.float32, device=dev)
+        dl = torch.empty(n, dtype=torch.float32, device=dev) if dloss else None
+        bad = torch.empty(1, dtype=torch.int32, device=dev)
+        check(_lib.lib().recad_mf_hvp_seeds(C.byref(st), _ptr(dUe), _ptr(dUb), _ptr(dIe), _ptr(dIb), _ptr(samples), n, n,
+                                            _ptr(alpha), _ptr(beta), _ptr(dl), _ptr(bad), _stream(dev)), "recad_mf_hvp_seeds")
+    return alpha, beta, dl
 
 
 def lightgcn_backward(st, gO):

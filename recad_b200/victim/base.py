@@ -102,6 +102,37 @@ class BaseVictim(LazyMixin, torch.nn.Module):
         if users.numel() and bool(((users < 0) | (users >= n_users)).any() | ((items < 0) | (items >= n_items)).any()):
             raise ops.RecadError("a user or item id is out of range")
 
+    def _loss_rows(self, batch, what):
+        """The train_step rows of a caller's batch dict (keys of input_describe()["train_step"], int64 CUDA [n] each on
+        the model's device) as one int64 [n, 3] tensor; RecadError otherwise.  Ids are range-checked by the kernels."""
+        names = tuple(self.input_describe()["train_step"])
+        if not isinstance(batch, dict) or set(names) - set(batch):
+            raise ops.RecadError(f"{what}: batch must be a dict with the keys {names}")
+        cols = [batch[k] for k in names]
+        for k, c in zip(names, cols):
+            if not isinstance(c, torch.Tensor) or not c.is_cuda or c.device != self._dev:
+                raise ops.RecadError(f"{what}: batch[{k!r}] must be a CUDA tensor on {self._dev}")
+            if c.dtype != torch.int64 or c.dim() != 1:
+                raise ops.RecadError(f"{what}: batch[{k!r}] must be int64 [n], got {c.dtype} {list(c.shape)}")
+        n = cols[0].numel()
+        if n == 0 or any(c.numel() != n for c in cols):
+            raise ops.RecadError(f"{what}: the batch columns must have the same positive length")
+        return torch.stack([c.detach() for c in cols], 1).contiguous()
+
+    def _check_vectors(self, vectors, shapes, what):
+        """RecadError unless `vectors` is a sequence of float32 CUDA tensors on the model's device with the given shapes
+        (the trainable tables in parameters() order); returns them detached and contiguous."""
+        if not isinstance(vectors, (tuple, list)) or len(vectors) != len(shapes):
+            raise ops.RecadError(f"{what}: vectors must be a tuple of {len(shapes)} tensors shaped {shapes}")
+        out = []
+        for v, shp in zip(vectors, shapes):
+            if not isinstance(v, torch.Tensor) or not v.is_cuda or v.device != self._dev:
+                raise ops.RecadError(f"{what}: vectors must be CUDA tensors on {self._dev}")
+            if v.dtype != torch.float32 or tuple(v.shape) != tuple(shp):
+                raise ops.RecadError(f"{what}: float32 {list(shp)} needed, got {v.dtype} {list(v.shape)}")
+            out.append(v.detach().contiguous())
+        return out
+
     @staticmethod
     def _vp(t):
         return C.c_void_p(t.data_ptr()) if t is not None else None

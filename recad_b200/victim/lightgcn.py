@@ -277,6 +277,49 @@ class LightGCN(BaseVictim):
         U = self.num_users
         return ops.fullrank_eval(O[:U], O[U:], user_ids, train_rowptr, train_col, targets, K) + (0.0,)
 
+    # ------------------------------------------------------------------ second order
+    def _loss_directions(self, batch, vectors, what):
+        """Rows, the direction V [N, D], O = P E and dO = P V for the training loss of `batch` (fresh buffers: the model's
+        tables, moments and cached propagation are not touched)."""
+        self._require_instance(what)
+        if self.dropout and self.training:
+            raise ops.RecadError(f"LightGCN.{what}: not defined under graph dropout in training mode (call eval() first)")
+        samples = self._loss_rows(batch, f"LightGCN.{what}")
+        U, I, D = self.num_users, self.num_items, self.latent_dim
+        vu, vi = self._check_vectors(vectors, [(U, D), (I, D)], f"LightGCN.{what}")
+        with torch.cuda.device(self._dev):
+            V = torch.cat([vu, vi])
+            O, _ = ops.lightgcn_propagate_layers(self._st, self.E, keep=False)
+            dO, _ = ops.lightgcn_propagate_layers(self._st, V, keep=False)
+        return samples, V, O, dO
+
+    def loss_hvp(self, batch, vectors):
+        """H v for the BPR training loss of `batch` taken as one batch (what train_step minimises for it: mean softplus +
+        lambda * 0.5 * sum of the squared rows / n), H its Hessian with respect to (embedding_user.weight,
+        embedding_item.weight) at the current tables.  batch: dict of int64 CUDA [n] users / positive_items /
+        negative_items; vectors: (v_user [U, D], v_item [I, D]) float32.  Returns (Hv_user, Hv_item).  Deterministic; the
+        model is not changed.  H v = P^T H_O (P v) + (lambda / n) cnt * v (DESIGN.md, "Second order")."""
+        samples, V, O, dO = self._loss_directions(batch, vectors, "loss_hvp")
+        U, N, n = self.num_users, self.num_users + self.num_items, samples.shape[0]
+        lam = float(self.config["lambda"])
+        with torch.cuda.device(self._dev):
+            alpha, beta, _ = ops.bpr_hvp_seeds(O, dO, U, samples)
+            u, p, q = samples.unbind(1)
+            HO, _, _ = ops.pair_scores_hvp(O[:U], dO[:U], O[U:], dO[U:], torch.cat([u, u]), torch.cat([q, p]), alpha, beta)
+            hv = ops.lightgcn_backward(self._st, HO)
+            cnt = torch.bincount(torch.cat([u, p + U, q + U]), minlength=N)       # exact integer multiplicities
+            hv.addcmul_(V, (cnt.float() * (lam / n)).unsqueeze(1))
+        return hv[:U], hv[U:]
+
+    def sample_directional_derivatives(self, batch, vectors):
+        """For every row b of `batch`, the derivative of its own loss l_b = softplus(x_b) + lambda * 0.5 * (|E_u|^2 + |E_p|^2 +
+        |E_n|^2) along `vectors` (shaped as for loss_hvp): <grad l_b, v>, float32 [n], unnormalised (the batch loss is the
+        mean of the l_b).  Deterministic; the model is not changed."""
+        samples, V, O, dO = self._loss_directions(batch, vectors, "sample_directional_derivatives")
+        with torch.cuda.device(self._dev):
+            _, _, dloss = ops.bpr_hvp_seeds(O, dO, self.num_users, samples, float(self.config["lambda"]), self.E, V, dloss=True)
+        return dloss
+
     def input_describe(self):
         return {
             "train_step": {"users": (torch.int64, "batch"), "positive_items": (torch.int64, "batch"),

@@ -132,6 +132,35 @@ class MF(BaseVictim):
             score = score + self.user_bias.weight.view(-1)[user_ids].unsqueeze(1)
         return topi, topv, rank, score, self.mean_value
 
+    # ------------------------------------------------------------------ second order
+    def _loss_seeds(self, batch, vectors, what, dloss):
+        self._require_instance(what)
+        samples = self._loss_rows(batch, f"MF.{what}")
+        U, I, D = self.num_users, self.num_items, self.D
+        vecs = self._check_vectors(vectors, [(U, D), (U, 1), (I, D), (I, 1)], f"MF.{what}")
+        self._sync_mean()
+        with torch.cuda.device(self._dev):
+            alpha, beta, dl = ops.mf_hvp_seeds(self._st, *vecs, samples, dloss=dloss)
+        return samples, vecs, alpha, beta, dl
+
+    def loss_hvp(self, batch, vectors):
+        """H v for the BCE training loss of `batch` taken as one batch (what train_step minimises for it), H its Hessian
+        with respect to (user_emb, user_bias, item_emb, item_bias) at the current tables, `mean` held constant.
+        batch: dict of int64 CUDA [n] users / items / labels; vectors: (v_Ue [U, D], v_Ub [U, 1], v_Ie [I, D], v_Ib [I, 1])
+        float32.  Returns the four products shaped likewise.  Deterministic; the model is not changed."""
+        samples, (vUe, _, vIe, _), alpha, beta, _ = self._loss_seeds(batch, vectors, "loss_hvp", False)
+        U, I = self.num_users, self.num_items
+        with torch.cuda.device(self._dev):
+            out, hUb, hIb = ops.pair_scores_hvp(self.user_emb.weight.detach(), vUe, self.item_emb.weight.detach(), vIe,
+                                                samples[:, 0].contiguous(), samples[:, 1].contiguous(), alpha, beta, bias=True)
+        return out[:U], hUb.view(U, 1), out[U:], hIb.view(I, 1)
+
+    def sample_directional_derivatives(self, batch, vectors):
+        """For every row b of `batch`, the derivative of its own BCE loss along `vectors` (shaped as for loss_hvp):
+        <grad l_b, v>, float32 [n], unnormalised (the batch loss is the mean of the l_b).  Deterministic; the model is not
+        changed."""
+        return self._loss_seeds(batch, vectors, "sample_directional_derivatives", True)[4]
+
     def input_describe(self):
         return {
             "train_step": {"users": (torch.int64, "batch"), "items": (torch.int64, "batch"), "labels": (torch.int64, "batch")},
