@@ -592,6 +592,19 @@ int recad_ncf_grad(const recad_ncf* st, const int64_t* samples, const int64_t* p
  * stream: an id out of range gives RECAD_ERR_ARG (no memory outside the tables is addressed). */
 int recad_ncf_backward(const recad_ncf* st, const int64_t* users, const int64_t* items, int64_t B, const float* dpred,
                        float* grads, void* stream);
+/* Hessian-vector product of the training loss (ncf.py:112-153): L = (1/n) sum_b BCEWithLogits(pred_b, label_b) over the n rows
+ * samples [dev] int64[n, 3] = (user, item, label) taken as one batch (what train_step minimises for it; no regulariser, no
+ * dropout), at the current parameters, in the model's tower precision.  vec [dev] float[n_params] is the direction in the
+ * layout of recad_ncf_layout; out [dev] float[n_params] (NULL: not wanted) = H vec, written whole (padding zero; the branch a
+ * variant does not read gets exactly zero); dloss [dev] float[n] (NULL: not wanted) = each row's unnormalised directional
+ * derivative l'_b dpred_b = <grad l_b, vec>.  With out NULL only the R-forward and the seeds run.  Rows are processed in
+ * chunks of max_batch, in order, the seeds normalised by the full n; no atomics, so the result is bit-stable at any n.
+ * work [dev] float[work_floats], work_floats >= recad_ncf_hvp_work_floats(factor, n_layers, st->max_batch); st->work is
+ * used as well.  st->params, m, v, grads and loss_acc are not touched.  Synchronises the stream: an id outside its table
+ * gives RECAD_ERR_ARG (no memory outside the tables is addressed). */
+int64_t recad_ncf_hvp_work_floats(int32_t factor, int32_t n_layers, int64_t max_batch);
+int recad_ncf_hvp(const recad_ncf* st, const int64_t* samples, int64_t n, const float* vec, float* out, float* dloss,
+                  float* work, int64_t work_floats, void* stream);
 
 /* The tensor-core GEMM of the NCF tower, exposed for testing: C[M, N] = A[M, K] . B[N, K]^T (+ bias[N]) (ReLU) on
  * tcgen05 (kind::tf32, fp32 accumulators in TMEM, TMA operands) with the 3xTF32 operand split, i.e. fp32-accurate.

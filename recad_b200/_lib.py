@@ -153,6 +153,8 @@ SIGNATURES = {
     "recad_ncf_graph_launches": (i64, []),
     "recad_ncf_grad": (C.c_int, [C.POINTER(NCF), vp, vp, i64, i64, vp]),
     "recad_ncf_backward": (C.c_int, [C.POINTER(NCF), vp, vp, i64, vp, vp, vp]),
+    "recad_ncf_hvp_work_floats": (i64, [i32, i32, i64]),
+    "recad_ncf_hvp": (C.c_int, [C.POINTER(NCF), vp, i64, vp, vp, vp, vp, i64, vp]),
     "recad_gemm_tn_tf32x3": (C.c_int, [vp, vp, i32, i32, i32, vp, i32, vp, vp, vp]),
     "recad_transpose_items": (C.c_int, [vp, i64, i32, vp, i64, vp]),
     "recad_fullrank_eval": (C.c_int, [vp, vp, i64, i64, i32, vp, i64, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp]),

@@ -1,7 +1,7 @@
 """Influence of training rows on an objective, from the victims' Hessian-vector products (loss_hvp) and per-row
 directional derivatives (sample_directional_derivatives) -- the estimate -grad(obj)^T H^-1 grad(l_z) of influence-function
 attacks and defenses (Fang et al., WWW 2020).  H is the Hessian of the training loss of the given rows taken as one batch,
-at the victim's current tables.  Works with any victim that has those two methods (LightGCN, MF)."""
+at the victim's current tables.  Works with any victim that has those two methods (LightGCN, MF, NCF)."""
 import math
 from collections import namedtuple
 

@@ -534,6 +534,25 @@ def mf_hvp_seeds(st, dUe, dUb, dIe, dIb, samples, dloss=False):
     return alpha, beta, dl
 
 
+def ncf_hvp(st, samples, vec_flat, out=True, dloss=False):
+    """Hessian-vector product of an NCF state's BCE training loss over the (user, item, label) rows samples int64 [n, 3] taken
+    as one batch, along vec_flat float32 [n_params] (recad_ncf_layout order) (recad_ncf_hvp): (H v [n_params] or None,
+    dloss [n] or None), dloss[b] = <grad l_b, v>.  Deterministic; the state's parameters, moments and loss accumulator are not
+    touched.  An id out of range raises RecadError."""
+    _need_cuda(samples, vec_flat)
+    dev = samples.device
+    n = samples.shape[0]
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        hv = torch.empty(st.n_params, dtype=torch.float32, device=dev) if out else None
+        dl = torch.empty(n, dtype=torch.float32, device=dev) if dloss else None
+        wf = int(L.recad_ncf_hvp_work_floats(st.factor, st.n_layers, st.max_batch))
+        work = torch.empty(max(wf, 1), dtype=torch.float32, device=dev)
+        check(L.recad_ncf_hvp(C.byref(st), _ptr(samples), n, _ptr(vec_flat), _ptr(hv), _ptr(dl), _ptr(work), wf, _stream(dev)),
+              "recad_ncf_hvp")
+    return hv, dl
+
+
 def lightgcn_backward(st, gO):
     """gE = (1 / (L + 1)) sum_l (A^T)^l gO (recad_lightgcn_backward) for a LightGCN state; the Horner loop runs through work
     buffers of its own, so the state's X0 / X1 are left alone."""

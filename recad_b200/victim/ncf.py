@@ -239,6 +239,33 @@ class NCF(BaseVictim):
                 outs.append(ops.rank_from_scores(scores, ub, train_rowptr, train_col, targets, K))
         return tuple(torch.cat([o[k] for o in outs]) for k in range(4)) + (0.0,)
 
+    # ------------------------------------------------------------------ second order
+    def _hvp(self, batch, vectors, what, out, dloss):
+        self._require_instance(what)
+        samples = self._loss_rows(batch, f"NCF.{what}")
+        vecs = self._check_vectors(vectors, [s for _, _, s in self._grad_slots], f"NCF.{what}")
+        with torch.cuda.device(self._dev):
+            flat = torch.zeros(self._st.n_params, dtype=torch.float32, device=self._dev)    # layout padding stays zero
+            for (off, n, _), v in zip(self._grad_slots, vecs):
+                flat[off:off + n] = v.view(-1)
+            return ops.ncf_hvp(self._st, samples, flat, out=out, dloss=dloss)
+
+    def loss_hvp(self, batch, vectors):
+        """H v for the BCE training loss of `batch` taken as one batch (what train_step minimises for it; no regulariser),
+        H its Hessian with respect to every parameter at the current values, in the model's tower precision.
+        batch: dict of int64 CUDA [n] users / items / labels; vectors: one float32 tensor per parameter, shaped as
+        parameters() (embed_user_GMF, embed_item_GMF, embed_user_MLP, embed_item_MLP, each MLP layer's weight and bias,
+        predict weight and bias).  Returns the product shaped the same way; parameters the variant does not read get exactly
+        zero.  Deterministic; the model is not changed."""
+        hv, _ = self._hvp(batch, vectors, "loss_hvp", True, False)
+        return tuple(hv[off:off + n].view(shape) for off, n, shape in self._grad_slots)
+
+    def sample_directional_derivatives(self, batch, vectors):
+        """For every row b of `batch`, the derivative of its own BCE loss along `vectors` (shaped as for loss_hvp):
+        <grad l_b, v>, float32 [n], unnormalised (the batch loss is the mean of the l_b).  Deterministic; the model is not
+        changed."""
+        return self._hvp(batch, vectors, "sample_directional_derivatives", False, True)[1]
+
     def input_describe(self):
         return {
             "train_step": {"users": (torch.int64, "batch"), "items": (torch.int64, "batch"), "labels": (torch.int64, "batch")},
