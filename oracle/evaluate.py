@@ -95,19 +95,42 @@ def full_rank_batched(user_emb, item_emb, user_ids, train_indptr, train_indices,
     return topi, topv, trank, tscore
 
 
+_F32_OVERFLOW_MID = 2.0 ** 128 - 2.0 ** 103      # halfway between FLT_MAX and 2^128: rounds to inf
+
+
+def fmaf(a, b, c):
+    """Correctly rounded float32 fused multiply-add a * b + c, elementwise (numpy broadcasting).
+    The product of two float32 is exact in float64; the float64 sum s = p + c is not, and rounding it
+    to float32 rounds twice.  That differs from one rounding of the exact sum only when s lies exactly
+    on a float32 rounding midpoint while the exact sum does not, so the sum's rounding error e is
+    recovered exactly (TwoSum) and, in that case, s is moved one float64 ulp toward e before the
+    cast, which puts it on the same side of the midpoint as the exact sum."""
+    p = np.asarray(a, dtype=np.float32).astype(np.float64) * np.asarray(b, dtype=np.float32).astype(np.float64)
+    c = np.asarray(c, dtype=np.float32).astype(np.float64)
+    with np.errstate(invalid="ignore", over="ignore"):
+        s = p + c
+        bb = s - p
+        e = (p - (s - bb)) + (c - bb)                       # TwoSum: p + c == s + e exactly (finite s)
+        r32 = s.astype(np.float32)
+        r = r32.astype(np.float64)
+        # the other float32 neighbour of s; s is a midpoint iff it is the mean of the two (exact in float64)
+        n = np.nextafter(r32, np.where(s > r, np.float32(np.inf), np.float32(-np.inf))).astype(np.float64)
+        mid = (np.isfinite(r) & (s != r) & ((r + n) * 0.5 == s)) | (np.abs(s) == _F32_OVERFLOW_MID)
+        mid &= e != 0
+        s = np.where(mid, np.nextafter(s, np.where(e > 0, np.inf, -np.inf)), s)
+        return s.astype(np.float32)
+
+
 def fma_dot_rows(u, items):
     """Float32 dot of one user row against every item row, accumulated with a
-    fused multiply-add per dimension in ascending d (acc = fma(u[d], i[d], acc)).
-    Emulated exactly in float64: the product of two float32 is exact in float64
-    and one rounding to float32 per step equals a hardware FMA (double rounding
-    cannot occur: the float64 sum of an exact 48-bit product and a 24-bit addend
-    is rounded once to 53 bits, then to 24; innocuous except in vanishingly rare
-    half-way cases, which the tests tolerate through the tie rule)."""
+    fused multiply-add per dimension in ascending d (acc = fma(u[d], i[d], acc)),
+    each step correctly rounded as a hardware FMA is (fmaf above): bit for bit
+    the exact CUDA-core kernel's chain."""
     acc = np.zeros(items.shape[0], dtype=np.float32)
-    u64 = u.astype(np.float64)
-    it64 = items.astype(np.float64)
+    u = np.asarray(u, dtype=np.float32)
+    items = np.asarray(items, dtype=np.float32)
     for d in range(items.shape[1]):
-        acc = (u64[d] * it64[:, d] + acc.astype(np.float64)).astype(np.float32)
+        acc = fmaf(u[d], items[:, d], acc)
     return acc
 
 

@@ -59,12 +59,18 @@ struct TcTargets {
   int32_t id[kTcMaxT];
 };
 
-// f = 2^k and 1 / f, both normal: beyond |k| = 126 the rescale is no longer exact (scores below 2^-100 or above 2^100
-// of the operands' own magnitude), elsewhere it is
-__device__ __forceinline__ void pow2_pair(int k, float& f, float& inv) {
-  k = max(-126, min(126, k));
-  f = __int_as_float((127 + k) << 23);
-  inv = __int_as_float((127 - k) << 23);
+// The MMAs leave a tile's scores scaled by 2^k, k = ku + kt, and the epilogue scales thresholds and bias into that
+// domain.  2^k is one normal fp32 only for |k| <= 126, but k reaches beyond when the user row's and the tile's largest
+// |x| multiply to below about 2^-96 (both 1 * 2^-50: k = 128) or above 2^156, so it is carried as two factors:
+// 2^k = f f2 with f = 2^ka, ka = k held to [-126, 126], and f2 = 2^(k - ka) held to the same range, inv = 1 / f.
+// Every rescale is exact for |k| <= 252 (f2 = 1 for |k| <= 126: the common case costs nothing); beyond, only for
+// operands whose every score is below fp32's smallest subnormal or above its largest value.
+__device__ __forceinline__ void pow2_pair(int k, float& f, float& inv, float& f2) {
+  const int ka = max(-126, min(126, k));
+  const int kb = max(-126, min(126, k - ka));
+  f = __int_as_float((127 + ka) << 23);
+  inv = __int_as_float((127 - ka) << 23);
+  f2 = __int_as_float((127 + kb) << 23);
 }
 
 // one arrival per warp on an mbarrier counted in warps (its lanes' TMEM loads have completed: tcgen05.wait::ld)
@@ -236,20 +242,20 @@ fullrank_tc_kernel(const __grid_constant__ TcMaps maps, const TcTargets tgt, con
       uint32_t v[16];
       tmem_ld16(lane_addr, v);
       tmem_ld_wait();
-      float f, inv;
-      pow2_pair(ku + __ldg(kexp + n_tiles), f, inv);
+      float f, inv, f2;
+      pow2_pair(ku + __ldg(kexp + n_tiles), f, inv, f2);
 #pragma unroll
       for (int t = 0; t < TMAX; ++t)
         if (t < T) {
           const float s = __uint_as_float(v[t]);
-          rank_state_set_score(rs, t, (item_bias ? fmaf(__ldg(item_bias + rs.tg[t]), f, s) : s) * inv);
+          rank_state_set_score(rs, t, (item_bias ? fmaf(__ldg(item_bias + rs.tg[t]) * f2, f, s) : s) * inv * pow2_inv(f2));
         }
     }
     tc_fence_before();
     warp_arrive(bar_acc_empty(0), 1);                // all 8 warps read the target tile
 
     // one 32-score chunk, in registers: bias, -inf for train / padding / idle, rank counters, top-K
-    auto chunk = [&](const uint32_t (&v)[32], int base, uint32_t train_mask, float f, float inv) {
+    auto chunk = [&](const uint32_t (&v)[32], int base, uint32_t train_mask, float f, float inv, float f2) {
       const int lim = min(32, (int)n_items - base);
       if (lim <= 0) return;                          // warp-uniform
       float s[32];
@@ -257,14 +263,14 @@ fullrank_tc_kernel(const __grid_constant__ TcMaps maps, const TcTargets tgt, con
       for (int e = 0; e < 32; ++e) s[e] = __uint_as_float(v[e]);
       if (item_bias) {                               // uniform addresses: one broadcast load per item
 #pragma unroll
-        for (int e = 0; e < 32; ++e) s[e] = (e < lim) ? fmaf(__ldg(item_bias + base + e), f, s[e]) : s[e];
+        for (int e = 0; e < 32; ++e) s[e] = (e < lim) ? fmaf(__ldg(item_bias + base + e) * f2, f, s[e]) : s[e];
       }
       const uint32_t drop = train_mask | (lim < 32 ? ~0u << lim : 0u) | (active ? 0u : ~0u);
       if (drop) {
 #pragma unroll
         for (int e = 0; e < 32; ++e) s[e] = ((drop >> e) & 1u) ? -INFINITY : s[e];
       }
-      rank_topk_chunk<32, TMAX>(s, base, T, rs, tau, myv, myi, K, 1, 0, min_pos, f, inv);
+      rank_topk_chunk<32, TMAX>(s, base, T, rs, tau, myv, myi, K, 1, 0, min_pos, f, inv, f2);
     };
 
     // warpgroup w ranks the whole tiles j = 1 + w, 3 + w, ...: the per-tile work (barrier, train mask, scale) is paid
@@ -285,8 +291,8 @@ fullrank_tc_kernel(const __grid_constant__ TcMaps maps, const TcTargets tgt, con
       }
       const int kt = kt_next;
       if (j + 2 <= nt) kt_next = __ldg(kexp + j + 1);
-      float f, inv;
-      pow2_pair(ku + kt, f, inv);
+      float f, inv, f2;
+      pow2_pair(ku + kt, f, inv, f2);
       mbar_wait(bar_acc_full(a), (uint32_t)(j / kTcAcc) & 1);
       tc_fence_after();
       if (dbg == 2) {                                // (profiling aid: TMA + MMA pipeline only)
@@ -297,13 +303,13 @@ fullrank_tc_kernel(const __grid_constant__ TcMaps maps, const TcTargets tgt, con
       uint32_t v[32];
       tmem_ld32(lane_addr + a * kTcN, v);
       tmem_ld_wait();
-      chunk(v, j0, m0, f, inv);
+      chunk(v, j0, m0, f, inv, f2);
       tmem_ld32(lane_addr + a * kTcN + 32, v);
       tmem_ld_wait();
       // the tile now lives in registers: hand the accumulator back BEFORE ranking its second half
       tc_fence_before();
       warp_arrive(bar_acc_empty(a), 2);              // the 4 warps of one warpgroup stand for all 8
-      chunk(v, j0 + 32, m1, f, inv);
+      chunk(v, j0 + 32, m1, f, inv, f2);
     }
     // merge: warpgroup 1 hands over its counts; its K-best list already sits next to warpgroup 0's
     if (wg == 1) {

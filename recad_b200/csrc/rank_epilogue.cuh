@@ -11,7 +11,9 @@
 //   * the top-K list is touched only when the chunk maximum beats the current K-th best.
 // The tensor-core kernel hands over scores in a power-of-two scaled domain, s' = s f (f = 2^k, exact): the thresholds
 // are scaled instead of the scores (s' > thr f  <=>  s > thr), and only a score entering the list is scaled back
-// (s' inv).  The exact kernel passes f = inv = 1.
+// (s' inv).  f may need two factors, f f2 (a scale beyond 2^126 is not one fp32): thresholds are multiplied by f, then
+// by f2, and a score entering the list by inv, then by 1 / f2 (pow2_inv: exact, f2 is a normal power of two).  The exact kernel
+// passes f = inv = f2 = 1.
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -67,6 +69,9 @@ static __device__ __noinline__ void topk_finalize(float* __restrict__ topv, int3
   }
 }
 
+// 1 / x for a normal power of two x, exact, without a division: the exponent field is negated about the bias
+__device__ __forceinline__ float pow2_inv(float x) { return __int_as_float(0x7f000000 - __float_as_int(x)); }
+
 // nextafterf(x, -inf) without its branches: one ulp down for finite x and +inf, -0 / +0 -> -denorm_min, -inf and nan stay
 __device__ __forceinline__ float next_down(float x) {
   const int b = __float_as_int(x);
@@ -76,13 +81,14 @@ __device__ __forceinline__ float next_down(float x) {
 
 // (a): per target, count the scores of this chunk that outrank it
 template <int NC, int TMAX>
-__device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t base, int T, RankState<TMAX>& rs, float f = 1.f) {
+__device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t base, int T, RankState<TMAX>& rs, float f = 1.f,
+                                                 float f2 = 1.f) {
 #pragma unroll
   for (int t = 0; t < TMAX; ++t) {
     if (t < T) {
       const int tg = rs.tg[t];
       if (base + NC <= tg || base > tg) {          // warp-uniform: targets are the same for every user
-        const float st = rs.st[t] * f;             // nextafter(st, -inf) is derived here, not carried in a register
+        const float st = rs.st[t] * f * f2;        // nextafter(st, -inf) is derived here, not carried in a register
         const float thr = base > tg ? st : next_down(st);
         int c0 = 0, c1 = 0, c2 = 0, c3 = 0;          // four independent chains: one warp per scheduler has
 #pragma unroll                                     // nothing else to hide the add latency behind
@@ -94,7 +100,7 @@ __device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t b
         }
         rs.rk[t] += (c0 + c1) + (c2 + c3);
       } else {                                     // the one chunk that holds the target itself
-        const float st = rs.st[t] * f;
+        const float st = rs.st[t] * f * f2;
 #pragma unroll
         for (int e = 0; e < NC; ++e) {
           const int item = (int)base + e;
@@ -109,9 +115,9 @@ __device__ __forceinline__ void rank_count_chunk(const float (&s)[NC], int64_t b
 template <int NC, int TMAX>
 __device__ __forceinline__ void rank_topk_chunk(float (&s)[NC], int64_t base, int T, RankState<TMAX>& rs, float& tau,
                                                 float* __restrict__ topv, int32_t* __restrict__ topi, int K, int stride,
-                                                int slot, int& min_pos, float f = 1.f, float inv = 1.f) {
+                                                int slot, int& min_pos, float f = 1.f, float inv = 1.f, float f2 = 1.f) {
   static_assert(NC % 8 == 0, "chunks are scanned in groups of 8");
-  rank_count_chunk<NC, TMAX>(s, base, T, rs, f);
+  rank_count_chunk<NC, TMAX>(s, base, T, rs, f, f2);
   // group maxima (8 consecutive items each): only a group that beats tau is looked at element by element
   float gm[NC / 8];
 #pragma unroll
@@ -123,7 +129,7 @@ __device__ __forceinline__ void rank_topk_chunk(float (&s)[NC], int64_t base, in
   float cmax = gm[0];
 #pragma unroll
   for (int q = 1; q < NC / 8; ++q) cmax = fmaxf(cmax, gm[q]);
-  float ts = tau * f;                                // tau in the scores' domain
+  float ts = tau * f * f2;                           // tau in the scores' domain
   if (cmax > ts) {
 #pragma unroll
     for (int q = 0; q < NC / 8; ++q) {
@@ -131,8 +137,8 @@ __device__ __forceinline__ void rank_topk_chunk(float (&s)[NC], int64_t base, in
 #pragma unroll
         for (int e = 8 * q; e < 8 * q + 8; ++e)
           if (s[e] > ts) {
-            tau = topk_replace(s[e] * inv, (int32_t)(base + e), topv, topi, K, stride, slot, min_pos);
-            ts = tau * f;
+            tau = topk_replace(s[e] * inv * pow2_inv(f2), (int32_t)(base + e), topv, topi, K, stride, slot, min_pos);
+            ts = tau * f * f2;
           }
       }
     }
