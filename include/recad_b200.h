@@ -484,6 +484,29 @@ int recad_bpr_hvp_seeds(const float* O, const float* dO, int64_t n_users, int64_
                         int64_t B_norm, int32_t D, const float* E, const float* V, float lambda, float* alpha, float* beta,
                         float* dloss, int32_t* bad, void* stream);
 
+/* Mixed second derivative of the BPR training loss L = (1/n) sum_b l_b (the loss recad_bpr_hvp_seeds differentiates, over
+ * the n rows samples [dev] int64[n, 3]) with respect to the values v of st->graph, along S [dev] float[N, D] (users first):
+ *   gvals [dev] float[nnz] (st->graph's entry order) = d/dv <S, grad_E L>, at the state's tables st->E.
+ * With O = P E, dO = P S (P = (1 / (L + 1)) sum_l A^l), a_b / c_b the seeds of recad_bpr_hvp_seeds (B_norm = n), G_O the
+ * H_O dO of recad_pair_scores_hvp and G_dO = the pair backward of c over O, gvals is the edge-value gradient of
+ * <G_O, O> + <G_dO, dO> with G held: (1 / (L + 1)) sum_{j < L} <t_j[r_k], Y_{L-1-j}[c_k]> over the 2D columns of the
+ * interleaved rows t_j (Horner iterates of [G_O | G_dO]) and Y_l = A^l [E | S].  The regulariser does not depend on v;
+ * L = 0: gvals = 0.  One recurrence at width 2D: A2 is st->graph's struct for width 2D (its own partial-sum scratch);
+ * st->graph_t must be NULL (symmetric values).  The state's buffers are not written.  work [dev] of
+ * recad_lightgcn_loss_mixed_values_work_bytes(N, D, n_layers, n) bytes (L + 2 buffers of N * 2D floats, one more
+ * for L >= 3, plus O(n)).  Atomic-free and bit-stable at any n; synchronises the stream once: an id outside its
+ * table gives RECAD_ERR_ARG. */
+int64_t recad_lightgcn_loss_mixed_values_work_bytes(int64_t n_rows, int32_t D, int32_t n_layers, int64_t n);
+int recad_lightgcn_loss_mixed_values(const recad_lightgcn* st, const recad_csr* A2, const float* S, const int64_t* samples,
+                                     int64_t n, float* gvals, void* work, int64_t work_bytes, void* stream);
+
+/* out [dev] float[n_out] = per index r, the sum of x[b] over the b with idx[b] = r, in ascending b, in double (0 where
+ * none); idx [dev] int64[n] with entries < 0 skipped.  One stable radix sort and one writer per output: atomic-free and
+ * bit-stable.  scratch [dev] of recad_pair_scores_backward_scratch_bytes(n) bytes.  Synchronises the stream: an index
+ * >= n_out gives RECAD_ERR_ARG. */
+int recad_index_sums(const int64_t* idx, const float* x, int64_t n, int64_t n_out, float* out, void* scratch,
+                     int64_t scratch_bytes, void* stream);
+
 /* ------------------------------------------------------------------------ *
  * MF pointwise BCE step  (recad/model/victim/mf.py:40-69)
  * ------------------------------------------------------------------------ */

@@ -4,6 +4,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <vector>
 
 #include "common.cuh"
 
@@ -369,12 +370,15 @@ pair_keys_kernel(const int64_t* __restrict__ ids, int64_t n_rows, int64_t B, int
 // one warp per sorted key; the warp of a row's first key writes dX[row] = sum g_b X[other_b] (+ beta_b V[other_b] when kTwo)
 // and db[row] = sum g_b; every other warp returns.  kTwo sums in double: a Hessian product's popular rows collect 10^5 and
 // more pairs, and a float running sum of that length loses ~sqrt(count) ulps (1e-5 of the row at 10^5 pairs).
-template <bool kTwo>
+// kJoint (with kTwo): X holds interleaved rows [O | dO] of 2 nvec float4s, gathered once per pair, and the row written is
+// [sum g_b O + beta_b dO | sum beta_b O] of the same width, both halves summed in double; V and db are not used.
+template <bool kTwo, bool kJoint = false>
 __global__ void __launch_bounds__(256)
 pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, const float* __restrict__ g,
                       const float* __restrict__ beta, const int64_t* __restrict__ other, int64_t n_other,
                       const float* __restrict__ X, const float* __restrict__ V, int nvec, float* __restrict__ dX,
                       float* __restrict__ db) {
+  static_assert(kTwo || !kJoint, "the joint rows need beta");
   const int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (k >= B) return;
@@ -389,6 +393,7 @@ pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, c
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     float gsum = 0.f;
     double dx = 0.0, dy = 0.0, dz = 0.0, dw = 0.0, dg = 0.0;       // kTwo accumulators
+    double ex = 0.0, ey = 0.0, ez = 0.0, ew = 0.0;                 // kJoint: the second half
     for (int64_t j = k; j < B; ++j) {
       const uint64_t key = keys[j];
       if ((key >> bbits) != row) break;
@@ -396,7 +401,20 @@ pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, c
       int64_t o = other[b];
       if (o < 0 || o >= n_other) o = 0;            // reported by the other side's key pass
       const float gv = g[b];
-      if constexpr (kTwo) {
+      if constexpr (kJoint) {
+        if (c < nvec) {
+          const double bv = (double)beta[b];
+          const float4 x = __ldg(X4 + o * 2 * nvec + c), y = __ldg(X4 + o * 2 * nvec + nvec + c);
+          dx = fma((double)gv, (double)x.x, fma(bv, (double)y.x, dx));
+          dy = fma((double)gv, (double)x.y, fma(bv, (double)y.y, dy));
+          dz = fma((double)gv, (double)x.z, fma(bv, (double)y.z, dz));
+          dw = fma((double)gv, (double)x.w, fma(bv, (double)y.w, dw));
+          ex = fma(bv, (double)x.x, ex);
+          ey = fma(bv, (double)x.y, ey);
+          ez = fma(bv, (double)x.z, ez);
+          ew = fma(bv, (double)x.w, ew);
+        }
+      } else if constexpr (kTwo) {
         dg += (double)gv;
         if (c < nvec) {
           const double bv = (double)beta[b];
@@ -418,8 +436,15 @@ pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, c
       acc = make_float4((float)dx, (float)dy, (float)dz, (float)dw);
       gsum = (float)dg;
     }
-    if (c < nvec) dX4[(int64_t)row * nvec + c] = acc;
-    if (c0 == 0 && lane == 0 && db) db[row] = gsum;
+    if constexpr (kJoint) {
+      if (c < nvec) {
+        dX4[(int64_t)row * 2 * nvec + c] = acc;
+        dX4[(int64_t)row * 2 * nvec + nvec + c] = make_float4((float)ex, (float)ey, (float)ez, (float)ew);
+      }
+    } else {
+      if (c < nvec) dX4[(int64_t)row * nvec + c] = acc;
+      if (c0 == 0 && lane == 0 && db) db[row] = gsum;
+    }
   }
 }
 
@@ -427,7 +452,8 @@ pair_grad_rows_kernel(const uint64_t* __restrict__ keys, int64_t B, int bbits, c
 // Seeds of the BPR loss's Hessian-vector product.  Per sample b, x = <O_u, O_n> - <O_u, O_p>, dx its derivative along
 // dO = P v, l' / l'' softplus's first two derivatives (torch's threshold 20, as bpr_kernel); the (u, n) pair gets
 // (a, c) = (l'' dx / B, l' / B) and the (u, p) pair (-a, -c).  dloss[b] = l' dx + lambda (<V_u, E_u> + <V_p, E_p> + <V_n, E_n>).
-// kSeedLanes lanes per sample, 128-bit loads, a fixed shuffle order: no atomics on the results.
+// kSeedLanes lanes per sample, 128-bit loads, a fixed shuffle order: no atomics on the results.  Rows of O / dO (and E / V)
+// are rstride float4s apart: nvec for tables of their own, 2 nvec for the interleaved [O | dO] rows (dO = O + D).
 // ------------------------------------------------------------------------------------------
 constexpr int kSeedLanes = 16;
 
@@ -435,9 +461,9 @@ __device__ __forceinline__ float dot4(const float4 a, const float4 b) { return a
 
 __global__ void __launch_bounds__(256)
 bpr_hvp_seeds_kernel(const float* __restrict__ O, const float* __restrict__ dO, int64_t n_users, int64_t n_items,
-                     const int64_t* __restrict__ samples, int64_t n, float inv_B, int nvec, const float* __restrict__ E,
-                     const float* __restrict__ V, float lambda, float* __restrict__ alpha, float* __restrict__ beta,
-                     float* __restrict__ dloss, int* __restrict__ bad) {
+                     const int64_t* __restrict__ samples, int64_t n, float inv_B, int nvec, int rstride,
+                     const float* __restrict__ E, const float* __restrict__ V, float lambda, float* __restrict__ alpha,
+                     float* __restrict__ beta, float* __restrict__ dloss, int* __restrict__ bad) {
   const int l = threadIdx.x % kSeedLanes;
   const int64_t group = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / kSeedLanes;
   const int64_t n_groups = (int64_t)gridDim.x * blockDim.x / kSeedLanes;
@@ -457,7 +483,7 @@ bpr_hvp_seeds_kernel(const float* __restrict__ O, const float* __restrict__ dO, 
         u = 0; p = 0; q = 0;
       }
     }
-    const int64_t ru = u * nvec, rp = (n_users + p) * nvec, rn = (n_users + q) * nvec;
+    const int64_t ru = u * rstride, rp = (n_users + p) * rstride, rn = (n_users + q) * rstride;
     float dn = 0.f, dp = 0.f, dx = 0.f, reg = 0.f;
     if (valid) {
       for (int c = l; c < nvec; c += kSeedLanes) {
@@ -498,6 +524,112 @@ static int bit_width(int64_t n) {     // bits needed for the values 0 .. n - 1 (
   int b = 1;
   while (b < 63 && ((int64_t)1 << b) < n) ++b;
   return b;
+}
+
+enum class PairMode { kBackward, kHvp, kJoint };
+
+// Both sides of the pair pass, one radix sort per side (ids checked into `bad`; the rows no pair reaches are left as they
+// are, so the caller zeroes the outputs).  kJoint: Xa / Xb are the interleaved [O | dO] rows of 2D floats of each side and
+// outA / outB receive rows of the same width (pair_grad_rows_kernel<true, true>); Va, Vb, dba, dbb are not used.
+static int pair_sides(PairMode mode, const float* Xa, const float* Va, int64_t n_a, const float* Xb, const float* Vb,
+                      int64_t n_b, int32_t D, const int64_t* ia, const int64_t* ib, int64_t B, const float* alpha,
+                      const float* beta, float* outA, float* outB, float* dba, float* dbb, uint64_t* keys, uint64_t* tmp,
+                      void* sort_scr, int* bad, cudaStream_t s) {
+  const int bbits = bit_width(B);
+  const unsigned kgrid = (unsigned)std::min<int64_t>((B + 255) / 256, (int64_t)sm_count() * 16);
+  const unsigned wgrid = (unsigned)((B * 32 + 255) / 256);
+  for (int side = 0; side < 2; ++side) {
+    const int64_t n_rows = side == 0 ? n_a : n_b, n_other = side == 0 ? n_b : n_a;
+    const int64_t* ids = side == 0 ? ia : ib;
+    pair_keys_kernel<<<kgrid, 256, 0, s>>>(ids, n_rows, B, bbits, keys, bad);
+    RECAD_LAUNCH_CHECK();
+    int rc = radix_sort_u64(keys, tmp, B, bbits + bit_width(n_rows), sort_scr, s);
+    if (rc) return rc;
+    const int64_t* other = side == 0 ? ib : ia;
+    const float* X = side == 0 ? Xb : Xa;
+    float* out = side == 0 ? outA : outB;
+    float* db = side == 0 ? dba : dbb;
+    if (mode == PairMode::kJoint)
+      pair_grad_rows_kernel<true, true><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, beta, other, n_other, X, nullptr, D / 4,
+                                                               out, nullptr);
+    else if (mode == PairMode::kHvp)
+      pair_grad_rows_kernel<true><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, beta, other, n_other, X, side == 0 ? Vb : Va,
+                                                         D / 4, out, db);
+    else
+      pair_grad_rows_kernel<false><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, nullptr, other, n_other, X, nullptr, D / 4,
+                                                          out, db);
+    RECAD_LAUNCH_CHECK();
+  }
+  return RECAD_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Per-index sums, atomic-free: key_b = idx_b << bbits | b (idx_b < 0 -> the sentinel n_out, sorted last and not written),
+// stably radix-sorted; the thread of a group's first key sums x over the group in ascending b, in double, and is the
+// output's only writer.
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+index_keys_kernel(const int64_t* __restrict__ idx, int64_t n, int64_t n_out, int bbits, uint64_t* __restrict__ keys,
+                  int* __restrict__ bad) {
+  for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < n; b += (int64_t)gridDim.x * blockDim.x) {
+    int64_t id = idx[b];
+    if (id >= n_out) { atomicOr(bad, 1); id = n_out; }
+    if (id < 0) id = n_out;
+    keys[b] = ((uint64_t)id << bbits) | (uint64_t)b;
+  }
+}
+
+__global__ void __launch_bounds__(256)
+index_sums_kernel(const uint64_t* __restrict__ keys, int64_t n, int bbits, uint64_t n_out, const float* __restrict__ x,
+                  float* __restrict__ out) {
+  const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const uint64_t row = keys[k] >> bbits;
+  if (row >= n_out || (k > 0 && (keys[k - 1] >> bbits) == row)) return;
+  const uint64_t bmask = (1ull << bbits) - 1;
+  double acc = 0.0;
+  for (int64_t j = k; j < n && (keys[j] >> bbits) == row; ++j) acc += (double)x[keys[j] & bmask];
+  out[row] = (float)acc;
+}
+
+// Workspace of recad_lightgcn_loss_mixed_values: [N, 2D] float buffers -- the forward layers Y_0 .. Y_{L-1} of [E | S]
+// (Y_0 only for L = 0), [O | dO] (L >= 1; it is the Horner's first ping-pong buffer once the pair pass has read it), the
+// pair pass's output G, the second ping-pong buffer (L >= 3) -- then the pairs' ids, seeds, sort keys and the id flag.
+struct MixedWork {
+  float* Y;   // Y_l = Y + l * N * 2D
+  float* OO;
+  float* G;
+  float* X1;
+  int64_t *ia, *ib;
+  float *alpha, *beta;
+  uint64_t *keys, *tmp;
+  void* sort_scr;
+  int* bad;
+};
+
+static int64_t mixed_work(int64_t N, int32_t D, int32_t L, int64_t n, char* base, MixedWork* w) {
+  const int64_t rowbuf = N * 2 * (int64_t)D * (int64_t)sizeof(float), B = 2 * n;   // a multiple of 32 bytes
+  const int64_t n_y = L > 0 ? L : 1;
+  int64_t off = 0;
+  auto take = [&](int64_t bytes) { char* p = base ? base + off : nullptr; off += align256(bytes); return p; };
+  char* Y = take(n_y * rowbuf);
+  char* OO = L > 0 ? take(rowbuf) : Y;
+  char* G = take(rowbuf);
+  char* X1 = L >= 3 ? take(rowbuf) : nullptr;
+  char* ia = take(B * 8);
+  char* ib = take(B * 8);
+  char* alpha = take(B * 4);
+  char* beta = take(B * 4);
+  char* keys = take(B * 8);
+  char* tmp = take(B * 8);
+  char* sort_scr = take(sort_scratch_bytes(B));
+  char* bad = take(sizeof(int));
+  if (w)
+    *w = MixedWork{reinterpret_cast<float*>(Y), reinterpret_cast<float*>(OO), reinterpret_cast<float*>(G),
+                   reinterpret_cast<float*>(X1), reinterpret_cast<int64_t*>(ia), reinterpret_cast<int64_t*>(ib),
+                   reinterpret_cast<float*>(alpha), reinterpret_cast<float*>(beta), reinterpret_cast<uint64_t*>(keys),
+                   reinterpret_cast<uint64_t*>(tmp), sort_scr, reinterpret_cast<int*>(bad)};
+  return off;
 }
 
 // Edge-value gradient riding on the Horner loop: at step k, before t_k's ping-pong buffer is written again,
@@ -732,28 +864,9 @@ int recad_pair_scores_hvp(const float* Xa, const float* Va, int64_t n_a, const f
   void* sort_scr = p;                                 p += align256(sort_scratch_bytes(B));
   int* bad = reinterpret_cast<int*>(p);
   RECAD_CUDA_CHECK(cudaMemsetAsync(bad, 0, sizeof(int), s));
-  const int bbits = bit_width(B);
-  const unsigned kgrid = (unsigned)std::min<int64_t>((B + 255) / 256, (int64_t)sm_count() * 16);
-  const unsigned wgrid = (unsigned)((B * 32 + 255) / 256);
-  for (int side = 0; side < 2; ++side) {
-    const int64_t n_rows = side == 0 ? n_a : n_b, n_other = side == 0 ? n_b : n_a;
-    const int64_t* ids = side == 0 ? ia : ib;
-    pair_keys_kernel<<<kgrid, 256, 0, s>>>(ids, n_rows, B, bbits, keys, bad);
-    RECAD_LAUNCH_CHECK();
-    int rc = radix_sort_u64(keys, tmp, B, bbits + bit_width(n_rows), sort_scr, s);
-    if (rc) return rc;
-    const int64_t* other = side == 0 ? ib : ia;
-    const float* X = side == 0 ? Xb : Xa;
-    float* out = side == 0 ? outA : outB;
-    float* db = side == 0 ? dba : dbb;
-    if (beta)
-      pair_grad_rows_kernel<true><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, beta, other, n_other, X, side == 0 ? Vb : Va,
-                                                         D / 4, out, db);
-    else
-      pair_grad_rows_kernel<false><<<wgrid, 256, 0, s>>>(keys, B, bbits, alpha, nullptr, other, n_other, X, nullptr, D / 4,
-                                                          out, db);
-    RECAD_LAUNCH_CHECK();
-  }
+  const int rc = pair_sides(beta ? PairMode::kHvp : PairMode::kBackward, Xa, Va, n_a, Xb, Vb, n_b, D, ia, ib, B, alpha, beta,
+                            outA, outB, dba, dbb, keys, tmp, sort_scr, bad, s);
+  if (rc) return rc;
   int h_bad = 0;
   RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, s));
   RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
@@ -772,8 +885,8 @@ int recad_bpr_hvp_seeds(const float* O, const float* dO, int64_t n_users, int64_
   RECAD_CUDA_CHECK(cudaMemsetAsync(bad, 0, sizeof(int32_t), s));
   const int64_t want = (n * kSeedLanes + 255) / 256;
   const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sm_count() * 32));
-  bpr_hvp_seeds_kernel<<<grid, 256, 0, s>>>(O, dO, n_users, n_items, samples, n, 1.0f / (float)B_norm, D / 4, E, V, lambda,
-                                            alpha, beta, dloss, bad);
+  bpr_hvp_seeds_kernel<<<grid, 256, 0, s>>>(O, dO, n_users, n_items, samples, n, 1.0f / (float)B_norm, D / 4, D / 4, E, V,
+                                            lambda, alpha, beta, dloss, bad);
   RECAD_LAUNCH_CHECK();
   int32_t h_bad = 0;
   RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
@@ -822,6 +935,109 @@ int recad_lightgcn_backward_values(const recad_lightgcn* st, const float* gO, co
   const HornerValues hv{X, gvals, 1.0f / (float)(L + 1)};
   const float* t = nullptr;
   return lightgcn_horner(st, gO, 1.0f / (float)(L + 1), gE, &t, stream, &hv);
+}
+
+int64_t recad_lightgcn_loss_mixed_values_work_bytes(int64_t n_rows, int32_t D, int32_t n_layers, int64_t n) {
+  if (n_rows <= 0 || D < 4 || n_layers < 0 || n <= 0) return -1;
+  return mixed_work(n_rows, D, n_layers, n, nullptr, nullptr);
+}
+
+int recad_lightgcn_loss_mixed_values(const recad_lightgcn* st, const recad_csr* A2, const float* S, const int64_t* samples,
+                                     int64_t n, float* gvals, void* work, int64_t work_bytes, void* stream) {
+  int rc = check_lightgcn(st);
+  if (rc) return rc;
+  RECAD_REQUIRE(A2 && S && samples && gvals && work && n > 0, RECAD_ERR_ARG, "lightgcn_loss_mixed_values: bad argument");
+  const recad_csr* A = st->graph;
+  RECAD_REQUIRE(!st->graph_t && A->n_cols == A->n_rows && A2->n_rows == A->n_rows && A2->n_cols == A->n_cols &&
+                    A2->nnz == A->nnz,
+                RECAD_ERR_ARG, "lightgcn_loss_mixed_values: A2 must be the state's own (symmetric) graph at width 2D");
+  const int32_t D = st->D, D2 = 2 * st->D;
+  const int L = st->n_layers;
+  RECAD_REQUIRE(D2 <= 1024, RECAD_ERR_UNSUPPORTED, "lightgcn_loss_mixed_values: D = %d above 512", D);
+  RECAD_REQUIRE(n < ((int64_t)1 << 31) - 1, RECAD_ERR_OVERFLOW, "lightgcn_loss_mixed_values: n below 2^31 - 1");
+  const int64_t U = st->n_users, N = st->n_users + st->n_items;
+  RECAD_REQUIRE(work_bytes >= mixed_work(N, D, L, n, nullptr, nullptr), RECAD_ERR_SCRATCH,
+                "lightgcn_loss_mixed_values: work too small");
+  MixedWork w;
+  mixed_work(N, D, L, n, static_cast<char*>(work), &w);
+  cudaStream_t s = as_stream(stream);
+  const size_t row2 = (size_t)D2 * sizeof(float), row1 = (size_t)D * sizeof(float);
+  const int64_t stride = N * D2;
+  // Y_0 = [E | S]; Y_{l+1} = A Y_l and [O | dO] = (1 / (L + 1)) sum_l Y_l: recad_lightgcn_propagate's calls at width 2D
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.Y, row2, st->E, row1, row1, N, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.Y + D, row2, S, row1, row1, N, cudaMemcpyDeviceToDevice, s));
+  for (int k = 0; k < L; ++k) {
+    const bool last = k == L - 1;
+    rc = recad_spmm(A2, w.Y + k * stride, last ? nullptr : w.Y + (k + 1) * stride, k == 0 ? w.Y : w.OO, w.OO,
+                    last ? 1.0f / (float)(L + 1) : 1.0f, D2, stream);
+    if (rc) return rc;
+  }
+  // seeds (a_b, c_b) from the interleaved rows, then G = [G_O | G_dO] by the pairs (u, neg), (u, pos)
+  RECAD_CUDA_CHECK(cudaMemsetAsync(w.bad, 0, sizeof(int), s));
+  const int64_t want = (n * kSeedLanes + 255) / 256;
+  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sm_count() * 32));
+  bpr_hvp_seeds_kernel<<<grid, 256, 0, s>>>(w.OO, w.OO + D, U, st->n_items, samples, n, 1.0f / (float)n, D / 4, D2 / 4,
+                                            nullptr, nullptr, 0.0f, w.alpha, w.beta, nullptr, w.bad);
+  RECAD_LAUNCH_CHECK();
+  const size_t row3 = 3 * sizeof(int64_t);
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ia, sizeof(int64_t), samples, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ia + n, sizeof(int64_t), samples, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ib, sizeof(int64_t), samples + 2, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ib + n, sizeof(int64_t), samples + 1, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice,
+                                     s));
+  RECAD_CUDA_CHECK(cudaMemsetAsync(w.G, 0, (size_t)stride * sizeof(float), s));
+  rc = pair_sides(PairMode::kJoint, w.OO, nullptr, U, w.OO + U * D2, nullptr, st->n_items, D, w.ia, w.ib, 2 * n, w.alpha,
+                  w.beta, w.G, w.G + U * D2, nullptr, nullptr, w.keys, w.tmp, w.sort_scr, w.bad, s);
+  if (rc) return rc;
+  int h_bad = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, w.bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "lightgcn_loss_mixed_values: an id is out of range");
+  if (L == 0) {
+    if (A->nnz) RECAD_CUDA_CHECK(cudaMemsetAsync(gvals, 0, A->nnz * sizeof(float), s));
+    return RECAD_OK;
+  }
+  // g_v = (1 / (L + 1)) sum_j <t_j[r], Y_{L-1-j}[c]> over the 2D columns, t_j the Horner iterates of G over A
+  recad_lightgcn joint = *st;
+  joint.graph = A2;
+  joint.graph_t = nullptr;
+  joint.D = D2;
+  joint.X0 = w.OO;
+  joint.X1 = w.X1;
+  std::vector<const float*> layers(L);
+  for (int l = 0; l < L; ++l) layers[l] = w.Y + l * stride;
+  const HornerValues hv{layers.data(), gvals, 1.0f / (float)(L + 1)};
+  const float* t = nullptr;
+  return lightgcn_horner(&joint, w.G, 1.0f / (float)(L + 1), nullptr, &t, stream, &hv);
+}
+
+int recad_index_sums(const int64_t* idx, const float* x, int64_t n, int64_t n_out, float* out, void* scratch,
+                     int64_t scratch_bytes, void* stream) {
+  RECAD_REQUIRE(idx && x && out && scratch && n > 0 && n_out > 0, RECAD_ERR_ARG, "index_sums: bad argument");
+  RECAD_REQUIRE(n < ((int64_t)1 << 32) - 1 && n_out < ((int64_t)1 << 31), RECAD_ERR_OVERFLOW,
+                "index_sums: n below 2^32 - 1 and n_out below 2^31");
+  RECAD_REQUIRE(scratch_bytes >= recad_pair_scores_backward_scratch_bytes(n), RECAD_ERR_SCRATCH, "index_sums: scratch too small");
+  cudaStream_t s = as_stream(stream);
+  char* p = static_cast<char*>(scratch);
+  uint64_t* keys = reinterpret_cast<uint64_t*>(p);    p += align256(n * 8);
+  uint64_t* tmp = reinterpret_cast<uint64_t*>(p);     p += align256(n * 8);
+  void* sort_scr = p;                                 p += align256(sort_scratch_bytes(n));
+  int* bad = reinterpret_cast<int*>(p);
+  RECAD_CUDA_CHECK(cudaMemsetAsync(bad, 0, sizeof(int), s));
+  RECAD_CUDA_CHECK(cudaMemsetAsync(out, 0, n_out * sizeof(float), s));
+  const int bbits = bit_width(n);
+  const unsigned grid = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 16);
+  index_keys_kernel<<<grid, 256, 0, s>>>(idx, n, n_out, bbits, keys, bad);
+  RECAD_LAUNCH_CHECK();
+  const int rc = radix_sort_u64(keys, tmp, n, bbits + bit_width(n_out + 1), sort_scr, s);
+  if (rc) return rc;
+  index_sums_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(keys, n, bbits, (uint64_t)n_out, x, out);
+  RECAD_LAUNCH_CHECK();
+  int h_bad = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "index_sums: an index is out of range");
+  return RECAD_OK;
 }
 
 }  // extern "C"

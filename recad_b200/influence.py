@@ -1,15 +1,20 @@
 """Influence of training rows on an objective, from the victims' Hessian-vector products (loss_hvp) and per-row
 directional derivatives (sample_directional_derivatives) -- the estimate -grad(obj)^T H^-1 grad(l_z) of influence-function
 attacks and defenses (Fang et al., WWW 2020).  H is the Hessian of the training loss of the given rows taken as one batch,
-at the victim's current tables.  Works with any victim that has those two methods (LightGCN, MF, NCF)."""
+at the victim's current tables.  Works with any victim that has those two methods (LightGCN, MF, NCF).
+
+interaction_hypergradient: for LightGCN, whose training loss depends on the interactions both as training rows and as
+graph edges, the derivative of an objective of the retrained tables with respect to every interaction weight."""
 import math
 from collections import namedtuple
 
 import torch
 
+from . import ops
 from ._lib import RecadError
 
 Influence = namedtuple("Influence", ["values", "s", "iterations", "residual"])
+Hypergradient = namedtuple("Hypergradient", ["values", "direct", "implicit", "s", "iterations", "residual"])
 
 
 def conjugate_gradient(hvp, rhs, damping, max_iter=100, rtol=1e-6):
@@ -59,6 +64,13 @@ def sample_influence(victim, batch, objective_grads, damping, max_iter=100, rtol
     Sign convention: with the loss L = (1/n) sum_b l_b, removing row b changes the trained tables by about
     +(1/n) H^-1 grad(l_b), so the predicted change of the objective when row b is removed is (1/n) values[b]
     (positive: removing the row raises the objective); up-weighting row b by eps changes it by -eps values[b]."""
+    s_t, iters, res = _solve(victim, batch, objective_grads, damping, max_iter, rtol)
+    return Influence(victim.sample_directional_derivatives(batch, s_t), s_t, iters, res)
+
+
+def _solve(victim, batch, objective_grads, damping, max_iter, rtol):
+    """s = (H + damping I)^-1 grad(obj) by conjugate_gradient in float64 over victim.loss_hvp: (s as float32 tensors shaped
+    like objective_grads, iterations, relative residual)."""
     grads = [g.detach() for g in objective_grads]
     shapes = [g.shape for g in grads]
     sizes = [g.numel() for g in grads]
@@ -71,5 +83,54 @@ def sample_influence(victim, batch, objective_grads, damping, max_iter=100, rtol
 
     rhs = torch.cat([g.reshape(-1) for g in grads]).double()
     s, iters, res = conjugate_gradient(hvp, rhs, damping, max_iter, rtol)
-    s_t = unflat(s)
-    return Influence(victim.sample_directional_derivatives(batch, s_t), s_t, iters, res)
+    return unflat(s), iters, res
+
+
+def interaction_hypergradient(victim, batch, objective, damping, max_iter=100, rtol=1e-6):
+    """dJ/dw for every interaction weight w_k (one per stored entry of victim.Graph, CSR order, at the base point
+    w = Graph.mult) of an objective J of the LightGCN tables trained on the BPR loss of `batch` (the rows as for
+    loss_hvp, weighted by w_k(b) / mult_k(b) where k(b) is the entry (u_b, U + pos_b) when it is stored):
+
+        dJ/dw = dJ/dw|_E - M^T s,   s = (H + damping I)^-1 grad_E J,   M^T s = d/dw [s^T grad_E L(E; w)]
+
+    at the victim's current tables, taken as trained (grad_E L ~ 0).  objective(edge_values) returns a scalar tensor built
+    from victim(users, items, edge_values=edge_values); it is evaluated at ops.normalized_values(Graph, w) with w and
+    the tables requiring a gradient (their requires_grad flags are restored afterwards).  s is solved by
+    conjugate_gradient in float64 over loss_hvp.  M^T s = N'(w)^T loss_mixed_values(batch, s) (the graph part) + the
+    sample part, (1 / (n mult_k)) sum over the rows with k(b) = k of s^T grad l_b (rows whose positive pair is not stored
+    have none).  Returns Hypergradient(values = direct - implicit, direct, implicit, s, iterations, residual), the first
+    three float32 [nnz].  When both entries of an interaction carry one weight, its sensitivity is values[k] +
+    values[T[k]] (k = Graph.entry_index(u, U + i), T = Graph.transpose_permutation()).  LightGCN only (DESIGN.md,
+    "Second order"); deterministic; the tables are not changed."""
+    from .victim.lightgcn import LightGCN
+    if not isinstance(victim, LightGCN):
+        raise RecadError(f"interaction_hypergradient: LightGCN victims only (got {type(victim).__name__})")
+    victim._require_instance("interaction_hypergradient")
+    g, U = victim.Graph, victim.num_users
+    params = list(victim.parameters())
+    flags = [p.requires_grad for p in params]
+    w = g.mult.detach().clone().requires_grad_(True)
+    try:
+        for p in params:
+            p.requires_grad_(True)
+        with torch.enable_grad():
+            J = objective(ops.normalized_values(g, w))
+            if not isinstance(J, torch.Tensor) or J.numel() != 1:
+                raise RecadError("interaction_hypergradient: the objective must return a scalar tensor")
+            gw, *gE = torch.autograd.grad(J.reshape(()), [w] + params, allow_unused=True)
+    finally:
+        for p, f in zip(params, flags):
+            p.requires_grad_(f)
+    direct = torch.zeros_like(w) if gw is None else gw.detach()
+    gE = [torch.zeros_like(p) if x is None else x for p, x in zip(params, gE)]
+    s, iters, res = _solve(victim, batch, gE, damping, max_iter, rtol)
+
+    gv = victim.loss_mixed_values(batch, s)
+    w = g.mult.detach().clone().requires_grad_(True)
+    with torch.enable_grad():
+        graph_part, = torch.autograd.grad(ops.normalized_values(g, w), w, gv)
+    dl = victim.sample_directional_derivatives(batch, s)
+    k = g.entry_index(batch["users"], U + batch["positive_items"], missing=-1)
+    sample_part = ops.index_sums(k, dl, g.nnz) / (dl.numel() * g.mult)
+    implicit = graph_part + sample_part
+    return Hypergradient(direct - implicit, direct, implicit, s, iters, res)

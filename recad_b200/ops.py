@@ -320,8 +320,9 @@ class Graph:
             self._tperm = T
         return self._tperm
 
-    def entry_index(self, rows, cols):
-        """int64 positions (CSR entry order) of the stored entries (rows[j], cols[j]); RecadError if a pair is not stored.
+    def entry_index(self, rows, cols, missing=None):
+        """int64 positions (CSR entry order) of the stored entries (rows[j], cols[j]); RecadError if a pair is not stored,
+        unless `missing` is given: an int returned at the pairs that are not stored (out-of-range ids still raise).
         With transpose_permutation, entry_index(r, c) and T[entry_index(r, c)] are the two entries of one interaction."""
         with torch.cuda.device(self.device):
             rows = torch.as_tensor(rows, device=self.device).long()
@@ -335,6 +336,9 @@ class Graph:
                 self._ekeys = r * self.n_cols + self.colidx.long()              # ascending: CSR order with sorted columns
             q = rows * self.n_cols + cols
             k = torch.searchsorted(self._ekeys, q.reshape(-1)).clamp_(max=max(self.nnz - 1, 0)).reshape(q.shape)
+            if missing is not None:
+                found = self._ekeys[k] == q if self.nnz else torch.zeros_like(q, dtype=torch.bool)
+                return torch.where(found, k, torch.full_like(k, int(missing)))
             if q.numel() and (self.nnz == 0 or not bool((self._ekeys[k] == q).all())):
                 raise RecadError("entry_index: a (row, column) pair is not a stored entry")
         return k
@@ -516,6 +520,41 @@ def bpr_hvp_seeds(O, dO, n_users, samples, lam=0.0, E=None, V=None, dloss=False)
                                              _ptr(E if dloss else None), _ptr(V if dloss else None), float(lam), _ptr(alpha),
                                              _ptr(beta), _ptr(dl), _ptr(bad), _stream(dev)), "recad_bpr_hvp_seeds")
     return alpha, beta, dl
+
+
+def lightgcn_loss_mixed_values(st, graph, S, samples):
+    """recad_lightgcn_loss_mixed_values: d/dv <S, grad_E L> (float32 [nnz], the graph's entry order) for the BPR loss of the
+    rows samples int64 [n, 3] at a LightGCN state over `graph` (its own values), S float32 [N, D].  Fresh buffers only."""
+    _need_cuda(S, samples)
+    dev = S.device
+    N, D = S.shape
+    n = samples.shape[0]
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        nbytes = int(L.recad_lightgcn_loss_mixed_values_work_bytes(N, D, st.n_layers, n))
+        work = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+        out = torch.empty(graph.nnz, dtype=torch.float32, device=dev)
+        check(L.recad_lightgcn_loss_mixed_values(C.byref(st), C.byref(graph.struct(2 * D)), _ptr(S), _ptr(samples), n, _ptr(out),
+                                                 _ptr(work), nbytes, _stream(dev)), "recad_lightgcn_loss_mixed_values")
+    return out
+
+
+def index_sums(idx, x, n_out):
+    """out[r] = sum of x[b] over the b with idx[b] = r (float32 [n_out]; entries of idx below 0 are skipped), atomic-free and
+    bit-stable (recad_index_sums: one stable sort, one writer per output, summed in double).  An index >= n_out raises."""
+    _need_cuda(idx, x)
+    dev = x.device
+    n = int(x.numel())
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        out = torch.zeros(n_out, dtype=torch.float32, device=dev)
+        if n == 0:
+            return out
+        nbytes = int(L.recad_pair_scores_backward_scratch_bytes(n))
+        scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        check(L.recad_index_sums(_ptr(idx.contiguous().long()), _ptr(x.contiguous().float()), n, int(n_out), _ptr(out),
+                                 _ptr(scratch), nbytes, _stream(dev)), "recad_index_sums")
+    return out
 
 
 def mf_hvp_seeds(st, dUe, dUb, dIe, dIb, samples, dloss=False):

@@ -278,9 +278,8 @@ class LightGCN(BaseVictim):
         return ops.fullrank_eval(O[:U], O[U:], user_ids, train_rowptr, train_col, targets, K) + (0.0,)
 
     # ------------------------------------------------------------------ second order
-    def _loss_directions(self, batch, vectors, what):
-        """Rows, the direction V [N, D], O = P E and dO = P V for the training loss of `batch` (fresh buffers: the model's
-        tables, moments and cached propagation are not touched)."""
+    def _loss_inputs(self, batch, vectors, what):
+        """The rows of `batch` as int64 [n, 3] and the direction V [N, D], checked."""
         self._require_instance(what)
         if self.dropout and self.training:
             raise ops.RecadError(f"LightGCN.{what}: not defined under graph dropout in training mode (call eval() first)")
@@ -288,7 +287,13 @@ class LightGCN(BaseVictim):
         U, I, D = self.num_users, self.num_items, self.latent_dim
         vu, vi = self._check_vectors(vectors, [(U, D), (I, D)], f"LightGCN.{what}")
         with torch.cuda.device(self._dev):
-            V = torch.cat([vu, vi])
+            return samples, torch.cat([vu, vi])
+
+    def _loss_directions(self, batch, vectors, what):
+        """Rows, the direction V [N, D], O = P E and dO = P V for the training loss of `batch` (fresh buffers: the model's
+        tables, moments and cached propagation are not touched)."""
+        samples, V = self._loss_inputs(batch, vectors, what)
+        with torch.cuda.device(self._dev):
             O, _ = ops.lightgcn_propagate_layers(self._st, self.E, keep=False)
             dO, _ = ops.lightgcn_propagate_layers(self._st, V, keep=False)
         return samples, V, O, dO
@@ -319,6 +324,16 @@ class LightGCN(BaseVictim):
         with torch.cuda.device(self._dev):
             _, _, dloss = ops.bpr_hvp_seeds(O, dO, self.num_users, samples, float(self.config["lambda"]), self.E, V, dloss=True)
         return dloss
+
+    def loss_mixed_values(self, batch, vectors):
+        """g_v = d/dv <v_vec, grad_E L>: the mixed second derivative of the BPR training loss of `batch` (as for loss_hvp)
+        with respect to the graph's edge values v, along `vectors` (shaped as for loss_hvp), at the current tables and the
+        graph's own values.  Float32 [Graph.nnz] in CSR entry order; zeros for n_layers = 0 (the regulariser does not
+        depend on v).  Chain it through ops.normalized_values for interaction weights.  Deterministic; the model is not
+        changed.  One recurrence over the interleaved [E | v_vec] rows at width 2D (DESIGN.md, "Second order")."""
+        samples, V = self._loss_inputs(batch, vectors, "loss_mixed_values")
+        with torch.cuda.device(self._dev):
+            return ops.lightgcn_loss_mixed_values(self._st, self.Graph, V, samples)
 
     def input_describe(self):
         return {
