@@ -500,6 +500,29 @@ int64_t recad_lightgcn_loss_mixed_values_work_bytes(int64_t n_rows, int32_t D, i
 int recad_lightgcn_loss_mixed_values(const recad_lightgcn* st, const recad_csr* A2, const float* S, const int64_t* samples,
                                      int64_t n, float* gvals, void* work, int64_t work_bytes, void* stream);
 
+/* Gradient of f(W) = <gO, O> + <S, grad_E L> with respect to one weight W put on both entries (u, U + i), (U + i, u) of
+ * an interaction, for the users sel [dev] int64[n_sel] against every item, stored or not:
+ *   out [dev] float[n_sel, n_items] (row-major) = d_u d_i (g_v(u, U+i) + g_v(U+i, u)) + coef_u + coef_{U+i} + sample part,
+ * at the state's tables and the base point W = mult (0 where not stored).  O = P E as in recad_lightgcn_propagate; L the
+ * loss of recad_lightgcn_loss_mixed_values over the n rows samples [dev] int64[n, 3], each row weighted by w_k / mult_k
+ * when its positive pair k = (u, U + pos) is stored; g_v the SDDMM formula of that entry with the seed G = its mixed seed
+ * + [gO | 0] (valid at unstored pairs as well); coef the per-row term of recad_csr_normalize_backward (pass 1) from g_v at
+ * the stored entries; the sample part (1 / (n mult_k)) sum of the row derivatives along S (the dloss of
+ * recad_bpr_hvp_seeds with lambda) over the rows with positive pair k, at the stored pairs of sel's rows.
+ * gO, S [dev] float[N, D] (users first) or NULL (zero); n = 0: no rows (S and samples may be NULL).  mult [dev] float[nnz],
+ * tperm [dev] int64[nnz] (the transpose permutation) and d_inv [dev] float[N] are st->graph's multiplicities, structure
+ * transpose and normalisation factors (d_r = (s_r + 1e-14)^(-1/2)); A2 is st->graph's struct at width 2D; st->graph_t
+ * must be NULL.  One recurrence at width 2D whose Horner pass also gathers the split GEMM operands, then one 3xTF32
+ * tensor-core GEMM [n_sel, 4 L D + 1] x [n_items, 4 L D + 1]^T with the column bias coef_{U+i}; L = 0: the sample part
+ * only.  work [dev] of recad_lightgcn_candidate_weight_grads_work_bytes bytes.  D <= 512.  Atomic-free and bit-stable;
+ * synchronises the stream once: an id of sel outside [0, n_users) or of samples outside its table gives RECAD_ERR_ARG. */
+int64_t recad_lightgcn_candidate_weight_grads_work_bytes(int64_t n_users, int64_t n_items, int32_t D, int32_t n_layers,
+                                                         int64_t n, int64_t nnz, int64_t n_sel);
+int recad_lightgcn_candidate_weight_grads(const recad_lightgcn* st, const recad_csr* A2, const float* mult,
+                                          const int64_t* tperm, const float* d_inv, const float* gO, const float* S,
+                                          const int64_t* samples, int64_t n, float lambda, const int64_t* sel, int64_t n_sel,
+                                          float* out, void* work, int64_t work_bytes, void* stream);
+
 /* out [dev] float[n_out] = per index r, the sum of x[b] over the b with idx[b] = r, in ascending b, in double (0 where
  * none); idx [dev] int64[n] with entries < 0 skipped.  One stable radix sort and one writer per output: atomic-free and
  * bit-stable.  scratch [dev] of recad_pair_scores_backward_scratch_bytes(n) bytes.  Synchronises the stream: an index

@@ -138,6 +138,9 @@ SIGNATURES = {
     "recad_lightgcn_loss_mixed_values_work_bytes": (i64, [i64, i32, i32, i64]),
     "recad_lightgcn_loss_mixed_values": (C.c_int, [C.POINTER(LightGCN), C.POINTER(CSR), vp, vp, i64, vp, vp, i64, vp]),
     "recad_index_sums": (C.c_int, [vp, vp, i64, i64, vp, vp, i64, vp]),
+    "recad_lightgcn_candidate_weight_grads_work_bytes": (i64, [i64, i64, i32, i32, i64, i64, i64]),
+    "recad_lightgcn_candidate_weight_grads": (C.c_int, [C.POINTER(LightGCN), C.POINTER(CSR), vp, vp, vp, vp, vp, vp, i64, f32,
+                                                        vp, i64, vp, vp, i64, vp]),
     "recad_csr_sddmm": (C.c_int, [C.POINTER(CSR), vp, vp, i32, f32, i32, vp, vp]),
     "recad_csr_row_sums": (C.c_int, [vp, vp, i64, i64, vp, vp]),
     "recad_csr_normalize_backward": (C.c_int, [vp, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp]),

@@ -7,8 +7,14 @@
 #include <vector>
 
 #include "common.cuh"
+#include "tc_common.cuh"
 
 namespace recad {
+
+int gemm_tc(const float* A_hi, const float* A_lo, int M, int lda, const float* B_hi, const float* B_lo, int N, int ldb, int K,
+            float* Cm, int ldc, const float* bias, bool relu, float* out_hi, float* out_lo, int ld_split, cudaStream_t s);
+int csr_normalize_coef(const int64_t* rowptr, const int32_t* colidx, const int64_t* tperm, const float* w, const float* d_inv,
+                       const float* gv, int64_t n_rows, float* coef, cudaStream_t s);
 
 // ------------------------------------------------------------------------------------------
 // BPR forward + backward.  A group of LPR lanes owns one sample; each lane holds VPL float4 columns
@@ -640,20 +646,81 @@ struct HornerValues {
   float scale;
 };
 
+// Operand gather riding on the same loop (recad_lightgcn_candidate_weight_grads): at step k, before t_k's ping-pong buffer is
+// written again, the rows of t_k and X[L - 1 - k] (interleaved rows of width W = st->D) land in columns [2kW, 2(k+1)W) of
+// the split (3xTF32 hi / lo) GEMM operands, which gemm_tc reads row-major with row stride ld:
+//   A row r (r < n_sel, user sel[r]): [t_k | X[L-1-k]][sel[r]] * d_inv[sel[r]] * scale
+//   B row i (i < n_items):            [X[L-1-k] | t_k][n_users + i] * d_inv[n_users + i]
+// so that <A_r, B_i> summed over k is scale * d_u d_i (g(u, U + i) + g(U + i, u)), g the unscaled SDDMM of the two entries
+// of one interaction, stored or not.  Ids of sel outside [0, n_users) read row 0 (the caller reports them).
+struct HornerGather {
+  const float* const* X;   // host array of the L forward layers, as HornerValues::X
+  const int64_t* sel;
+  int64_t n_sel, n_users, n_items;
+  const float* d_inv;      // [n_users + n_items]
+  float scale;
+  int ld;
+  float *a_hi, *a_lo, *b_hi, *b_lo;
+};
+
+// one thread per float4 of one step's 2W-wide column block, the n_sel A rows first, then the n_items B rows
+__global__ void __launch_bounds__(256)
+gather_split_kernel(const float* __restrict__ t, const float* __restrict__ X, int nvec, const int64_t* __restrict__ sel,
+                    int64_t n_sel, int64_t n_users, int64_t n_items, const float* __restrict__ d_inv, float scale, int ld,
+                    int col0, float* __restrict__ a_hi, float* __restrict__ a_lo, float* __restrict__ b_hi,
+                    float* __restrict__ b_lo) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t row = e / (2 * nvec);
+  const int q = (int)(e - row * 2 * nvec);
+  if (row >= n_sel + n_items) return;
+  const bool a_side = row < n_sel;
+  int64_t src;
+  float f;
+  if (a_side) {
+    src = sel[row];
+    if (src < 0 || src >= n_users) src = 0;
+    f = d_inv[src] * scale;
+  } else {
+    src = n_users + (row - n_sel);
+    f = d_inv[src];
+  }
+  // A: t first, then X; B: X first, then t
+  const bool from_t = (q < nvec) == a_side;
+  const float4 x = __ldg(reinterpret_cast<const float4*>(from_t ? t : X) + src * nvec + (q < nvec ? q : q - nvec));
+  const float v[4] = {x.x * f, x.y * f, x.z * f, x.w * f};
+  float h[4], l[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) split_tf32(v[k], h[k], l[k]);
+  const int64_t off = (a_side ? row : row - n_sel) * ld + col0 + 4 * q;
+  *reinterpret_cast<float4*>((a_side ? a_hi : b_hi) + off) = make_float4(h[0], h[1], h[2], h[3]);
+  *reinterpret_cast<float4*>((a_side ? a_lo : b_lo) + off) = make_float4(l[0], l[1], l[2], l[3]);
+}
+
+static int horner_gather(const HornerGather* hg, int k, int L, const float* t, int32_t W, void* stream) {
+  const int nvec = W / 4;
+  const int64_t threads = (hg->n_sel + hg->n_items) * 2 * nvec;
+  gather_split_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, as_stream(stream)>>>(
+      t, hg->X[L - 1 - k], nvec, hg->sel, hg->n_sel, hg->n_users, hg->n_items, hg->d_inv, hg->scale, hg->ld, 2 * k * W,
+      hg->a_hi, hg->a_lo, hg->b_hi, hg->b_lo);
+  RECAD_LAUNCH_CHECK();
+  return RECAD_OK;
+}
+
 // Horner: t <- g + A t, L times, so that t = (I + A + ... + A^L) g, over graph_t when set.  The last step is scaled by
 // alpha and lands in `out`; out == nullptr: it lands in the X0 / X1 ping-pong buffer of its parity.  *res = the result.
 // hv: the SDDMM of each step on its t_k; with out == nullptr as well, the last SpMM (which gvals does not need) is skipped
-// and *res is nullptr.
+// and *res is nullptr.  hg (only with hv): the operand gather of each step on its t_k, after the SDDMM.
 static int lightgcn_horner(const recad_lightgcn* st, const float* g, float alpha, float* out, const float** res,
-                           void* stream, const HornerValues* hv = nullptr) {
+                           void* stream, const HornerValues* hv = nullptr, const HornerGather* hg = nullptr) {
   const recad_csr* A = st->graph_t ? st->graph_t : st->graph;
   const int L = st->n_layers;
   const float* t = g;
   for (int k = 0; k < L; ++k) {
     const bool last = k == L - 1;
     if (hv) {
-      const int rc = recad_csr_sddmm(st->graph, t, hv->X[L - 1 - k], st->D, hv->scale, k > 0, hv->gvals, stream);
+      int rc = recad_csr_sddmm(st->graph, t, hv->X[L - 1 - k], st->D, hv->scale, k > 0, hv->gvals, stream);
       if (rc) return rc;
+      if (hg && (rc = horner_gather(hg, k, L, t, st->D, stream))) return rc;
       if (last && !out) {
         *res = nullptr;
         return RECAD_OK;
@@ -677,6 +744,197 @@ static int check_lightgcn(const recad_lightgcn* st) {
   RECAD_REQUIRE(st->E && st->O && (st->n_layers < 2 || (st->X0 && st->X1)) && (st->n_layers < 1 || st->X0),
                 RECAD_ERR_ARG, "lightgcn: null buffer");
   return RECAD_OK;
+}
+
+// The mixed driver's recurrences up to the Horner pass: Y_0 = [E | S] ([E | 0] when S is null), Y_{l+1} = A Y_l and
+// [O | dO] = (1 / (L + 1)) sum_l Y_l (recad_lightgcn_propagate's calls at width 2D), then, for n > 0 rows, the seeds
+// (a_b, c_b) from the interleaved rows (and each row's own directional derivative along S into dloss, when given, with the
+// regulariser's weight lambda) and
+// G = [G_O | G_dO] by the pairs (u, neg), (u, pos); G = 0 for n = 0.  Zeroes w.bad first; ids are flagged there.
+static int mixed_recurrence(const recad_lightgcn* st, const recad_csr* A2, const float* S, const int64_t* samples, int64_t n,
+                            const MixedWork& w, float* dloss, float lambda, void* stream) {
+  cudaStream_t s = as_stream(stream);
+  const int32_t D = st->D, D2 = 2 * st->D;
+  const int L = st->n_layers;
+  const int64_t U = st->n_users, N = st->n_users + st->n_items;
+  const size_t row2 = (size_t)D2 * sizeof(float), row1 = (size_t)D * sizeof(float);
+  const int64_t stride = N * D2;
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.Y, row2, st->E, row1, row1, N, cudaMemcpyDeviceToDevice, s));
+  if (S) RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.Y + D, row2, S, row1, row1, N, cudaMemcpyDeviceToDevice, s));
+  else RECAD_CUDA_CHECK(cudaMemset2DAsync(w.Y + D, row2, 0, row1, N, s));
+  for (int k = 0; k < L; ++k) {
+    const bool last = k == L - 1;
+    const int rc = recad_spmm(A2, w.Y + k * stride, last ? nullptr : w.Y + (k + 1) * stride, k == 0 ? w.Y : w.OO, w.OO,
+                              last ? 1.0f / (float)(L + 1) : 1.0f, D2, stream);
+    if (rc) return rc;
+  }
+  RECAD_CUDA_CHECK(cudaMemsetAsync(w.bad, 0, sizeof(int), s));
+  if (n == 0) {
+    RECAD_CUDA_CHECK(cudaMemsetAsync(w.G, 0, (size_t)stride * sizeof(float), s));
+    return RECAD_OK;
+  }
+  const int64_t want = (n * kSeedLanes + 255) / 256;
+  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sm_count() * 32));
+  // E / V of the row regulariser's derivative: the two halves of Y_0
+  bpr_hvp_seeds_kernel<<<grid, 256, 0, s>>>(w.OO, w.OO + D, U, st->n_items, samples, n, 1.0f / (float)n, D / 4, D2 / 4,
+                                            dloss ? w.Y : nullptr, dloss ? w.Y + D : nullptr, lambda,
+                                            w.alpha, w.beta, dloss, w.bad);
+  RECAD_LAUNCH_CHECK();
+  const size_t row3 = 3 * sizeof(int64_t);
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ia, sizeof(int64_t), samples, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ia + n, sizeof(int64_t), samples, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ib, sizeof(int64_t), samples + 2, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
+  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ib + n, sizeof(int64_t), samples + 1, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice,
+                                     s));
+  RECAD_CUDA_CHECK(cudaMemsetAsync(w.G, 0, (size_t)stride * sizeof(float), s));
+  return pair_sides(PairMode::kJoint, w.OO, nullptr, U, w.OO + U * D2, nullptr, st->n_items, D, w.ia, w.ib, 2 * n, w.alpha,
+                    w.beta, w.G, w.G + U * D2, nullptr, nullptr, w.keys, w.tmp, w.sort_scr, w.bad, s);
+}
+
+// The Horner pass of G over A2 at width 2D with the SDDMM hook (gvals = g_v) and, when hg is given, the operand gather.
+static int mixed_horner(const recad_lightgcn* st, const recad_csr* A2, const MixedWork& w, float* gvals, HornerGather* hg,
+                        void* stream) {
+  const int L = st->n_layers;
+  const int64_t stride = (st->n_users + st->n_items) * 2 * (int64_t)st->D;
+  recad_lightgcn joint = *st;
+  joint.graph = A2;
+  joint.graph_t = nullptr;
+  joint.D = 2 * st->D;
+  joint.X0 = w.OO;
+  joint.X1 = w.X1;
+  std::vector<const float*> layers(L);
+  for (int l = 0; l < L; ++l) layers[l] = w.Y + l * stride;
+  const HornerValues hv{layers.data(), gvals, 1.0f / (float)(L + 1)};
+  if (hg) hg->X = layers.data();
+  const float* t = nullptr;
+  return lightgcn_horner(&joint, w.G, 1.0f / (float)(L + 1), nullptr, &t, stream, &hv, hg);
+}
+
+// ------------------------------------------------------------------------------------------
+// Candidate-interaction weight gradients (recad_lightgcn_candidate_weight_grads)
+// ------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+check_ids_kernel(const int64_t* __restrict__ ids, int64_t n, int64_t n_max, int* __restrict__ bad) {
+  const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k < n && (ids[k] < 0 || ids[k] >= n_max)) atomicOr(bad, 1);
+}
+
+// G[r, :D] += gO[r] over the interleaved [G_O | G_dO] rows (nvec = D / 4)
+__global__ void __launch_bounds__(256)
+add_first_half_kernel(float* __restrict__ G, const float* __restrict__ gO, int64_t n_rows, int nvec) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n_rows * nvec) return;
+  const int64_t row = e / nvec;
+  float4* g = reinterpret_cast<float4*>(G) + row * 2 * nvec + (e - row * nvec);
+  const float4 a = *g, b = __ldg(reinterpret_cast<const float4*>(gO) + e);
+  *g = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
+}
+
+// kpos[b] = the entry (u_b, n_users + p_b) of row u_b, -1 when it is not stored (or an id is out of range: the seeds kernel
+// flags it).  One thread per row of the batch, bisection over the user row's ascending columns: the lookup of
+// Graph.entry_index (which interaction_hypergradient uses), O(log deg) whatever the user's degree.
+__global__ void __launch_bounds__(256)
+positive_entry_kernel(const int64_t* __restrict__ samples, int64_t n, const int64_t* __restrict__ rowptr,
+                      const int32_t* __restrict__ colidx, int64_t n_users, int64_t n_items, int64_t* __restrict__ kpos) {
+  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= n) return;
+  const int64_t u = samples[3 * b], p = samples[3 * b + 1];
+  int64_t found = -1;
+  if (u >= 0 && u < n_users && p >= 0 && p < n_items) {
+    const int32_t col = (int32_t)(n_users + p);
+    int64_t lo = rowptr[u], hi = rowptr[u + 1];      // first column >= col in [lo, hi)
+    while (lo < hi) {
+      const int64_t mid = lo + ((hi - lo) >> 1);
+      if (__ldg(colidx + mid) < col) lo = mid + 1;
+      else hi = mid;
+    }
+    if (lo < rowptr[u + 1] && colidx[lo] == col) found = lo;
+  }
+  kpos[b] = found;
+}
+
+// The operands' last columns, hi / lo: A[r, K] = coef[sel[r]], B[i, K] = 1, columns K + 1 .. ld - 1 zero
+__global__ void __launch_bounds__(256)
+tail_split_kernel(const float* __restrict__ coef, const int64_t* __restrict__ sel, int64_t n_sel, int64_t n_users,
+                  int64_t n_items, int K, int ld, float* __restrict__ a_hi, float* __restrict__ a_lo, float* __restrict__ b_hi,
+                  float* __restrict__ b_lo) {
+  const int w = ld - K;
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= (n_sel + n_items) * w) return;
+  const int64_t row = e / w;
+  const int c = K + (int)(e - row * w);
+  float h = 0.f, l = 0.f;
+  if (row < n_sel) {
+    if (c == K) {
+      int64_t u = sel[row];
+      if (u < 0 || u >= n_users) u = 0;
+      split_tf32(coef[u], h, l);
+    }
+    a_hi[row * ld + c] = h;
+    a_lo[row * ld + c] = l;
+  } else {
+    b_hi[(row - n_sel) * ld + c] = c == K ? 1.f : 0.f;
+    b_lo[(row - n_sel) * ld + c] = 0.f;
+  }
+}
+
+// out[r, i] += es[k] / (n mult[k]) at the stored entries k = (sel[r], n_users + i) of the selected user rows: one warp per r,
+// one writer per (r, i) (a row's columns are distinct; a repeated id has rows of its own)
+__global__ void __launch_bounds__(256)
+sample_part_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ colidx, const float* __restrict__ mult,
+                   const float* __restrict__ es, float nf, const int64_t* __restrict__ sel, int64_t n_sel, int64_t n_users,
+                   int64_t n_items, float* __restrict__ out) {
+  const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (r >= n_sel) return;
+  const int64_t u = sel[r];
+  if (u < 0 || u >= n_users) return;
+  for (int64_t e = rowptr[u] + lane; e < rowptr[u + 1]; e += 32) {
+    const float v = es[e];
+    const int64_t i = (int64_t)colidx[e] - n_users;
+    if (v != 0.f && i >= 0 && i < n_items) out[r * n_items + i] += __fdiv_rn(v, __fmul_rn(nf, mult[e]));
+  }
+}
+
+// Workspace of recad_lightgcn_candidate_weight_grads: the mixed driver's (MixedWork), then g_v [nnz], coef [N], the rows'
+// directional derivatives and positive entries [n], the per-entry sums [nnz] and, for L >= 1, the split operands
+// A [n_sel, ld] and B [n_items, ld] (hi and lo each), ld = 4 L D + 4.
+struct CandWork {
+  MixedWork m;
+  float *gvals, *coef, *dloss;
+  int64_t* kpos;
+  float* es;
+  float *a_hi, *a_lo, *b_hi, *b_lo;
+};
+
+static int64_t cand_ld(int32_t D, int32_t L) { return L > 0 ? 4 * (int64_t)L * D + 4 : 0; }
+
+static int64_t cand_work(int64_t U, int64_t I, int32_t D, int32_t L, int64_t n, int64_t nnz, int64_t n_sel, char* base,
+                         CandWork* w) {
+  int64_t off = mixed_work(U + I, D, L, n, base, w ? &w->m : nullptr);
+  auto take = [&](int64_t bytes) { char* p = base ? base + off : nullptr; off += align256(bytes); return p; };
+  const int64_t ld = cand_ld(D, L);
+  char* gvals = take(nnz * 4);
+  char* coef = take((U + I) * 4);
+  char* dloss = take(n * 4);
+  char* kpos = take(n * 8);
+  char* es = take(nnz * 4);
+  char* a_hi = take(n_sel * ld * 4);
+  char* a_lo = take(n_sel * ld * 4);
+  char* b_hi = take(I * ld * 4);
+  char* b_lo = take(I * ld * 4);
+  if (w) {
+    w->gvals = reinterpret_cast<float*>(gvals);
+    w->coef = reinterpret_cast<float*>(coef);
+    w->dloss = reinterpret_cast<float*>(dloss);
+    w->kpos = reinterpret_cast<int64_t*>(kpos);
+    w->es = reinterpret_cast<float*>(es);
+    w->a_hi = reinterpret_cast<float*>(a_hi);
+    w->a_lo = reinterpret_cast<float*>(a_lo);
+    w->b_hi = reinterpret_cast<float*>(b_hi);
+    w->b_lo = reinterpret_cast<float*>(b_lo);
+  }
+  return off;
 }
 
 }  // namespace recad
@@ -955,39 +1213,13 @@ int recad_lightgcn_loss_mixed_values(const recad_lightgcn* st, const recad_csr* 
   const int L = st->n_layers;
   RECAD_REQUIRE(D2 <= 1024, RECAD_ERR_UNSUPPORTED, "lightgcn_loss_mixed_values: D = %d above 512", D);
   RECAD_REQUIRE(n < ((int64_t)1 << 31) - 1, RECAD_ERR_OVERFLOW, "lightgcn_loss_mixed_values: n below 2^31 - 1");
-  const int64_t U = st->n_users, N = st->n_users + st->n_items;
+  const int64_t N = st->n_users + st->n_items;
   RECAD_REQUIRE(work_bytes >= mixed_work(N, D, L, n, nullptr, nullptr), RECAD_ERR_SCRATCH,
                 "lightgcn_loss_mixed_values: work too small");
   MixedWork w;
   mixed_work(N, D, L, n, static_cast<char*>(work), &w);
   cudaStream_t s = as_stream(stream);
-  const size_t row2 = (size_t)D2 * sizeof(float), row1 = (size_t)D * sizeof(float);
-  const int64_t stride = N * D2;
-  // Y_0 = [E | S]; Y_{l+1} = A Y_l and [O | dO] = (1 / (L + 1)) sum_l Y_l: recad_lightgcn_propagate's calls at width 2D
-  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.Y, row2, st->E, row1, row1, N, cudaMemcpyDeviceToDevice, s));
-  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.Y + D, row2, S, row1, row1, N, cudaMemcpyDeviceToDevice, s));
-  for (int k = 0; k < L; ++k) {
-    const bool last = k == L - 1;
-    rc = recad_spmm(A2, w.Y + k * stride, last ? nullptr : w.Y + (k + 1) * stride, k == 0 ? w.Y : w.OO, w.OO,
-                    last ? 1.0f / (float)(L + 1) : 1.0f, D2, stream);
-    if (rc) return rc;
-  }
-  // seeds (a_b, c_b) from the interleaved rows, then G = [G_O | G_dO] by the pairs (u, neg), (u, pos)
-  RECAD_CUDA_CHECK(cudaMemsetAsync(w.bad, 0, sizeof(int), s));
-  const int64_t want = (n * kSeedLanes + 255) / 256;
-  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want, (int64_t)sm_count() * 32));
-  bpr_hvp_seeds_kernel<<<grid, 256, 0, s>>>(w.OO, w.OO + D, U, st->n_items, samples, n, 1.0f / (float)n, D / 4, D2 / 4,
-                                            nullptr, nullptr, 0.0f, w.alpha, w.beta, nullptr, w.bad);
-  RECAD_LAUNCH_CHECK();
-  const size_t row3 = 3 * sizeof(int64_t);
-  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ia, sizeof(int64_t), samples, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
-  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ia + n, sizeof(int64_t), samples, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
-  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ib, sizeof(int64_t), samples + 2, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice, s));
-  RECAD_CUDA_CHECK(cudaMemcpy2DAsync(w.ib + n, sizeof(int64_t), samples + 1, row3, sizeof(int64_t), n, cudaMemcpyDeviceToDevice,
-                                     s));
-  RECAD_CUDA_CHECK(cudaMemsetAsync(w.G, 0, (size_t)stride * sizeof(float), s));
-  rc = pair_sides(PairMode::kJoint, w.OO, nullptr, U, w.OO + U * D2, nullptr, st->n_items, D, w.ia, w.ib, 2 * n, w.alpha,
-                  w.beta, w.G, w.G + U * D2, nullptr, nullptr, w.keys, w.tmp, w.sort_scr, w.bad, s);
+  rc = mixed_recurrence(st, A2, S, samples, n, w, nullptr, 0.0f, stream);
   if (rc) return rc;
   int h_bad = 0;
   RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, w.bad, sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -998,17 +1230,89 @@ int recad_lightgcn_loss_mixed_values(const recad_lightgcn* st, const recad_csr* 
     return RECAD_OK;
   }
   // g_v = (1 / (L + 1)) sum_j <t_j[r], Y_{L-1-j}[c]> over the 2D columns, t_j the Horner iterates of G over A
-  recad_lightgcn joint = *st;
-  joint.graph = A2;
-  joint.graph_t = nullptr;
-  joint.D = D2;
-  joint.X0 = w.OO;
-  joint.X1 = w.X1;
-  std::vector<const float*> layers(L);
-  for (int l = 0; l < L; ++l) layers[l] = w.Y + l * stride;
-  const HornerValues hv{layers.data(), gvals, 1.0f / (float)(L + 1)};
-  const float* t = nullptr;
-  return lightgcn_horner(&joint, w.G, 1.0f / (float)(L + 1), nullptr, &t, stream, &hv);
+  return mixed_horner(st, A2, w, gvals, nullptr, stream);
+}
+
+int64_t recad_lightgcn_candidate_weight_grads_work_bytes(int64_t n_users, int64_t n_items, int32_t D, int32_t n_layers,
+                                                         int64_t n, int64_t nnz, int64_t n_sel) {
+  if (n_users <= 0 || n_items <= 0 || D < 4 || n_layers < 0 || n < 0 || nnz < 0 || n_sel < 0) return -1;
+  return cand_work(n_users, n_items, D, n_layers, n, nnz, n_sel, nullptr, nullptr);
+}
+
+int recad_lightgcn_candidate_weight_grads(const recad_lightgcn* st, const recad_csr* A2, const float* mult,
+                                          const int64_t* tperm, const float* d_inv, const float* gO, const float* S,
+                                          const int64_t* samples, int64_t n, float lambda, const int64_t* users, int64_t n_sel,
+                                          float* out, void* work, int64_t work_bytes, void* stream) {
+  int rc = check_lightgcn(st);
+  if (rc) return rc;
+  RECAD_REQUIRE(A2 && mult && tperm && d_inv && users && out && work && n_sel > 0 && n >= 0 && (n == 0 || (S && samples)),
+                RECAD_ERR_ARG, "lightgcn_candidate_weight_grads: bad argument");
+  const recad_csr* A = st->graph;
+  RECAD_REQUIRE(!st->graph_t && A->n_cols == A->n_rows && A2->n_rows == A->n_rows && A2->n_cols == A->n_cols &&
+                    A2->nnz == A->nnz,
+                RECAD_ERR_ARG, "lightgcn_candidate_weight_grads: A2 must be the state's own (symmetric) graph at width 2D");
+  const int32_t D = st->D;
+  const int L = st->n_layers;
+  RECAD_REQUIRE(D <= 512, RECAD_ERR_UNSUPPORTED, "lightgcn_candidate_weight_grads: D = %d above 512", D);
+  const int64_t U = st->n_users, I = st->n_items, N = U + I, nnz = A->nnz, ld = cand_ld(D, L);
+  RECAD_REQUIRE(n < ((int64_t)1 << 31) - 1 && n_sel < ((int64_t)1 << 31) && I < ((int64_t)1 << 31) && ld < ((int64_t)1 << 31),
+                RECAD_ERR_OVERFLOW, "lightgcn_candidate_weight_grads: n, users, items and 4 L D below 2^31");
+  RECAD_REQUIRE(work_bytes >= cand_work(U, I, D, L, n, nnz, n_sel, nullptr, nullptr), RECAD_ERR_SCRATCH,
+                "lightgcn_candidate_weight_grads: work too small");
+  CandWork w;
+  cand_work(U, I, D, L, n, nnz, n_sel, static_cast<char*>(work), &w);
+  cudaStream_t s = as_stream(stream);
+  rc = mixed_recurrence(st, A2, S, samples, n, w.m, w.dloss, lambda, stream);
+  if (rc) return rc;
+  check_ids_kernel<<<(unsigned)((n_sel + 255) / 256), 256, 0, s>>>(users, n_sel, U, w.m.bad);
+  RECAD_LAUNCH_CHECK();
+  // G = the mixed seed + [gO | 0]: one Horner pass carries the objective's and the loss's parts together
+  if (gO) {
+    add_first_half_kernel<<<(unsigned)((N * (D / 4) + 255) / 256), 256, 0, s>>>(w.m.G, gO, N, D / 4);
+    RECAD_LAUNCH_CHECK();
+  }
+  // per-entry sums of the rows' directional derivatives over the rows whose positive pair is that stored entry
+  if (n > 0) {
+    positive_entry_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(samples, n, A->rowptr, A->colidx, U, I, w.kpos);
+    RECAD_LAUNCH_CHECK();
+    RECAD_CUDA_CHECK(cudaMemsetAsync(w.es, 0, nnz * sizeof(float), s));
+    const int bbits = bit_width(n);
+    const unsigned grid = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 16);
+    index_keys_kernel<<<grid, 256, 0, s>>>(w.kpos, n, nnz, bbits, w.m.keys, w.m.bad);
+    RECAD_LAUNCH_CHECK();
+    rc = radix_sort_u64(w.m.keys, w.m.tmp, n, bbits + bit_width(nnz + 1), w.m.sort_scr, s);
+    if (rc) return rc;
+    index_sums_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(w.m.keys, n, bbits, (uint64_t)nnz, w.dloss, w.es);
+    RECAD_LAUNCH_CHECK();
+  }
+  if (L == 0) {
+    RECAD_CUDA_CHECK(cudaMemsetAsync(out, 0, (size_t)n_sel * I * sizeof(float), s));
+  } else {
+    // g_v at the stored entries and, gathered at every step, the operands of <a_u, b_i>
+    HornerGather hg{nullptr, users, n_sel, U, I, d_inv, 1.0f / (float)(L + 1), (int)ld, w.a_hi, w.a_lo, w.b_hi, w.b_lo};
+    rc = mixed_horner(st, A2, w.m, w.gvals, &hg, stream);
+    if (rc) return rc;
+    // the row-sum term coef_r = -0.5 d_r^3 P_r of the normalisation backward, then column K = [coef_u] x [1]
+    rc = csr_normalize_coef(A->rowptr, A->colidx, tperm, mult, d_inv, w.gvals, N, w.coef, s);
+    if (rc) return rc;
+    const int K = (int)(4 * (int64_t)L * D);
+    tail_split_kernel<<<(unsigned)(((n_sel + I) * (ld - K) + 255) / 256), 256, 0, s>>>(w.coef, users, n_sel, U, I, K, (int)ld,
+                                                                                         w.a_hi, w.a_lo, w.b_hi, w.b_lo);
+    RECAD_LAUNCH_CHECK();
+    rc = gemm_tc(w.a_hi, w.a_lo, (int)n_sel, (int)ld, w.b_hi, w.b_lo, (int)I, (int)ld, K + 1, out, (int)I, w.coef + U, false,
+                 nullptr, nullptr, 0, s);
+    if (rc) return rc;
+  }
+  if (n > 0) {
+    sample_part_kernel<<<(unsigned)((n_sel * 32 + 255) / 256), 256, 0, s>>>(A->rowptr, A->colidx, mult, w.es, (float)n, users,
+                                                                            n_sel, U, I, out);
+    RECAD_LAUNCH_CHECK();
+  }
+  int h_bad = 0;
+  RECAD_CUDA_CHECK(cudaMemcpyAsync(&h_bad, w.m.bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+  RECAD_CUDA_CHECK(cudaStreamSynchronize(s));
+  RECAD_REQUIRE(!h_bad, RECAD_ERR_ARG, "lightgcn_candidate_weight_grads: a user or sample id is out of range");
+  return RECAD_OK;
 }
 
 int recad_index_sums(const int64_t* idx, const float* x, int64_t n, int64_t n_out, float* out, void* scratch,

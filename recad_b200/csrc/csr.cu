@@ -256,6 +256,16 @@ __global__ void append_item_tails_kernel(const uint64_t* __restrict__ item_keys,
   new_mult[p] = 1.0f;
 }
 
+// pass 1 of the normalisation backward on its own: coef [n_rows] from gv [nnz]; no host synchronisation.  Also the row term
+// of an interaction that is not stored yet (recad_lightgcn_candidate_weight_grads)
+int csr_normalize_coef(const int64_t* rowptr, const int32_t* colidx, const int64_t* tperm, const float* w, const float* d_inv,
+                       const float* gv, int64_t n_rows, float* coef, cudaStream_t s) {
+  const int T = 256;
+  norm_bwd_rows_kernel<<<(unsigned)((n_rows * 32 + T - 1) / T), T, 0, s>>>(rowptr, colidx, tperm, w, d_inv, gv, n_rows, coef);
+  RECAD_LAUNCH_CHECK();
+  return RECAD_OK;
+}
+
 }  // namespace recad
 
 using namespace recad;
@@ -368,9 +378,9 @@ int recad_csr_normalize_backward(const int64_t* rowptr, const int32_t* colidx, c
   int rc = check_nnz(rowptr, n_rows, nnz, s, "csr_normalize_backward");
   if (rc) return rc;
   if (nnz == 0) return RECAD_OK;
+  rc = csr_normalize_coef(rowptr, colidx, tperm, w, d_inv, gv, n_rows, coef, s);
+  if (rc) return rc;
   const int T = 256;
-  norm_bwd_rows_kernel<<<(unsigned)((n_rows * 32 + T - 1) / T), T, 0, s>>>(rowptr, colidx, tperm, w, d_inv, gv, n_rows, coef);
-  RECAD_LAUNCH_CHECK();
   const int64_t threads = (nnz + kNormPerThread - 1) / kNormPerThread;
   norm_bwd_entries_kernel<<<(unsigned)((threads + T - 1) / T), T, 0, s>>>(rowptr, colidx, d_inv, gv, coef, n_rows, nnz, gw);
   RECAD_LAUNCH_CHECK();

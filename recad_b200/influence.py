@@ -4,7 +4,8 @@ attacks and defenses (Fang et al., WWW 2020).  H is the Hessian of the training 
 at the victim's current tables.  Works with any victim that has those two methods (LightGCN, MF, NCF).
 
 interaction_hypergradient: for LightGCN, whose training loss depends on the interactions both as training rows and as
-graph edges, the derivative of an objective of the retrained tables with respect to every interaction weight."""
+graph edges, the derivative of an objective of the retrained tables with respect to every interaction weight;
+candidate_hypergradient: the same derivative for chosen users against every item, at interactions not stored yet too."""
 import math
 from collections import namedtuple
 
@@ -15,6 +16,7 @@ from ._lib import RecadError
 
 Influence = namedtuple("Influence", ["values", "s", "iterations", "residual"])
 Hypergradient = namedtuple("Hypergradient", ["values", "direct", "implicit", "s", "iterations", "residual"])
+CandidateHypergradient = namedtuple("CandidateHypergradient", ["values", "s", "iterations", "residual"])
 
 
 def conjugate_gradient(hvp, rhs, damping, max_iter=100, rtol=1e-6):
@@ -134,3 +136,46 @@ def interaction_hypergradient(victim, batch, objective, damping, max_iter=100, r
     sample_part = ops.index_sums(k, dl, g.nnz) / (dl.numel() * g.mult)
     implicit = graph_part + sample_part
     return Hypergradient(direct - implicit, direct, implicit, s, iters, res)
+
+
+def candidate_hypergradient(victim, batch, objective, users, damping, max_iter=100, rtol=1e-6):
+    """dJ/dW[r, i] for one weight W on both entries of the interaction (users[r], item i), for every item, stored or not
+    (W = Graph.mult on stored pairs, 0 on the others), of an objective J of the LightGCN tables trained on the BPR loss of
+    `batch` (rows weighted as for interaction_hypergradient):
+
+        dJ/dW = dJ/dW|_E - M^T s,   s = (H + damping I)^-1 grad_E J
+
+    at the victim's current tables, taken as trained.  objective(user_out, item_out) returns a scalar tensor built from
+    the two outputs of computer(); its gradient gO comes from torch autograd on a fresh propagation, grad_E J =
+    P^T gO, s is solved by conjugate_gradient in float64 over loss_hvp, and values =
+    victim.candidate_weight_gradients(users, gO, batch, -s).  At a stored pair, values equals values[k] + values[T[k]] of
+    interaction_hypergradient for the same objective.  Sign convention: a negative values[r, i] means that adding the
+    interaction (users[r], i) -- raising its weight from 0 -- lowers J to first order (a positive one, that it raises J).
+    Returns CandidateHypergradient(values float32 [len(users), num_items], s, iterations, residual).  LightGCN only
+    (DESIGN.md, "Second order"); deterministic; the model is not changed."""
+    from .victim.lightgcn import LightGCN
+    if not isinstance(victim, LightGCN):
+        raise RecadError(f"candidate_hypergradient: LightGCN victims only (got {type(victim).__name__})")
+    victim._require_instance("candidate_hypergradient")
+    if victim.dropout and victim.training:
+        raise RecadError("candidate_hypergradient: not defined under graph dropout in training mode (call eval() first)")
+    # the users and the batch are checked before the propagation and the solve, not after them
+    victim._check_candidate_users(users, "candidate_hypergradient")
+    if users.numel() and bool(((users < 0) | (users >= victim.num_users)).any()):
+        raise RecadError("candidate_hypergradient: a user id is out of range")
+    victim._loss_rows(batch, "candidate_hypergradient")
+    U = victim.num_users
+    with torch.cuda.device(victim._dev):
+        O, _ = ops.lightgcn_propagate_layers(victim._st, victim.E, keep=False)
+        uo = O[:U].clone().requires_grad_(True)
+        io = O[U:].clone().requires_grad_(True)
+        with torch.enable_grad():
+            J = objective(uo, io)
+            if not isinstance(J, torch.Tensor) or J.numel() != 1:
+                raise RecadError("candidate_hypergradient: the objective must return a scalar tensor")
+            gu, gi = torch.autograd.grad(J.reshape(()), [uo, io], allow_unused=True)
+        gO = [torch.zeros_like(uo) if g is None else g.detach().float().contiguous() for g in (gu, gi)]
+        gE = ops.lightgcn_backward(victim._st, torch.cat(gO))
+    s, iters, res = _solve(victim, batch, [gE[:U], gE[U:]], damping, max_iter, rtol)
+    values = victim.candidate_weight_gradients(users, gO, batch, [-x for x in s])
+    return CandidateHypergradient(values, s, iters, res)

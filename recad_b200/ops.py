@@ -539,6 +539,38 @@ def lightgcn_loss_mixed_values(st, graph, S, samples):
     return out
 
 
+def lightgcn_candidate_weight_grads(st, graph, users, gO=None, S=None, samples=None, lam=0.0):
+    """recad_lightgcn_candidate_weight_grads: float32 [len(users), n_items], the gradient of <gO, O> + <S, grad_E L> with
+    respect to one weight on both entries of every interaction (users[r], item i), stored or not, at the base point
+    W = graph.mult (0 where not stored), for a LightGCN state over `graph` (its own values).  users int64 [R]; gO, S float32
+    [N, D] or None; samples int64 [n, 3] (with S) or None; lam the regulariser's weight in the rows' losses.  d_inv is
+    weights_d_inv(graph, graph.mult), so the base point's values are normalized_values(graph, graph.mult) bit for bit.
+    Fresh buffers only."""
+    _need_cuda(users, gO, S, samples)
+    if (S is None) != (samples is None):
+        raise RecadError("lightgcn_candidate_weight_grads: S and samples go together")
+    if graph.mult is None:
+        raise RecadError("lightgcn_candidate_weight_grads: the graph carries no interaction weights (mult)")
+    dev = users.device
+    U, I, D = st.n_users, st.n_items, st.D
+    n = 0 if samples is None else int(samples.shape[0])
+    R = int(users.numel())
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        out = torch.empty((R, I), dtype=torch.float32, device=dev)
+        if R == 0:
+            return out
+        users = users.contiguous().long()
+        d_inv = weights_d_inv(graph, graph.mult)
+        nbytes = int(L.recad_lightgcn_candidate_weight_grads_work_bytes(U, I, D, st.n_layers, n, graph.nnz, R))
+        work = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=dev)
+        check(L.recad_lightgcn_candidate_weight_grads(
+            C.byref(st), C.byref(graph.struct(2 * D)), _ptr(graph.mult), _ptr(graph.transpose_permutation()), _ptr(d_inv),
+            _ptr(gO), _ptr(S), _ptr(samples), n, float(lam), _ptr(users), R, _ptr(out), _ptr(work), nbytes, _stream(dev)),
+            "recad_lightgcn_candidate_weight_grads")
+    return out
+
+
 def index_sums(idx, x, n_out):
     """out[r] = sum of x[b] over the b with idx[b] = r (float32 [n_out]; entries of idx below 0 are skipped), atomic-free and
     bit-stable (recad_index_sums: one stable sort, one writer per output, summed in double).  An index >= n_out raises."""
@@ -763,6 +795,17 @@ def lightgcn_propagate_values(st_vals, E):
     return O
 
 
+def weights_d_inv(graph, weights):
+    """d_r = (s_r + 1e-14)^(-1/2) of the row sums s_r of per-entry weights [nnz] (recad_csr_row_sums, then the host
+    expression d_inv_from_degree): the normalisation factors normalized_values uses."""
+    dev = graph.device
+    with torch.cuda.device(dev):
+        sums = torch.empty(graph.n_rows, dtype=torch.float32, device=dev)
+        check(_lib.lib().recad_csr_row_sums(_ptr(graph.rowptr), _ptr(weights), graph.n_rows, graph.nnz, _ptr(sums),
+                                            _stream(dev)), "recad_csr_row_sums")
+        return torch.from_numpy(d_inv_from_degree(sums.cpu().numpy())).to(dev)
+
+
 class NormalizedValues(torch.autograd.Function):
     """vals_k = d_r w_k d_c from per-entry weights (recad_csr_row_sums, the host d_inv, recad_csr_normalize); backward by
     recad_csr_normalize_backward."""
@@ -772,10 +815,7 @@ class NormalizedValues(torch.autograd.Function):
         dev = graph.device
         lib = _lib.lib()
         with torch.cuda.device(dev):
-            sums = torch.empty(graph.n_rows, dtype=torch.float32, device=dev)
-            check(lib.recad_csr_row_sums(_ptr(graph.rowptr), _ptr(weights), graph.n_rows, graph.nnz, _ptr(sums), _stream(dev)),
-                  "recad_csr_row_sums")
-            d_inv = torch.from_numpy(d_inv_from_degree(sums.cpu().numpy())).to(dev)
+            d_inv = weights_d_inv(graph, weights)
             vals = torch.empty(graph.nnz, dtype=torch.float32, device=dev)
             check(lib.recad_csr_normalize(_ptr(graph.rowptr), _ptr(graph.colidx), _ptr(weights), _ptr(d_inv), graph.n_rows,
                                           _ptr(vals), _stream(dev)), "recad_csr_normalize")

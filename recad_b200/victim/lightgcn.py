@@ -335,6 +335,41 @@ class LightGCN(BaseVictim):
         with torch.cuda.device(self._dev):
             return ops.lightgcn_loss_mixed_values(self._st, self.Graph, V, samples)
 
+    def _check_candidate_users(self, users, what):
+        """RecadError unless `users` is an int64 / int32 CUDA tensor [R] on the model's device (ids are range-checked by the
+        kernel)."""
+        if not isinstance(users, torch.Tensor) or not users.is_cuda or users.device != self._dev:
+            raise ops.RecadError(f"{what}: users must be a CUDA tensor on {self._dev}")
+        if users.dim() != 1 or users.dtype not in (torch.int64, torch.int32):
+            raise ops.RecadError(f"{what}: users must be int64 [R], got {users.dtype} {list(users.shape)}")
+
+    def candidate_weight_gradients(self, users, gO=None, batch=None, vectors=None):
+        """df/dW[r, i] for f(W) = <gO, O(W)> + <v_vec, grad_E L_batch(E; W)>, W one weight on both entries (users[r], U + i)
+        and (U + i, users[r]) of an interaction, for every item i, stored or not: float32 [len(users), num_items].  The base
+        point is W = Graph.mult on stored pairs and 0 elsewhere, at the current tables; O = (users_out, items_out) of
+        computer().  gO: (g_user [U, D], g_item [I, D]) float32 or None; batch and vectors (shaped as for loss_hvp) go
+        together or are both None; L_batch weights row b by w_k / mult_k when its positive pair k is stored.  users: int64
+        CUDA ids (repeats allowed; empty gives [0, num_items]).  At a stored pair the value is the sum over the pair's two
+        entries of normalized_values' backward of the edge-value gradient, plus the sample part of interaction_hypergradient.
+        Deterministic; the model is not changed.  One width-2D recurrence and one tensor-core GEMM (DESIGN.md, "Second
+        order")."""
+        what = "LightGCN.candidate_weight_gradients"
+        self._require_instance("candidate_weight_gradients")
+        if self.dropout and self.training:
+            raise ops.RecadError(f"{what}: not defined under graph dropout in training mode (call eval() first)")
+        if (batch is None) != (vectors is None):
+            raise ops.RecadError(f"{what}: batch and vectors go together")
+        self._check_candidate_users(users, what)
+        U, I, D = self.num_users, self.num_items, self.latent_dim
+        G = S = samples = None
+        with torch.cuda.device(self._dev):
+            if gO is not None:
+                G = torch.cat(self._check_vectors(gO, [(U, D), (I, D)], what))
+            if batch is not None:
+                samples, S = self._loss_inputs(batch, vectors, "candidate_weight_gradients")
+            return ops.lightgcn_candidate_weight_grads(self._st, self.Graph, users.long(), G, S, samples,
+                                                       float(self.config["lambda"]))
+
     def input_describe(self):
         return {
             "train_step": {"users": (torch.int64, "batch"), "positive_items": (torch.int64, "batch"),
